@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: decoded Mpixel/s for a batch of 1080p key frames through -yuvf (recon + loop filter -> I420).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload yuvf|yuv|ppm] [--batch B]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload yuvf|yuv|ppm] [--batch B] [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...      (one rank per GPU)
     python bench.py --impl reference ...                                              (reference CPU arm)
 
@@ -317,6 +317,8 @@ def gpu_arm(args):
     else:
         buf, offs, sizes = ctx.download_i420(batch)
     parity = check(buf, offs, sizes)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(Path(args.dump_outputs), args.workload, buf, offs, sizes)
     del buf
     batch.free()
     ctx.trim()
@@ -444,6 +446,40 @@ def gpu_arm(args):
     if world > 1:
         dist.destroy_process_group()
     return 0
+
+
+DUMP_BYTES = 64 << 20
+DUMP_SAMPLES_PER_FRAME = 8192
+
+
+def dump_outputs(out_dir, name, buf, offs, sizes):
+    """Writes what the last timed step computed (frame i = buf[offs[i]:offs[i]+sizes[i]]) to out_dir, so that two builds can be
+    compared output for output; the inputs are the same files on every run. At most DUMP_BYTES in all:
+      <name>_frame0.npy       every byte of frame 0, float32
+      <name>_sample.npy       (frames, K) float32: the bytes at K positions per frame, drawn with a fixed seed (the same
+                              positions for every frame of one size)
+      <name>_frame_sums.npy   float64 sum of every byte of each frame (exact), so that a change outside the sample shows too"""
+    import numpy as np
+    out_dir.mkdir(parents=True, exist_ok=True)
+    offs, sizes = offs.astype(np.int64), sizes.astype(np.int64)
+    n = len(offs)
+    frame0 = buf[offs[0]:offs[0] + sizes[0]].astype(np.float32)
+    payload = DUMP_BYTES - 3 * 4096  # room for the three .npy headers (128 bytes each as numpy writes them today)
+    k = int(min(DUMP_SAMPLES_PER_FRAME, sizes.min(), (payload - frame0.nbytes - 8 * n) // (4 * n)))
+    if k < 1:
+        raise SystemExit(f"--dump-outputs: {n} frames do not fit {DUMP_BYTES >> 20} MB")
+    positions = {}
+    sample = np.empty((n, k), np.float32)
+    sums = np.empty(n, np.float64)
+    for i, (o, s) in enumerate(zip(offs, sizes)):
+        if s not in positions:
+            positions[s] = np.sort(np.random.default_rng(int(s)).choice(int(s), k, replace=False))
+        frame = buf[o:o + s]
+        sample[i] = frame[positions[s]]
+        sums[i] = frame.sum(dtype=np.uint64)
+    np.save(out_dir / f"{name}_frame0.npy", frame0)
+    np.save(out_dir / f"{name}_sample.npy", sample)
+    np.save(out_dir / f"{name}_frame_sums.npy", sums)
 
 
 def _layout(ctx, kfs, ppm):
@@ -757,7 +793,12 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-configs", action="store_true")
     ap.add_argument("--no-bind", action="store_true", help="do not bind ranks to the CPUs local to their GPU")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed (rank 0) as .npy files to DIR")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if not (args.impl == "b200" and args.gpus > 1 and world == 1):  # (the relaunching parent just passes its children's output on)
         claim_stdout()

@@ -2,7 +2,8 @@
    - digests produced by the UNMODIFIED reference decoder binary on 254 .webp inputs (tests/golden/digests.json),
    - RGB pixels of the reference's dwebp-derived golden PNGs (149 of those inputs), i.e. libwebp itself,
    - digests of the reference hot path on 120 struct-level fuzz frames (simple filter, sharpness, lf deltas, int16 wrap),
-   - and, where oracle/_ref exists (the CPU container), the reference library called directly on fresh fuzz frames."""
+   - and the reference library called directly on fresh fuzz frames where oracle/_ref is built, else its digests
+     (tests/golden/ref_checks.json)."""
 import ctypes as C
 import json
 
@@ -73,37 +74,58 @@ def test_oracle_matches_reference_fuzz_digests(oracle):
     assert min(seen.values()) >= 30, seen  # the branches no bitstream fixture reaches are exercised
 
 
-@pytest.mark.parametrize("seed", range(0, 60))
-def test_oracle_vs_reference_library(oracle, reference, seed):
+def library_case(seed):
     rng = np.random.default_rng(seed + 777)
     w, h = int(rng.integers(1, 120)), int(rng.integers(1, 120))
-    fr = fuzz_frame(seed + 5000, w, h, amp=[5, 40, 400, 2500][seed % 4], density=[0.05, 0.2, 0.6][seed % 3], raw=bool(seed % 2))
-    for filt in (False, True):
-        assert np.array_equal(oracle.decode_i420(fr, filt), reference.decode_i420(fr, filt))
-    # has_coeff == NULL is legal input (vp8_loopfilter.c:226)
-    assert np.array_equal(oracle.decode_i420(fr, True, drop_has_coeff=True), reference.decode_i420(fr, True, drop_has_coeff=True))
-    yuvf = oracle.decode_i420(fr, True)
-    rgb = oracle.rgb(yuvf, w, h)
-    assert oracle.ppm(rgb, w, h) == reference.ppm_bytes(yuvf, w, h)
-    assert oracle.png(rgb, w, h) == reference.png_bytes(yuvf, w, h)
-    # stand-alone loop filter on padded planes
+    return fuzz_frame(seed + 5000, w, h, amp=[5, 40, 400, 2500][seed % 4], density=[0.05, 0.2, 0.6][seed % 3], raw=bool(seed % 2))
+
+
+def library_outputs(checker, oracle, fr):
+    """sha256 of what `checker` (the oracle or the reference library) computes for one fuzz frame."""
+    w, h = fr.width, fr.height
+    out = {"yuv": checker.decode_i420(fr, False), "yuvf": checker.decode_i420(fr, True),
+           # has_coeff == NULL is legal input (vp8_loopfilter.c:226)
+           "yuvf_no_has_coeff": checker.decode_i420(fr, True, drop_has_coeff=True)}
+    yuvf = out["yuvf"]
+    if checker is oracle:
+        rgb = oracle.rgb(yuvf, w, h)
+        out["ppm"], out["png"] = oracle.ppm(rgb, w, h), oracle.png(rgb, w, h)
+    else:
+        out["ppm"], out["png"] = checker.ppm_bytes(yuvf, w, h), checker.png_bytes(yuvf, w, h)
+    # stand-alone loop filter on padded planes (the oracle's reconstruction as input for both)
     y, u, v = oracle.recon_padded(fr)
-    y2, u2, v2 = y.copy(), u.copy(), v.copy()
-    oracle.loopfilter_padded(fr, y, u, v)
-    reference.loopfilter_padded(fr, y2, u2, v2)
-    assert np.array_equal(y, y2) and np.array_equal(u, u2) and np.array_equal(v, v2)
+    checker.loopfilter_padded(fr, y, u, v)
+    out.update(lf_y=y, lf_u=u, lf_v=v)
+    return {k: sha(v) for k, v in out.items()}
 
 
-def test_rgb_closed_form_on_tiny_and_odd_sizes(oracle, reference):
+def rgb_cases():
     rng = np.random.default_rng(5)
     for w, h in [(1, 1), (2, 2), (3, 5), (16, 16), (17, 9), (18, 10), (31, 32), (64, 7), (2, 1), (1, 2), (5, 1)]:
-        i420 = rng.integers(0, 256, w * h + 2 * ((w + 1) // 2) * ((h + 1) // 2)).astype(np.uint8)
-        assert np.array_equal(oracle.rgb(i420, w, h), reference.rgb(i420, w, h)), (w, h)
+        yield f"{w}x{h}", w, h, rng.integers(0, 256, w * h + 2 * ((w + 1) // 2) * ((h + 1) // 2)).astype(np.uint8)
 
 
-def test_png_block_boundaries(oracle, reference):
+def png_cases():
     # raw scanline stream sizes around the 65535-byte stored-block limit
     rng = np.random.default_rng(9)
     for w, h in [(21845, 1), (150, 145), (149, 146), (2731, 8), (300, 73)]:
-        i420 = rng.integers(0, 256, w * h + 2 * ((w + 1) // 2) * ((h + 1) // 2)).astype(np.uint8)
-        assert oracle.png(oracle.rgb(i420, w, h), w, h) == reference.png_bytes(i420, w, h), (w, h)
+        yield f"{w}x{h}", w, h, rng.integers(0, 256, w * h + 2 * ((w + 1) // 2) * ((h + 1) // 2)).astype(np.uint8)
+
+
+@pytest.mark.parametrize("seed", range(0, 60))
+def test_oracle_vs_reference_library(oracle, reference, ref_digests, seed):
+    fr = library_case(seed)
+    want = library_outputs(reference, oracle, fr) if reference is not None else ref_digests["library"][str(seed)]
+    assert library_outputs(oracle, oracle, fr) == want
+
+
+def test_rgb_closed_form_on_tiny_and_odd_sizes(oracle, reference, ref_digests):
+    for key, w, h, i420 in rgb_cases():
+        want = sha(reference.rgb(i420, w, h)) if reference is not None else ref_digests["rgb"][key]
+        assert sha(oracle.rgb(i420, w, h)) == want, (w, h)
+
+
+def test_png_block_boundaries(oracle, reference, ref_digests):
+    for key, w, h, i420 in png_cases():
+        want = sha(reference.png_bytes(i420, w, h)) if reference is not None else ref_digests["png"][key]
+        assert sha(oracle.png(oracle.rgb(i420, w, h), w, h)) == want, (w, h)
