@@ -463,6 +463,100 @@ void frame_params(const Vp8DecodedFrame* f, int16_t dq[4][6], uint8_t lf[4][2][4
 	}
 }
 
+// Header arithmetic of a batch entry. any_filter looks only at the segments in use, so m.has_seg is set first.
+void frame_setup(FrameMeta& m, const Vp8DecodedFrame* f) {
+	frame_params(f, m.dq, m.lf);
+	m.lf_simple = f->lf_use_simple;
+	m.any_filter = false;
+	for (int s = 0; s < (m.has_seg ? 4 : 1); s++)
+		for (int k = 0; k < 2; k++) m.any_filter |= m.lf[s][k][0] != 0;
+}
+
+// The nine arrays of a dense frame, in FrameMeta::in_off order, and how many bytes of each a batch takes: none of an
+// array it does not read (without need_coeffs only what the loop filter reads is staged).
+struct DenseArrays {
+	const uint8_t* src[9];
+	size_t sz[9];
+};
+DenseArrays dense_arrays(const Vp8DecodedFrame* f, bool need_coeffs, bool has_seg) {
+	const size_t mb = (size_t)f->mb_cols * f->mb_rows, cmb = need_coeffs ? mb : 0;
+	return {{(const uint8_t*)f->coeff_y, (const uint8_t*)f->coeff_u, (const uint8_t*)f->coeff_v, (const uint8_t*)f->coeff_y2, f->bmode,
+	         f->ymode, f->uv_mode, f->segment_id, f->has_coeff},
+	        {cmb * 512, cmb * 128, cmb * 128, cmb * 32, cmb * 16, mb, cmb, has_seg ? mb : 0, f->has_coeff ? mb : 0}};
+}
+
+// ------------------------------------------------------------------------------------------------ output slots
+// Every output holds frame after frame, each in a 256-byte aligned slot: the batch arenas and the caller's buffer of a
+// pipelined call alike. A PPM slot has kPpmSlot bytes of header room in front of the RGB.
+int ppm_header(char* buf, uint32_t w, uint32_t h) { return snprintf(buf, 32, "P6\n%u %u\n255\n", w, h); }
+
+// Bytes of a frame's slot that its output in `format` takes.
+size_t out_bytes(size_t w, size_t h, int format) {
+	return format == VP8_GPU_OUT_PNG   ? vp8_png_file_bytes((uint32_t)w, (uint32_t)h)
+	       : format == VP8_GPU_OUT_PPM ? kPpmSlot + w * h * 3
+	                                   : w * h + 2 * ((w + 1) / 2) * ((h + 1) / 2);
+}
+size_t out_slot_bytes(size_t w, size_t h, int format) { return align_up(out_bytes(w, h, format)); }
+
+// A PNG is one IDAT chunk, whose length field is 31 bits.
+bool png_fits(uint64_t w, uint64_t h) { return (3 * w + 1) * h <= 0x7FFFFFFFull; }
+
+// Frame i's file in its downloaded slot at dst + slot: offsets[i] / sizes[i], and the PPM header in front of the RGB.
+void report_slot(uint8_t* dst, size_t slot, uint32_t w, uint32_t h, int format, int i, size_t* offsets, size_t* sizes) {
+	size_t at = slot, bytes = out_bytes(w, h, format);
+	if (format == VP8_GPU_OUT_PPM) {
+		char hdr[32];
+		const int hl = ppm_header(hdr, w, h);
+		at += kPpmSlot - hl;
+		bytes -= kPpmSlot - hl;
+		memcpy(dst + at, hdr, hl);
+	}
+	if (offsets) offsets[i] = at;
+	if (sizes) sizes[i] = bytes;
+}
+
+// Frame i's slot in the batch's arena of `format`.
+size_t slot_off(const vp8_gpu_batch* b, int i, int format) {
+	return format == VP8_GPU_OUT_PNG ? b->png_off[i] : format == VP8_GPU_OUT_PPM ? b->meta[i].rgb_off : b->meta[i].tight_off;
+}
+
+// The batch's arena of `format`: device block, size, and the bytes up to the end of the last frame (what a download copies).
+struct OutArena {
+	const uint8_t* dev;
+	size_t bytes, used;
+};
+OutArena out_arena(const vp8_gpu_batch* b, int format) {
+	const FrameMeta& last = b->meta.back();
+	const size_t used = slot_off(b, b->n - 1, format) + out_bytes(last.width, last.height, format);
+	if (format == VP8_GPU_OUT_PNG) return {b->d_png, b->png_bytes, used};
+	if (format == VP8_GPU_OUT_PPM) return {b->d_rgb, b->rgb_bytes, used};
+	return {b->d_tight, b->tight_bytes, used};
+}
+
+// vp8_gpu_download_i420 / _ppm / _png once the batch holds that output.
+int download_out(vp8_gpu_ctx* c, vp8_gpu_batch* b, int format, uint8_t* dst, size_t cap, size_t* offsets, size_t* sizes) {
+	const OutArena a = out_arena(b, format);
+	if (cap < a.bytes) return fail(EINVAL, "destination too small");
+	CU(cudaSetDevice(c->device));
+	if (download(c, b->stream, dst, a.dev, a.used)) return -1;
+	for (int i = 0; i < b->n; i++) report_slot(dst, slot_off(b, i, format), b->meta[i].width, b->meta[i].height, format, i, offsets, sizes);
+	return 0;
+}
+
+// Slots of the I420 and PPM arenas (the PNG one is laid out on first use: png_layout).
+void out_layout(vp8_gpu_batch* b) {
+	size_t tight = 0, rgb = 0;
+	for (FrameMeta& m : b->meta) {
+		m.tight_off = tight;
+		tight += out_slot_bytes(m.width, m.height, VP8_GPU_OUT_I420);
+		m.rgb_off = rgb;
+		rgb += out_slot_bytes(m.width, m.height, VP8_GPU_OUT_PPM);
+		b->max_mb_cols = std::max<int>(b->max_mb_cols, m.mb_cols);
+	}
+	b->tight_bytes = tight;
+	b->rgb_bytes = rgb;
+}
+
 // ------------------------------------------------------------------------------------------------ batches
 void batch_destroy(vp8_gpu_ctx* c, vp8_gpu_batch* b, bool known_idle = false) {
 	if (!b) return;
@@ -508,7 +602,7 @@ int batch_create(vp8_gpu_ctx* c, const Vp8KeyFrameHeader* const* kf, const Vp8De
 	b->stream = st ? st : c->stream;
 	b->have_coeffs = need_coeffs;
 	b->meta.resize(n);
-	size_t in = 0, tight = 0, pad = 0, rgb = 0;
+	size_t in = 0, pad = 0;
 	for (int i = 0; i < n; i++) {
 		FrameMeta& m = b->meta[i];
 		const Vp8DecodedFrame* f = fr[i];
@@ -516,14 +610,9 @@ int batch_create(vp8_gpu_ctx* c, const Vp8KeyFrameHeader* const* kf, const Vp8De
 		m.height = kf[i]->height;
 		m.mb_cols = f->mb_cols;
 		m.mb_rows = f->mb_rows;
-		const size_t mb = (size_t)m.mb_cols * m.mb_rows;
 		m.has_seg = f->segmentation_enabled && f->segment_id;
 		m.has_hc = f->has_coeff != nullptr;
-		const size_t sz[9] = {need_coeffs ? mb * 512 : 0, need_coeffs ? mb * 128 : 0, need_coeffs ? mb * 128 : 0,
-		                      need_coeffs ? mb * 32 : 0,  need_coeffs ? mb * 16 : 0,  mb,
-		                      need_coeffs ? mb : 0,       m.has_seg ? mb : 0,         m.has_hc ? mb : 0};
-		const uint8_t* src[9] = {(const uint8_t*)f->coeff_y, (const uint8_t*)f->coeff_u, (const uint8_t*)f->coeff_v,
-		                         (const uint8_t*)f->coeff_y2, f->bmode, f->ymode, f->uv_mode, f->segment_id, f->has_coeff};
+		const auto [src, sz] = dense_arrays(f, need_coeffs, m.has_seg);
 		// Arrays carved from one host block (vp8_parse arenas do that) travel as ONE transfer and keep their relative
 		// placement on the device; scattered arrays (the reference's ten callocs) are laid out and copied one by one.
 		const uint8_t *lo = nullptr, *hi = nullptr;
@@ -564,9 +653,6 @@ int batch_create(vp8_gpu_ctx* c, const Vp8KeyFrameHeader* const* kf, const Vp8De
 				in += align_up(sz[k]);
 			}
 		}
-		const size_t cw = (m.width + 1) / 2, ch = (m.height + 1) / 2;
-		m.tight_off = tight;
-		tight += align_up((size_t)m.width * m.height + 2 * cw * ch);
 		const size_t pw = (size_t)m.mb_cols * 16, ph = (size_t)m.mb_rows * 16;
 		m.pad_off[0] = pad;
 		pad += align_up(pw * ph);
@@ -574,19 +660,11 @@ int batch_create(vp8_gpu_ctx* c, const Vp8KeyFrameHeader* const* kf, const Vp8De
 		pad += align_up(pw * ph / 4);
 		m.pad_off[2] = pad;
 		pad += align_up(pw * ph / 4);
-		m.rgb_off = rgb;
-		rgb += align_up(kPpmSlot + (size_t)m.width * m.height * 3);
-		frame_params(f, m.dq, m.lf);
-		m.lf_simple = f->lf_use_simple;
-		m.any_filter = false;
-		for (int s = 0; s < (m.has_seg ? 4 : 1); s++)
-			for (int k = 0; k < 2; k++) m.any_filter |= m.lf[s][k][0] != 0;
-		b->max_mb_cols = std::max<int>(b->max_mb_cols, m.mb_cols);
+		frame_setup(m, f);
 	}
+	out_layout(b);
 	b->in_bytes = align_up(in);
-	b->tight_bytes = tight;
 	b->pad_bytes = pad;
-	b->rgb_bytes = rgb;
 
 	if (dev_alloc(c, b->in_bytes, (void**)&b->d_in) || dev_alloc(c, sizeof(Vp8ImgDesc) * n, (void**)&b->d_desc)) {
 		batch_destroy(c, b);
@@ -595,8 +673,6 @@ int batch_create(vp8_gpu_ctx* c, const Vp8KeyFrameHeader* const* kf, const Vp8De
 	Uploader up{c, b->stream};
 	for (int i = 0; i < n; i++) {
 		const FrameMeta& m = b->meta[i];
-		const Vp8DecodedFrame* f = fr[i];
-		const size_t mb = (size_t)m.mb_cols * m.mb_rows;
 		if (m.span_src) {
 			size_t bytes = m.span_bytes;
 			int j = i;
@@ -611,10 +687,7 @@ int batch_create(vp8_gpu_ctx* c, const Vp8KeyFrameHeader* const* kf, const Vp8De
 			i = j;
 			continue;
 		}
-		const void* src[9] = {f->coeff_y, f->coeff_u, f->coeff_v, f->coeff_y2, f->bmode, f->ymode, f->uv_mode, f->segment_id, f->has_coeff};
-		const size_t sz[9] = {need_coeffs ? mb * 512 : 0, need_coeffs ? mb * 128 : 0, need_coeffs ? mb * 128 : 0,
-		                      need_coeffs ? mb * 32 : 0,  need_coeffs ? mb * 16 : 0,  mb,
-		                      need_coeffs ? mb : 0,       m.has_seg ? mb : 0,         m.has_hc ? mb : 0};
+		const auto [src, sz] = dense_arrays(fr[i], need_coeffs, m.has_seg);
 		for (int k = 0; k < 9; k++)
 			if (sz[k] && up.put(b->d_in + m.in_off[k], src[k], sz[k])) {
 				batch_destroy(c, b);
@@ -666,6 +739,30 @@ int ensure_planes(vp8_gpu_ctx* c, vp8_gpu_batch* b, int layout) {
 	return 0;
 }
 
+// A frame's Y/U/V in the batch's planes: tight (the I420 slot, visible size) or padded (whole macroblocks).
+struct PlaneView {
+	uint8_t *y, *u, *v;
+	uint32_t w, h, stride_y, stride_uv;
+};
+PlaneView plane_view(const vp8_gpu_batch* b, const FrameMeta& m, bool tight) {
+	if (tight) {
+		const uint32_t cw = (m.width + 1) / 2;
+		uint8_t* y = b->d_tight + m.tight_off;
+		uint8_t* u = y + (size_t)m.width * m.height;
+		return {y, u, u + (size_t)cw * ((m.height + 1) / 2), m.width, m.height, m.width, cw};
+	}
+	const uint32_t pw = m.mb_cols * 16;
+	return {b->d_pad + m.pad_off[0], b->d_pad + m.pad_off[1], b->d_pad + m.pad_off[2], pw, m.mb_rows * 16, pw, pw / 2};
+}
+
+// Frames whose every macroblock has filter level 0 come out of m07 unchanged (vp8_loopfilter.c:220), so a batch made
+// only of such frames takes the reconstruction-only kernel.
+int wavefront_mode(const vp8_gpu_batch* b, bool filtered) {
+	bool any = false;
+	for (auto& m : b->meta) any |= m.any_filter;
+	return (filtered && any) ? VP8_K_RECON_FILTER : VP8_K_RECON;
+}
+
 // Descriptors for one launch. kernel_mode: Vp8KernelMode; layout: where the pixels go.
 int push_descs(vp8_gpu_ctx* c, vp8_gpu_batch* b, int kernel_mode, int layout) {
 	if (b->desc_key == kernel_mode * 2 + layout) return 0; // already resident
@@ -676,31 +773,21 @@ int push_descs(vp8_gpu_ctx* c, vp8_gpu_batch* b, int kernel_mode, int layout) {
 		memset(&d, 0, sizeof(d));
 		d.mb_cols = m.mb_cols;
 		d.mb_rows = m.mb_rows;
-		const uint32_t pw = m.mb_cols * 16, ph = m.mb_rows * 16;
-		if (layout == VP8_GPU_TIGHT) {
-			const size_t cw = (m.width + 1) / 2, ch = (m.height + 1) / 2;
-			d.out_w = m.width;
-			d.out_h = m.height;
-			d.out_stride_y = m.width;
-			d.out_stride_uv = (uint32_t)cw;
-			d.out_y = b->d_tight + m.tight_off;
-			d.out_u = d.out_y + (size_t)m.width * m.height;
-			d.out_v = d.out_u + cw * ch;
-		} else {
-			d.out_w = pw;
-			d.out_h = ph;
-			d.out_stride_y = pw;
-			d.out_stride_uv = pw / 2;
-			d.out_y = b->d_pad + m.pad_off[0];
-			d.out_u = b->d_pad + m.pad_off[1];
-			d.out_v = b->d_pad + m.pad_off[2];
-		}
+		const PlaneView o = plane_view(b, m, layout == VP8_GPU_TIGHT);
+		d.out_w = o.w;
+		d.out_h = o.h;
+		d.out_stride_y = o.stride_y;
+		d.out_stride_uv = o.stride_uv;
+		d.out_y = o.y;
+		d.out_u = o.u;
+		d.out_v = o.v;
 		if (kernel_mode == VP8_K_FILTER) {
-			d.src_y = b->d_pad + m.pad_off[0];
-			d.src_u = b->d_pad + m.pad_off[1];
-			d.src_v = b->d_pad + m.pad_off[2];
-			d.src_stride_y = pw;
-			d.src_stride_uv = pw / 2;
+			const PlaneView s = plane_view(b, m, false);
+			d.src_y = s.y;
+			d.src_u = s.u;
+			d.src_v = s.v;
+			d.src_stride_y = s.stride_y;
+			d.src_stride_uv = s.stride_uv;
 		}
 		const uint8_t* in = b->d_in;
 		d.coeff_y = (const int16_t*)(in + m.in_off[0]);
@@ -811,6 +898,30 @@ int plan_launch(const vp8_gpu_ctx* c, int n, int max_mb_cols, int max_rows, int 
 	return 0;
 }
 
+// Device-side timing of a launch, read by vp8_gpu_kernel_time / _rgb_time / _png_time: begin_timed takes an event pair
+// (a recycled one if there is one) and records its first event, end_timed records the second and files the pair.
+using TimedPair = std::pair<cudaEvent_t, cudaEvent_t>;
+int begin_timed(vp8_gpu_ctx* c, cudaStream_t st, TimedPair* ev) {
+	if (!c->spare.empty()) {
+		*ev = c->spare.back();
+		c->spare.pop_back();
+	} else {
+		CU(cudaEventCreate(&ev->first));
+		CU(cudaEventCreate(&ev->second));
+	}
+	CU(cudaEventRecord(ev->first, st));
+	return 0;
+}
+int end_timed(vp8_gpu_ctx* c, std::vector<TimedPair>& list, const TimedPair& ev, cudaStream_t st) {
+	CU(cudaEventRecord(ev.second, st));
+	list.push_back(ev);
+	if (list.size() > 4096) { // nobody is asking: recycle the oldest
+		c->spare.push_back(list.front());
+		list.erase(list.begin());
+	}
+	return 0;
+}
+
 int launch_wavefront(vp8_gpu_ctx* c, vp8_gpu_batch* b, int kernel_mode, int layout) {
 	if (push_descs(c, b, kernel_mode, layout)) return -1;
 	int max_rows = 0;
@@ -850,15 +961,8 @@ int launch_wavefront(vp8_gpu_ctx* c, vp8_gpu_batch* b, int kernel_mode, int layo
 		if (dev_alloc(c, need, (void**)&b->d_scratch)) return -1;
 		b->scratch_bytes = need;
 	}
-	std::pair<cudaEvent_t, cudaEvent_t> ev{nullptr, nullptr};
-	if (!c->spare.empty()) {
-		ev = c->spare.back();
-		c->spare.pop_back();
-	} else {
-		CU(cudaEventCreate(&ev.first));
-		CU(cudaEventCreate(&ev.second));
-	}
-	CU(cudaEventRecord(ev.first, b->stream));
+	TimedPair ev;
+	if (begin_timed(c, b->stream, &ev)) return -1;
 	int rc = 0;
 	for (auto& sg : segs) {
 		const LaunchPlan& p = sg.plan;
@@ -869,12 +973,7 @@ int launch_wavefront(vp8_gpu_ctx* c, vp8_gpu_batch* b, int kernel_mode, int layo
 		if (rc != 0) break;
 		c->launches++;
 	}
-	CU(cudaEventRecord(ev.second, b->stream));
-	c->timed.push_back(ev);
-	if (c->timed.size() > 4096) { // nobody is asking: recycle the oldest
-		c->spare.push_back(c->timed.front());
-		c->timed.erase(c->timed.begin());
-	}
+	if (end_timed(c, c->timed, ev, b->stream)) return -1;
 	if (rc != 0) return fail(EIO, "wavefront launch", (cudaError_t)rc);
 	const LaunchPlan& p = segs.front().plan; // what is reported: the shape of the first (biggest) segment
 	c->last_warps = p.warps;
@@ -886,8 +985,6 @@ int launch_wavefront(vp8_gpu_ctx* c, vp8_gpu_batch* b, int kernel_mode, int layo
 	c->last_smem = p.groups ? vp8_lockstep_smem_bytes(p.groups, b->max_mb_cols) : vp8_pairs_smem_bytes(p.warps, b->max_mb_cols);
 	return 0;
 }
-
-int ppm_header(char* buf, uint32_t w, uint32_t h) { return snprintf(buf, 32, "P6\n%u %u\n255\n", w, h); }
 
 // ------------------------------------------------------------------------------------------------ default context
 std::mutex g_default_mu;
@@ -916,7 +1013,24 @@ int write_all(int fd, const void* p, size_t n) {
 	return 0;
 }
 
-int png_tables_ready(vp8_gpu_ctx* c);
+// Checksum tables of the m09 kernels: one host copy for the process (descriptor heads are computed from it) ...
+const uint8_t* png_host_tables() {
+	static std::once_flag once;
+	static std::vector<uint8_t> t;
+	std::call_once(once, [] {
+		t.resize(vp8_png_tables_bytes());
+		vp8_png_tables(t.data());
+	});
+	return t.data();
+}
+
+// ... and one in device memory per context.
+int png_tables_ready(vp8_gpu_ctx* c) {
+	if (c->d_png_tables) return 0;
+	CU(cudaMalloc(&c->d_png_tables, vp8_png_tables_bytes()));
+	CU(cudaMemcpy(c->d_png_tables, png_host_tables(), vp8_png_tables_bytes(), cudaMemcpyHostToDevice));
+	return 0;
+}
 
 // RGB24 of a host I420 image through the device (m08 kernel only) - or, as_png, the -png file of it (m08 + m09 kernels).
 int rgb_of_host_image(vp8_gpu_ctx* c, const Yuv420Image* img, std::vector<uint8_t>& rgb, bool as_png = false) {
@@ -953,24 +1067,19 @@ int rgb_of_host_image(vp8_gpu_ctx* c, const Yuv420Image* img, std::vector<uint8_
 		else c->launches++;
 	}
 	if (!rc && as_png) {
-		if ((3 * (uint64_t)w + 1) * h > 0x7FFFFFFFull) rc = fail(EFBIG, "image too large for a single IDAT");
+		if (!png_fits(w, h)) rc = fail(EFBIG, "image too large for a single IDAT");
 		const size_t file_len = rc ? 0 : vp8_png_file_bytes(w, h), png_bytes = align_up(file_len), side = 256 + vp8_png_accum_bytes();
 		uint8_t *d_png = nullptr, *d_side = nullptr; // side block: descriptor, then the accumulators
 		if (!rc) rc = png_tables_ready(c);
 		if (!rc && (dev_alloc(c, png_bytes, (void**)&d_png) || dev_alloc(c, side, (void**)&d_side))) rc = -1;
 		if (!rc) {
-			static std::vector<uint8_t> tables;
-			if (tables.empty()) { // callers hold g_default_mu
-				tables.resize(vp8_png_tables_bytes());
-				vp8_png_tables(tables.data());
-			}
 			Vp8PngDesc pd;
 			memset(&pd, 0, sizeof(pd));
 			pd.rgb = d_rgb;
 			pd.out = d_png;
 			pd.width = w;
 			pd.height = h;
-			vp8_png_fill_desc(&pd, tables.data());
+			vp8_png_fill_desc(&pd, png_host_tables());
 			if (push_table(c, d_side, &pd, sizeof(pd), c->stream)) rc = -1;
 		}
 		if (!rc) {
@@ -1259,16 +1368,6 @@ int png_frame(const uint8_t* rgb, uint32_t w, uint32_t h, std::vector<uint8_t>& 
 	return 0;
 }
 
-// Checksum tables of the m09 kernels in device memory, once per context.
-int png_tables_ready(vp8_gpu_ctx* c) {
-	if (c->d_png_tables) return 0;
-	std::vector<uint8_t> t(vp8_png_tables_bytes());
-	vp8_png_tables(t.data());
-	CU(cudaMalloc(&c->d_png_tables, t.size()));
-	CU(cudaMemcpy(c->d_png_tables, t.data(), t.size(), cudaMemcpyHostToDevice));
-	return 0;
-}
-
 } // namespace
 
 // ================================================================================================ C-ABI: batch interface
@@ -1426,12 +1525,7 @@ int vp8_gpu_run(vp8_gpu_ctx* c, vp8_gpu_batch* b, int filtered, int layout) {
 	if (!b->have_coeffs) return fail(EINVAL, "batch holds no coefficients");
 	CU(cudaSetDevice(c->device));
 	if (ensure_planes(c, b, layout)) return -1;
-	// frames whose every macroblock has filter level 0 come out of m07 unchanged (vp8_loopfilter.c:220), so a
-	// batch made only of such frames takes the reconstruction-only kernel
-	bool any = false;
-	for (auto& m : b->meta) any |= m.any_filter;
-	const int mode = (filtered && any) ? VP8_K_RECON_FILTER : VP8_K_RECON;
-	if (launch_wavefront(c, b, mode, layout)) return -1;
+	if (launch_wavefront(c, b, wavefront_mode(b, filtered), layout)) return -1;
 	b->state = layout == VP8_GPU_TIGHT ? PLANES_TIGHT : PLANES_PADDED;
 	b->filtered = filtered != 0;
 	b->have_rgb = false;
@@ -1454,9 +1548,7 @@ int vp8_gpu_filter(vp8_gpu_ctx* c, vp8_gpu_batch* b) {
 	if (!c || !b) return fail(EINVAL, "bad arguments");
 	if (b->state != PLANES_PADDED || b->filtered) return fail(EINVAL, "vp8_gpu_filter needs unfiltered macroblock-aligned planes");
 	CU(cudaSetDevice(c->device));
-	bool any = false;
-	for (auto& m : b->meta) any |= m.any_filter;
-	if (any && launch_wavefront(c, b, VP8_K_FILTER, VP8_GPU_PADDED)) return -1;
+	if (wavefront_mode(b, true) == VP8_K_RECON_FILTER && launch_wavefront(c, b, VP8_K_FILTER, VP8_GPU_PADDED)) return -1;
 	b->filtered = true;
 	b->have_rgb = false;
 	return 0;
@@ -1474,20 +1566,12 @@ static int push_rgb_descs(vp8_gpu_ctx* c, vp8_gpu_batch* b, int state) {
 		memset(&d, 0, sizeof(d));
 		d.width = m.width;
 		d.height = m.height;
-		if (state == PLANES_TIGHT) {
-			const size_t cw = (m.width + 1) / 2, ch = (m.height + 1) / 2;
-			d.y = b->d_tight + m.tight_off;
-			d.u = d.y + (size_t)m.width * m.height;
-			d.v = d.u + cw * ch;
-			d.stride_y = m.width;
-			d.stride_uv = (uint32_t)cw;
-		} else {
-			d.y = b->d_pad + m.pad_off[0];
-			d.u = b->d_pad + m.pad_off[1];
-			d.v = b->d_pad + m.pad_off[2];
-			d.stride_y = m.mb_cols * 16;
-			d.stride_uv = m.mb_cols * 8;
-		}
+		const PlaneView p = plane_view(b, m, state == PLANES_TIGHT);
+		d.y = p.y;
+		d.u = p.u;
+		d.v = p.v;
+		d.stride_y = p.stride_y;
+		d.stride_uv = p.stride_uv;
 		d.rgb = b->d_rgb + m.rgb_off + kPpmSlot;
 	}
 	if (push_table(c, b->d_rgbdesc, h.data(), sizeof(Vp8RgbDesc) * b->n, b->stream)) return -1;
@@ -1502,9 +1586,7 @@ static int push_rgb_descs(vp8_gpu_ctx* c, vp8_gpu_batch* b, int state) {
 static int push_png_descs(vp8_gpu_ctx* c, vp8_gpu_batch* b);
 static int push_tables_ahead(vp8_gpu_ctx* c, vp8_gpu_batch* b, int filtered, int format) {
 	if (ensure_planes(c, b, VP8_GPU_TIGHT)) return -1;
-	bool any = false;
-	for (auto& m : b->meta) any |= m.any_filter;
-	if (push_descs(c, b, (filtered && any) ? VP8_K_RECON_FILTER : VP8_K_RECON, VP8_GPU_TIGHT)) return -1;
+	if (push_descs(c, b, wavefront_mode(b, filtered), VP8_GPU_TIGHT)) return -1;
 	if (format != VP8_GPU_OUT_I420 && push_rgb_descs(c, b, PLANES_TIGHT)) return -1;
 	return format == VP8_GPU_OUT_PNG ? push_png_descs(c, b) : 0;
 }
@@ -1516,22 +1598,10 @@ int vp8_gpu_rgb(vp8_gpu_ctx* c, vp8_gpu_batch* b) {
 	if (push_rgb_descs(c, b, b->state)) return -1;
 	std::vector<uint32_t> tiles(b->n);
 	for (int i = 0; i < b->n; i++) tiles[i] = vp8_rgb_tiles(b->meta[i].width, b->meta[i].height);
-	std::pair<cudaEvent_t, cudaEvent_t> ev{nullptr, nullptr};
-	if (!c->spare.empty()) {
-		ev = c->spare.back();
-		c->spare.pop_back();
-	} else {
-		CU(cudaEventCreate(&ev.first));
-		CU(cudaEventCreate(&ev.second));
-	}
-	CU(cudaEventRecord(ev.first, b->stream));
+	TimedPair ev;
+	if (begin_timed(c, b->stream, &ev)) return -1;
 	const int rc = vp8_launch_rgb(b->d_rgbdesc, b->n, tiles.data(), b->stream);
-	CU(cudaEventRecord(ev.second, b->stream));
-	c->timed_rgb.push_back(ev);
-	if (c->timed_rgb.size() > 4096) {
-		c->spare.push_back(c->timed_rgb.front());
-		c->timed_rgb.erase(c->timed_rgb.begin());
-	}
+	if (end_timed(c, c->timed_rgb, ev, b->stream)) return -1;
 	if (rc) return fail(EIO, "rgb launch", (cudaError_t)rc);
 	c->launches += (b->n + 65534) / 65535;
 	b->have_rgb = true;
@@ -1540,7 +1610,6 @@ int vp8_gpu_rgb(vp8_gpu_ctx* c, vp8_gpu_batch* b) {
 }
 
 // m09 on the device (vp8_png.cu): slot layout, work items and accumulators of the batch, sent on the batch's stream.
-static size_t png_slot_bytes(size_t w, size_t h) { return align_up(vp8_png_file_bytes((uint32_t)w, (uint32_t)h)); }
 static int png_layout(vp8_gpu_batch* b) {
 	if (!b->png_off.empty()) return 0;
 	size_t off = 0;
@@ -1548,12 +1617,12 @@ static int png_layout(vp8_gpu_batch* b) {
 	b->png_off.resize(b->n);
 	for (int i = 0; i < b->n; i++) {
 		const FrameMeta& m = b->meta[i];
-		if ((3 * (uint64_t)m.width + 1) * m.height > 0x7FFFFFFFull) {
+		if (!png_fits(m.width, m.height)) {
 			b->png_off.clear();
 			return fail(EFBIG, "image too large for a single IDAT");
 		}
 		b->png_off[i] = off;
-		off += png_slot_bytes(m.width, m.height);
+		off += out_slot_bytes(m.width, m.height, VP8_GPU_OUT_PNG);
 		ctas += vp8_png_ctas(m.width, m.height);
 	}
 	if (ctas > 0x7FFFFFFFull) {
@@ -1572,12 +1641,6 @@ static int push_png_descs(vp8_gpu_ctx* c, vp8_gpu_batch* b) {
 	if (!b->d_pngdesc && dev_alloc(c, sizeof(Vp8PngDesc) * b->n, (void**)&b->d_pngdesc)) return -1;
 	if (!b->d_pngacc && dev_alloc(c, vp8_png_accum_bytes() * b->n, &b->d_pngacc)) return -1;
 	if (b->pngdesc_up) return 0;
-	static std::once_flag once;
-	static std::vector<uint8_t> host_tables;
-	std::call_once(once, [] {
-		host_tables.resize(vp8_png_tables_bytes());
-		vp8_png_tables(host_tables.data());
-	});
 	std::vector<Vp8PngDesc> h(b->n);
 	uint32_t first = 0;
 	for (int i = 0; i < b->n; i++) {
@@ -1595,7 +1658,7 @@ static int push_png_descs(vp8_gpu_ctx* c, vp8_gpu_batch* b) {
 			memcpy(d.head, h[i - 1].head, sizeof(d.head));
 			d.crc_init = h[i - 1].crc_init;
 		} else {
-			vp8_png_fill_desc(&d, host_tables.data());
+			vp8_png_fill_desc(&d, png_host_tables());
 		}
 	}
 	if (push_table(c, b->d_pngdesc, h.data(), sizeof(Vp8PngDesc) * b->n, b->stream)) return -1;
@@ -1608,22 +1671,10 @@ int vp8_gpu_png(vp8_gpu_ctx* c, vp8_gpu_batch* b) {
 	if (!b->have_rgb) return fail(EINVAL, "run vp8_gpu_rgb first");
 	CU(cudaSetDevice(c->device));
 	if (push_png_descs(c, b)) return -1;
-	std::pair<cudaEvent_t, cudaEvent_t> ev{nullptr, nullptr};
-	if (!c->spare.empty()) {
-		ev = c->spare.back();
-		c->spare.pop_back();
-	} else {
-		CU(cudaEventCreate(&ev.first));
-		CU(cudaEventCreate(&ev.second));
-	}
-	CU(cudaEventRecord(ev.first, b->stream));
+	TimedPair ev;
+	if (begin_timed(c, b->stream, &ev)) return -1;
 	const int rc = vp8_launch_png(b->d_pngdesc, b->n, b->png_ctas, c->d_png_tables, b->d_pngacc, b->stream);
-	CU(cudaEventRecord(ev.second, b->stream));
-	c->timed_png.push_back(ev);
-	if (c->timed_png.size() > 4096) {
-		c->spare.push_back(c->timed_png.front());
-		c->timed_png.erase(c->timed_png.begin());
-	}
+	if (end_timed(c, c->timed_png, ev, b->stream)) return -1;
 	if (rc) return fail(EIO, "png launch", (cudaError_t)rc);
 	c->launches += 2;
 	b->have_png = true;
@@ -1635,16 +1686,7 @@ size_t vp8_gpu_png_bytes(vp8_gpu_batch* b) { return b && !png_layout(b) ? b->png
 int vp8_gpu_download_png(vp8_gpu_ctx* c, vp8_gpu_batch* b, uint8_t* dst, size_t cap, size_t* offsets, size_t* sizes) {
 	if (!c || !b || !dst) return fail(EINVAL, "bad arguments");
 	if (!b->have_png) return fail(EINVAL, "run vp8_gpu_png first");
-	if (cap < b->png_bytes) return fail(EINVAL, "destination too small");
-	CU(cudaSetDevice(c->device));
-	const FrameMeta& last = b->meta.back();
-	const size_t used = b->png_off.back() + vp8_png_file_bytes(last.width, last.height);
-	if (download(c, b->stream, dst, b->d_png, used)) return -1;
-	for (int i = 0; i < b->n; i++) {
-		if (offsets) offsets[i] = b->png_off[i];
-		if (sizes) sizes[i] = vp8_png_file_bytes(b->meta[i].width, b->meta[i].height);
-	}
-	return 0;
+	return download_out(c, b, VP8_GPU_OUT_PNG, dst, cap, offsets, sizes);
 }
 
 size_t vp8_gpu_i420_bytes(const vp8_gpu_batch* b) { return b ? b->tight_bytes : 0; }
@@ -1654,36 +1696,13 @@ int vp8_gpu_batch_size(const vp8_gpu_batch* b) { return b ? b->n : 0; }
 int vp8_gpu_download_i420(vp8_gpu_ctx* c, vp8_gpu_batch* b, uint8_t* dst, size_t cap, size_t* offsets, size_t* sizes) {
 	if (!c || !b || !dst) return fail(EINVAL, "bad arguments");
 	if (b->state != PLANES_TIGHT) return fail(EINVAL, "tight planes required (vp8_gpu_run with VP8_GPU_TIGHT)");
-	if (cap < b->tight_bytes) return fail(EINVAL, "destination too small");
-	CU(cudaSetDevice(c->device));
-	const FrameMeta& last = b->meta.back();
-	const size_t used = last.tight_off + (size_t)last.width * last.height + 2 * (size_t)((last.width + 1) / 2) * ((last.height + 1) / 2);
-	if (download(c, b->stream, dst, b->d_tight, used)) return -1;
-	for (int i = 0; i < b->n; i++) {
-		const FrameMeta& m = b->meta[i];
-		if (offsets) offsets[i] = m.tight_off;
-		if (sizes) sizes[i] = (size_t)m.width * m.height + 2 * (size_t)((m.width + 1) / 2) * ((m.height + 1) / 2);
-	}
-	return 0;
+	return download_out(c, b, VP8_GPU_OUT_I420, dst, cap, offsets, sizes);
 }
 
 int vp8_gpu_download_ppm(vp8_gpu_ctx* c, vp8_gpu_batch* b, uint8_t* dst, size_t cap, size_t* offsets, size_t* sizes) {
 	if (!c || !b || !dst) return fail(EINVAL, "bad arguments");
 	if (!b->have_rgb) return fail(EINVAL, "run vp8_gpu_rgb first");
-	if (cap < b->rgb_bytes) return fail(EINVAL, "destination too small");
-	CU(cudaSetDevice(c->device));
-	const FrameMeta& last = b->meta.back();
-	const size_t used = last.rgb_off + kPpmSlot + (size_t)last.width * last.height * 3;
-	if (download(c, b->stream, dst, b->d_rgb, used)) return -1;
-	for (int i = 0; i < b->n; i++) {
-		const FrameMeta& m = b->meta[i];
-		char hdr[32];
-		const int hl = ppm_header(hdr, m.width, m.height);
-		memcpy(dst + m.rgb_off + kPpmSlot - hl, hdr, hl);
-		if (offsets) offsets[i] = m.rgb_off + kPpmSlot - hl;
-		if (sizes) sizes[i] = hl + (size_t)m.width * m.height * 3;
-	}
-	return 0;
+	return download_out(c, b, VP8_GPU_OUT_PPM, dst, cap, offsets, sizes);
 }
 
 int vp8_gpu_download_padded(vp8_gpu_ctx* c, vp8_gpu_batch* b, int i, uint8_t* y, uint8_t* u, uint8_t* v) {
@@ -1861,35 +1880,6 @@ struct FrameGeom {
 	uint32_t width, height;
 };
 
-// Shell of a batch whose input arena holds compact frames: geometry, output layout, nothing uploaded yet.
-vp8_gpu_batch* compact_batch_shell(const FrameGeom* g, int n, cudaStream_t st) {
-	vp8_gpu_batch* b = new (std::nothrow) vp8_gpu_batch;
-	if (!b) return nullptr;
-	b->n = n;
-	b->stream = st;
-	b->meta.resize(n);
-	size_t tight = 0, rgb = 0;
-	for (int i = 0; i < n; i++) {
-		FrameMeta& m = b->meta[i];
-		m.width = g[i].width;
-		m.height = g[i].height;
-		m.mb_cols = (m.width + 15) / 16;
-		m.mb_rows = (m.height + 15) / 16;
-		m.compact = true;
-		const size_t cw = (m.width + 1) / 2, ch = (m.height + 1) / 2;
-		m.tight_off = tight;
-		tight += align_up((size_t)m.width * m.height + 2 * cw * ch);
-		m.pad_off[0] = m.pad_off[1] = m.pad_off[2] = 0;
-		m.rgb_off = rgb;
-		rgb += align_up(kPpmSlot + (size_t)m.width * m.height * 3);
-		b->max_mb_cols = std::max<int>(b->max_mb_cols, m.mb_cols);
-	}
-	b->tight_bytes = tight;
-	b->pad_bytes = 0;
-	b->rgb_bytes = rgb;
-	return b;
-}
-
 // Per-frame parameters of a compact batch entry from the frame's scalars; head / packed = offsets inside the device arena.
 void compact_meta(FrameMeta& m, const Vp8DecodedFrame* f, size_t head, size_t packed) {
 	const vp8c::Layout L = vp8c::layout((size_t)m.mb_cols * m.mb_rows);
@@ -1904,11 +1894,7 @@ void compact_meta(FrameMeta& m, const Vp8DecodedFrame* f, size_t head, size_t pa
 	m.in_off[6] = head + L.o_uv;
 	m.in_off[7] = head + L.o_seg;
 	m.in_off[8] = head + L.o_hc;
-	frame_params(f, m.dq, m.lf);
-	m.lf_simple = f->lf_use_simple;
-	m.any_filter = false;
-	for (int s = 0; s < (m.has_seg ? 4 : 1); s++)
-		for (int k = 0; k < 2; k++) m.any_filter |= m.lf[s][k][0] != 0;
+	frame_setup(m, f);
 }
 
 int stage_reserve(vp8_gpu_ctx* c, int slot, size_t bytes) {
@@ -1941,6 +1927,59 @@ void pool_run(vp8_gpu_ctx* c, int threads, const std::function<void()>& work) {
 	else work();
 }
 
+// The part of a compact chunk that does not depend on its producer. The batch's device arena takes in_bytes, the compact
+// frames the first `packed` of them (their blocks are counted with 32-bit indices). Then, in this order:
+//   queue(b): batch entries that need no host pass, and copies straight from the caller's memory - queued first, so that
+//             the copy engine works on them while the host threads fill the staging slot;
+//   fill(b, stage, &used): when `staged`, the host pass that writes the compact frames into the pinned staging slot
+//             (counted as host work); the `used` bytes then cross as one transfer.
+// Either returns -1 with errno set on failure, and the batch is destroyed.
+int compact_chunk(vp8_gpu_ctx* c, const FrameGeom* g, int n, size_t packed, size_t in_bytes, bool staged, int slot, cudaStream_t st,
+                  const std::function<int(vp8_gpu_batch*)>& queue, const std::function<int(vp8_gpu_batch*, uint8_t*, size_t*)>& fill,
+                  vp8_gpu_batch** out) {
+	if (packed / 32 > 0xffffffffull) return fail(EINVAL, "compact chunk exceeds the 32-bit block index; use a smaller chunk");
+	vp8_gpu_batch* b = new (std::nothrow) vp8_gpu_batch;
+	if (!b) return fail(ENOMEM, "batch");
+	b->n = n;
+	b->stream = st;
+	b->meta.resize(n);
+	for (int i = 0; i < n; i++) {
+		FrameMeta& m = b->meta[i];
+		m.width = g[i].width;
+		m.height = g[i].height;
+		m.mb_cols = (m.width + 15) / 16;
+		m.mb_rows = (m.height + 15) / 16;
+		m.compact = true;
+		m.pad_off[0] = m.pad_off[1] = m.pad_off[2] = 0;
+	}
+	out_layout(b);
+	b->in_bytes = in_bytes;
+	staged = staged && packed;
+	int rc = 0;
+	if ((staged && stage_reserve(c, slot, packed)) || dev_alloc(c, in_bytes, (void**)&b->d_in) || dev_alloc(c, sizeof(Vp8ImgDesc) * n, (void**)&b->d_desc))
+		rc = -1;
+	if (!rc && queue) rc = queue(b);
+	if (!rc && staged) {
+		const auto t_c0 = std::chrono::steady_clock::now();
+		size_t used = 0;
+		rc = fill(b, c->cstage[slot], &used);
+		c->trace_compact_ms += std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_c0).count();
+		if (!rc) {
+			const cudaError_t e = cudaMemcpyAsync(b->d_in, c->cstage[slot], used, cudaMemcpyHostToDevice, st);
+			if (e != cudaSuccess) rc = fail(EIO, "compact chunk upload", e);
+			else c->h2d += used;
+		}
+	}
+	if (rc) {
+		const int saved = errno;
+		batch_destroy(c, b);
+		errno = saved;
+		return -1;
+	}
+	*out = b;
+	return 0;
+}
+
 // A dense frame whose arrays sit in ONE pinned block (vp8_parse arenas mark theirs) and whose blocks are mostly non-zero gains
 // nothing from compaction - the host would read 6.7 MB (1080p) to write nearly as much - so it is handed to the copy engine
 // as it is and the kernel reads it through the dense layout (Vp8ImgDesc::compact = 0 for that image; a chunk may mix).
@@ -1948,12 +1987,10 @@ void pool_run(vp8_gpu_ctx* c, int threads, const std::function<void()>& work) {
 bool dense_passthrough(const Vp8DecodedFrame* f, const uint8_t** lo_out, size_t* bytes_out) {
 	if (f->stats_opaque[21] != kArenaMagic) return false;
 	const size_t mb = (size_t)f->mb_cols * f->mb_rows;
-	const uint8_t* src[9] = {(const uint8_t*)f->coeff_y, (const uint8_t*)f->coeff_u, (const uint8_t*)f->coeff_v, (const uint8_t*)f->coeff_y2,
-	                         f->bmode, f->ymode, f->uv_mode, f->segmentation_enabled ? f->segment_id : nullptr, f->has_coeff};
-	const size_t sz[9] = {mb * 512, mb * 128, mb * 128, mb * 32, mb * 16, mb, mb, mb, mb};
+	const auto [src, sz] = dense_arrays(f, true, f->segmentation_enabled && f->segment_id);
 	const uint8_t *lo = nullptr, *hi = nullptr;
 	for (int k = 0; k < 9; k++) {
-		if (!src[k]) continue;
+		if (!sz[k]) continue;
 		if (!lo || src[k] < lo) lo = src[k];
 		if (!hi || src[k] + sz[k] > hi) hi = src[k] + sz[k];
 	}
@@ -2002,72 +2039,49 @@ int batch_create_compact(vp8_gpu_ctx* c, const Vp8KeyFrameHeader* const* kf, con
 		todo.push_back(i);
 		in += vp8c::shared_bound((size_t)fr[i]->mb_cols * fr[i]->mb_rows);
 	}
-	if (in / 32 > 0xffffffffull) return fail(EINVAL, "compact chunk exceeds the 32-bit block index; use a smaller chunk");
-	const size_t stage_bytes = in;
+	const size_t packed = in;
 	for (int i = 0; i < n; i++)
 		if (span[i].lo) {
 			span[i].off = align_up(in);
 			in = span[i].off + span[i].bytes;
 		}
-	vp8_gpu_batch* b = compact_batch_shell(g.data(), n, st);
-	if (!b) return fail(ENOMEM, "batch");
-	b->in_bytes = align_up(in);
-	if ((stage_bytes && stage_reserve(c, slot, stage_bytes)) || dev_alloc(c, b->in_bytes, (void**)&b->d_in) ||
-	    dev_alloc(c, sizeof(Vp8ImgDesc) * n, (void**)&b->d_desc)) {
-		batch_destroy(c, b);
-		return -1;
-	}
-	// the pass-through frames first: the copy engine works on them while the host threads compact the others
-	for (int i = 0; i < n; i++) {
-		if (!span[i].lo) continue;
-		const Vp8DecodedFrame* f = fr[i];
-		FrameMeta& m = b->meta[i];
-		m.compact = false;
-		m.has_seg = f->segmentation_enabled && f->segment_id;
-		m.has_hc = f->has_coeff != nullptr;
-		const uint8_t* src[9] = {(const uint8_t*)f->coeff_y, (const uint8_t*)f->coeff_u, (const uint8_t*)f->coeff_v, (const uint8_t*)f->coeff_y2,
-		                         f->bmode, f->ymode, f->uv_mode, m.has_seg ? f->segment_id : nullptr, f->has_coeff};
-		for (int k = 0; k < 9; k++) m.in_off[k] = span[i].off + (src[k] ? (size_t)(src[k] - span[i].lo) : 0);
-		frame_params(f, m.dq, m.lf);
-		m.lf_simple = f->lf_use_simple;
-		m.any_filter = false;
-		for (int s2 = 0; s2 < (m.has_seg ? 4 : 1); s2++)
-			for (int k = 0; k < 2; k++) m.any_filter |= m.lf[s2][k][0] != 0;
-		cudaError_t e = cudaMemcpyAsync(b->d_in + span[i].off, span[i].lo, span[i].bytes, cudaMemcpyHostToDevice, st);
-		if (e != cudaSuccess) {
-			batch_destroy(c, b);
-			return fail(EIO, "dense frame upload", e);
-		}
-		c->h2d += span[i].bytes;
-		c->trace_dense_frames++;
-	}
-	if (!todo.empty()) {
-		const auto t_c0 = std::chrono::steady_clock::now();
-		uint8_t* stage = c->cstage[slot];
-		std::atomic<size_t> cursor{0};
-		std::atomic<int> next{0};
-		const int nt = (int)todo.size();
-		const int threads = pool_threads(c, nt);
-		pool_run(c, threads, [&]() {
-			for (int k; (k = next.fetch_add(1)) < nt;) {
-				const int i = todo[k];
-				const size_t head = compact_frame(fr[i], stage, cursor);
-				compact_meta(b->meta[i], fr[i], head, 0);
-				b->meta[i].has_seg = fr[i]->segmentation_enabled && fr[i]->segment_id;
-				b->meta[i].has_hc = fr[i]->has_coeff != nullptr;
-			}
-		});
-		c->trace_compact_ms += std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_c0).count();
-		const size_t used = cursor.load();
-		cudaError_t e = cudaMemcpyAsync(b->d_in, stage, used, cudaMemcpyHostToDevice, st);
-		if (e != cudaSuccess) {
-			batch_destroy(c, b);
-			return fail(EIO, "compact chunk upload", e);
-		}
-		c->h2d += used;
-	}
-	*out = b;
-	return 0;
+	return compact_chunk(
+	    c, g.data(), n, packed, align_up(in), true, slot, st,
+	    [&](vp8_gpu_batch* b) { // the pass-through frames
+		    for (int i = 0; i < n; i++) {
+			    if (!span[i].lo) continue;
+			    const Vp8DecodedFrame* f = fr[i];
+			    FrameMeta& m = b->meta[i];
+			    m.compact = false;
+			    m.has_seg = f->segmentation_enabled && f->segment_id;
+			    m.has_hc = f->has_coeff != nullptr;
+			    const auto [src, sz] = dense_arrays(f, true, m.has_seg);
+			    for (int k = 0; k < 9; k++) m.in_off[k] = span[i].off + (sz[k] ? (size_t)(src[k] - span[i].lo) : 0);
+			    frame_setup(m, f);
+			    cudaError_t e = cudaMemcpyAsync(b->d_in + span[i].off, span[i].lo, span[i].bytes, cudaMemcpyHostToDevice, st);
+			    if (e != cudaSuccess) return fail(EIO, "dense frame upload", e);
+			    c->h2d += span[i].bytes;
+			    c->trace_dense_frames++;
+		    }
+		    return 0;
+	    },
+	    [&](vp8_gpu_batch* b, uint8_t* stage, size_t* used) {
+		    std::atomic<size_t> cursor{0};
+		    std::atomic<int> next{0};
+		    const int nt = (int)todo.size();
+		    pool_run(c, pool_threads(c, nt), [&]() {
+			    for (int k; (k = next.fetch_add(1)) < nt;) {
+				    const int i = todo[k];
+				    const size_t head = compact_frame(fr[i], stage, cursor);
+				    compact_meta(b->meta[i], fr[i], head, 0);
+				    b->meta[i].has_seg = fr[i]->segmentation_enabled && fr[i]->segment_id;
+				    b->meta[i].has_hc = fr[i]->has_coeff != nullptr;
+			    }
+		    });
+		    *used = cursor.load();
+		    return 0;
+	    },
+	    out);
 }
 
 int validate_compact(const Vp8CompactFrame* f) {
@@ -2094,46 +2108,31 @@ int batch_create_precompact(vp8_gpu_ctx* c, const Vp8CompactFrame* const* fr, in
 		const uint8_t* p = fr[i]->base + fr[i]->head_off;
 		direct = direct && is_pinned(p) && is_pinned(p + fr[i]->bytes - 1);
 	}
-	const size_t in = off[n];
-	if (in / 32 > 0xffffffffull) return fail(EINVAL, "compact chunk exceeds the 32-bit block index; use a smaller chunk");
-	vp8_gpu_batch* b = compact_batch_shell(g.data(), n, st);
-	if (!b) return fail(ENOMEM, "batch");
-	b->in_bytes = in;
-	if ((!direct && stage_reserve(c, slot, in)) || dev_alloc(c, in, (void**)&b->d_in) || dev_alloc(c, sizeof(Vp8ImgDesc) * n, (void**)&b->d_desc)) {
-		batch_destroy(c, b);
-		return -1;
-	}
-	for (int i = 0; i < n; i++) compact_meta(b->meta[i], &fr[i]->f, off[i], off[i] + vp8c::layout((size_t)fr[i]->f.mb_cols * fr[i]->f.mb_rows).o_packed);
-	cudaError_t e = cudaSuccess;
-	if (direct) {
-		for (int i = 0; i < n && e == cudaSuccess;) {
-			const uint8_t* src = fr[i]->base + fr[i]->head_off;
-			int j = i + 1;
-			while (j < n && fr[j]->base + fr[j]->head_off == src + (off[j] - off[i])) j++;
-			const size_t bytes = off[j - 1] - off[i] + fr[j - 1]->bytes;
-			e = cudaMemcpyAsync(b->d_in + off[i], src, bytes, cudaMemcpyHostToDevice, st);
-			c->h2d += bytes;
-			i = j;
-		}
-	} else {
-		const auto t_c0 = std::chrono::steady_clock::now();
-		uint8_t* stage = c->cstage[slot];
-		std::atomic<int> next{0};
-		const int threads = pool_threads(c, n);
-		pool_run(c, threads, [&]() {
-			for (int i; (i = next.fetch_add(1)) < n;) memcpy(stage + off[i], fr[i]->base + fr[i]->head_off, fr[i]->bytes);
-		});
-		c->trace_compact_ms += std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_c0).count();
-		const size_t used = off[n - 1] + fr[n - 1]->bytes;
-		e = cudaMemcpyAsync(b->d_in, stage, used, cudaMemcpyHostToDevice, st);
-		c->h2d += used;
-	}
-	if (e != cudaSuccess) {
-		batch_destroy(c, b);
-		return fail(EIO, "compact chunk upload", e);
-	}
-	*out = b;
-	return 0;
+	return compact_chunk(
+	    c, g.data(), n, off[n], off[n], !direct, slot, st,
+	    [&](vp8_gpu_batch* b) {
+		    for (int i = 0; i < n; i++) compact_meta(b->meta[i], &fr[i]->f, off[i], off[i] + vp8c::layout((size_t)fr[i]->f.mb_cols * fr[i]->f.mb_rows).o_packed);
+		    for (int i = 0; direct && i < n;) {
+			    const uint8_t* src = fr[i]->base + fr[i]->head_off;
+			    int j = i + 1;
+			    while (j < n && fr[j]->base + fr[j]->head_off == src + (off[j] - off[i])) j++;
+			    const size_t bytes = off[j - 1] - off[i] + fr[j - 1]->bytes;
+			    const cudaError_t e = cudaMemcpyAsync(b->d_in + off[i], src, bytes, cudaMemcpyHostToDevice, st);
+			    if (e != cudaSuccess) return fail(EIO, "compact chunk upload", e);
+			    c->h2d += bytes;
+			    i = j;
+		    }
+		    return 0;
+	    },
+	    [&](vp8_gpu_batch*, uint8_t* stage, size_t* used) {
+		    std::atomic<int> next{0};
+		    pool_run(c, pool_threads(c, n), [&]() {
+			    for (int i; (i = next.fetch_add(1)) < n;) memcpy(stage + off[i], fr[i]->base + fr[i]->head_off, fr[i]->bytes);
+		    });
+		    *used = off[n - 1] + fr[n - 1]->bytes;
+		    return 0;
+	    },
+	    out);
 }
 
 // (c) .webp bytes in: the worker threads parse straight into the pinned staging slot (one image per thread at a time).
@@ -2141,50 +2140,34 @@ int batch_create_webp(vp8_gpu_ctx* c, const uint8_t* const* files, const size_t*
                       vp8_gpu_batch** out) {
 	size_t in = 0;
 	for (int i = 0; i < n; i++) in += vp8c::shared_bound((size_t)((g[i].width + 15) / 16) * ((g[i].height + 15) / 16));
-	if (in / 32 > 0xffffffffull) return fail(EINVAL, "compact chunk exceeds the 32-bit block index; use a smaller chunk");
-	vp8_gpu_batch* b = compact_batch_shell(g, n, st);
-	if (!b) return fail(ENOMEM, "batch");
-	b->in_bytes = in;
-	if (stage_reserve(c, slot, in) || dev_alloc(c, in, (void**)&b->d_in) || dev_alloc(c, sizeof(Vp8ImgDesc) * n, (void**)&b->d_desc)) {
-		batch_destroy(c, b);
-		return -1;
-	}
-	const auto t_c0 = std::chrono::steady_clock::now();
-	uint8_t* stage = c->cstage[slot];
-	std::atomic<size_t> cursor{0};
-	std::atomic<int> next{0}, bad{0}, bad_errno{0};
-	const int threads = pool_threads(c, n);
-	// parse time goes with the file size and differs by two orders of magnitude between files: longest first, so that the
-	// chunk does not end with one thread on a big file and the others idle
-	std::vector<int> order(n);
-	for (int i = 0; i < n; i++) order[i] = i;
-	std::stable_sort(order.begin(), order.end(), [&](int a, int b2) { return sizes[a] > sizes[b2]; });
-	pool_run(c, threads, [&]() {
-		for (int k; (k = next.fetch_add(1)) < n;) {
-			const int i = order[k];
-			Vp8KeyFrameHeader kf;
-			Vp8CompactFrame cf;
-			if (vp8_parse_webp_shared(files[i], sizes[i], &kf, &cf, stage, in, &cursor) || kf.width != g[i].width || kf.height != g[i].height) {
-				if (!bad.fetch_add(1)) bad_errno = errno ? errno : EINVAL;
-				continue;
-			}
-			compact_meta(b->meta[i], &cf.f, cf.head_off, cf.packed_off);
-		}
-	});
-	c->trace_compact_ms += std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_c0).count();
-	if (bad.load()) {
-		batch_destroy(c, b);
-		return fail(bad_errno.load(), "a .webp file of the chunk failed to parse");
-	}
-	const size_t used = cursor.load();
-	cudaError_t e = cudaMemcpyAsync(b->d_in, stage, used, cudaMemcpyHostToDevice, st);
-	if (e != cudaSuccess) {
-		batch_destroy(c, b);
-		return fail(EIO, "compact chunk upload", e);
-	}
-	c->h2d += used;
-	*out = b;
-	return 0;
+	return compact_chunk(
+	    c, g, n, in, in, true, slot, st, nullptr,
+	    [&](vp8_gpu_batch* b, uint8_t* stage, size_t* used) {
+		    std::atomic<size_t> cursor{0};
+		    std::atomic<int> next{0}, bad{0}, bad_errno{0};
+		    const int threads = pool_threads(c, n);
+		    // parse time goes with the file size and differs by two orders of magnitude between files: longest first, so that the
+		    // chunk does not end with one thread on a big file and the others idle
+		    std::vector<int> order(n);
+		    for (int i = 0; i < n; i++) order[i] = i;
+		    std::stable_sort(order.begin(), order.end(), [&](int a, int b2) { return sizes[a] > sizes[b2]; });
+		    pool_run(c, threads, [&]() {
+			    for (int k; (k = next.fetch_add(1)) < n;) {
+				    const int i = order[k];
+				    Vp8KeyFrameHeader kf;
+				    Vp8CompactFrame cf;
+				    if (vp8_parse_webp_shared(files[i], sizes[i], &kf, &cf, stage, in, &cursor) || kf.width != g[i].width || kf.height != g[i].height) {
+					    if (!bad.fetch_add(1)) bad_errno = errno ? errno : EINVAL;
+					    continue;
+				    }
+				    compact_meta(b->meta[i], &cf.f, cf.head_off, cf.packed_off);
+			    }
+		    });
+		    if (bad.load()) return fail(bad_errno.load(), "a .webp file of the chunk failed to parse");
+		    *used = cursor.load();
+		    return 0;
+	    },
+	    out);
 }
 
 // Chunked pipeline: chunk k's host->device copies, kernels and device->host copy run on internal streams, so the
@@ -2195,18 +2178,13 @@ int batch_create_webp(vp8_gpu_ctx* c, const uint8_t* const* files, const size_t*
 using ChunkMaker = std::function<int(int, int, int, cudaStream_t, bool, vp8_gpu_batch**)>;
 
 static int out_format(int ppm) { return ppm == VP8_GPU_OUT_PNG ? VP8_GPU_OUT_PNG : ppm ? VP8_GPU_OUT_PPM : VP8_GPU_OUT_I420; }
-static size_t out_slot_bytes(size_t w, size_t h, int format) {
-	return format == VP8_GPU_OUT_PNG   ? png_slot_bytes(w, h)
-	       : format == VP8_GPU_OUT_PPM ? align_up(kPpmSlot + w * h * 3)
-	                                   : align_up(w * h + 2 * ((w + 1) / 2) * ((h + 1) / 2));
-}
 
 static int decode_pipelined(vp8_gpu_ctx* c, const FrameGeom* geom, int n, const ChunkMaker& make_chunk, int filtered, int format,
                             uint8_t* dst, size_t cap, size_t* offsets, size_t* sizes, int chunk, bool ramp = true) {
 	const bool want_ppm = format == VP8_GPU_OUT_PPM, want_png = format == VP8_GPU_OUT_PNG;
 	if (want_png)
 		for (int i = 0; i < n; i++)
-			if ((3 * (uint64_t)geom[i].width + 1) * geom[i].height > 0x7FFFFFFFull) return fail(EFBIG, "image too large for a single IDAT");
+			if (!png_fits(geom[i].width, geom[i].height)) return fail(EFBIG, "image too large for a single IDAT");
 	CU(cudaSetDevice(c->device));
 	if (chunk <= 0) chunk = 64;
 	// global layout
@@ -2304,17 +2282,8 @@ static int decode_pipelined(vp8_gpu_ctx* c, const FrameGeom* geom, int n, const 
 			rc = fail(EIO, "pipeline events", cudaGetLastError());
 			break;
 		}
-		const FrameMeta& last = b->meta.back();
-		if (want_png) {
-			const size_t used = b->png_off.back() + vp8_png_file_bytes(last.width, last.height);
-			rc = download(c, s_down, dst + off[first], b->d_png, used, false);
-		} else if (want_ppm) {
-			const size_t used = last.rgb_off + kPpmSlot + (size_t)last.width * last.height * 3;
-			rc = download(c, s_down, dst + off[first], b->d_rgb, used, false);
-		} else {
-			const size_t used = last.tight_off + (size_t)last.width * last.height + 2 * (size_t)((last.width + 1) / 2) * ((last.height + 1) / 2);
-			rc = download(c, s_down, dst + off[first], b->d_tight, used, false);
-		}
+		const OutArena a = out_arena(b, format);
+		rc = download(c, s_down, dst + off[first], a.dev, a.used, false);
 		if (!rc && cudaEventRecord(ch.done, s_down) != cudaSuccess) rc = fail(EIO, "pipeline events", cudaGetLastError());
 		mark(s_down);
 	}
@@ -2350,22 +2319,7 @@ static int decode_pipelined(vp8_gpu_ctx* c, const FrameGeom* geom, int n, const 
 		errno = saved;
 		return -1;
 	}
-	for (int i = 0; i < n; i++) {
-		const size_t w = geom[i].width, h = geom[i].height;
-		if (want_ppm) {
-			char hdr[32];
-			const int hl = ppm_header(hdr, (uint32_t)w, (uint32_t)h);
-			memcpy(dst + off[i] + kPpmSlot - hl, hdr, hl);
-			if (offsets) offsets[i] = off[i] + kPpmSlot - hl;
-			if (sizes) sizes[i] = hl + w * h * 3;
-		} else if (want_png) {
-			if (offsets) offsets[i] = off[i];
-			if (sizes) sizes[i] = vp8_png_file_bytes((uint32_t)w, (uint32_t)h);
-		} else {
-			if (offsets) offsets[i] = off[i];
-			if (sizes) sizes[i] = w * h + 2 * ((w + 1) / 2) * ((h + 1) / 2);
-		}
-	}
+	for (int i = 0; i < n; i++) report_slot(dst, off[i], geom[i].width, geom[i].height, format, i, offsets, sizes);
 	return 0;
 }
 
@@ -2506,7 +2460,7 @@ size_t vp8_gpu_decode_webp_bytes(const uint8_t* const* files, const size_t* file
 	for (int i = 0; files && file_sizes && i < n; i++) {
 		uint32_t w = 0, h = 0;
 		if (vp8_parse_webp_size(files[i], file_sizes[i], &w, &h)) return 0;
-		if (ppm == VP8_GPU_OUT_PNG && !((3 * (uint64_t)w + 1) * h <= 0x7FFFFFFFull)) return 0;
+		if (ppm == VP8_GPU_OUT_PNG && !png_fits(w, h)) return 0;
 		total += out_slot_bytes(w, h, out_format(ppm));
 	}
 	return total;
@@ -2593,7 +2547,7 @@ size_t vp8_gpu_decode_bytes(const Vp8KeyFrameHeader* const* kf, int n, int ppm) 
 	size_t total = 0;
 	for (int i = 0; kf && i < n; i++) {
 		const size_t w = kf[i]->width, h = kf[i]->height;
-		if (ppm == VP8_GPU_OUT_PNG && !((3 * (uint64_t)w + 1) * h <= 0x7FFFFFFFull)) return 0;
+		if (ppm == VP8_GPU_OUT_PNG && !png_fits(w, h)) return 0;
 		total += out_slot_bytes(w, h, out_format(ppm));
 	}
 	return total;

@@ -152,6 +152,23 @@ __device__ __forceinline__ bool planes_wide_ok(const Vp8ImgDesc* sd) {
 	return (a & 15) == 0 && (sd->out_w & 31) == 0 && sd->out_w == 16 * sd->mb_cols;
 }
 
+// B_PRED lane table: btab[half][mode 0..10][pixel] = lane(a) | lane(b)<<8 | lane(c)<<16 | kind<<24, written by threads
+// first, first + stride, ...
+__device__ __forceinline__ void fill_btab(uint32_t* btab, int first, int stride) {
+	for (int i = first; i < kBtabWords; i += stride) {
+		const int h = i / 176, m = (i % 176) / 16, p = i % 16, base = h * 16;
+		uint32_t a = 0, b = 0, c = 0, kind = 0;
+		if (m == 0) kind = 2;
+		else if (m == 1) { a = 5 - (p >> 2); b = 7 + (p & 3); c = 6; kind = 1; }
+		else if (m == 10) kind = 3;
+		else {
+			const int tap = c_bpred_taps[m * 16 + p], t0 = tap & 15;
+			a = t0; b = t0 + 1; c = (tap & 16) ? t0 : t0 + 2;
+		}
+		btab[i] = (base + a) | ((base + b) << 8) | ((base + c) << 16) | (VP8P_KIND_CODE(kind) << 24);
+	}
+}
+
 constexpr int kClusterProg = 1024; // progress stamps per image in cluster mode (VP8 frames have at most 1024 macroblock rows)
 // per-slot scratch in global memory (L2): [tf: 8 x line][tu: 2 x line][stamps] (vp8_mb_split uses the tf lines only)
 __host__ __device__ constexpr size_t scratch_stride(int line_px) { return (size_t)10 * line_px + kClusterProg * 4; }
@@ -206,21 +223,7 @@ vp8_mb_pairs(const Vp8ImgDesc* __restrict__ descs, int n_images, int line_px, ui
 	static_assert(sizeof(Vp8ImgDesc) <= 256, "descriptor must fit its shared-memory slot");
 	static_assert(4 * NW <= kProgRing, "progress ring too small");
 
-	// B_PRED lane table: btab[half][mode 0..10][pixel] = lane(a) | lane(b)<<8 | lane(c)<<16 | kind<<24
-	if (RECON) {
-		for (int i = tid; i < kBtabWords; i += NW * 32) {
-			const int h = i / 176, m = (i % 176) / 16, p = i % 16, base = h * 16;
-			uint32_t a = 0, b = 0, c = 0, kind = 0;
-			if (m == 0) kind = 2;
-			else if (m == 1) { a = 5 - (p >> 2); b = 7 + (p & 3); c = 6; kind = 1; }
-			else if (m == 10) kind = 3;
-			else {
-				const int tap = c_bpred_taps[m * 16 + p], t0 = tap & 15;
-				a = t0; b = t0 + 1; c = (tap & 16) ? t0 : t0 + 2;
-			}
-			btab[i] = (base + a) | ((base + b) << 8) | ((base + c) << 16) | (VP8P_KIND_CODE(kind) << 24);
-		}
-	}
+	if (RECON) fill_btab(btab, tid, NW * 32);
 
 	// ---- lane roles inside a half (hl = 0..15)
 	//   transforms / block prediction: hl < 8 luma blocks 2hl, 2hl+1 (same block row); 8,9: U; 10,11: V; 12: Y2
@@ -405,18 +408,7 @@ vp8_mb_split(const Vp8ImgDesc* __restrict__ descs, int n_images, int line_px, ui
 	const uint32_t next_line = dsmem_addr((uint32_t)__cvta_generic_to_shared(lines + (size_t)next_engine * 2 * line_px), next_rank);
 	const uint32_t next_above = dsmem_addr((uint32_t)__cvta_generic_to_shared(role ? &wsb[next_engine * 2].above_f : &wsb[next_engine * 2].above), next_rank);
 
-	for (int i = tid; i < kBtabWords; i += NW * 32) {
-		const int h = i / 176, m = (i % 176) / 16, p = i % 16, base = h * 16;
-		uint32_t a = 0, b = 0, c = 0, kind = 0;
-		if (m == 0) kind = 2;
-		else if (m == 1) { a = 5 - (p >> 2); b = 7 + (p & 3); c = 6; kind = 1; }
-		else if (m == 10) kind = 3;
-		else {
-			const int tap = c_bpred_taps[m * 16 + p], t0 = tap & 15;
-			a = t0; b = t0 + 1; c = (tap & 16) ? t0 : t0 + 2;
-		}
-		btab[i] = (base + a) | ((base + b) << 8) | ((base + c) << 16) | (VP8P_KIND_CODE(kind) << 24);
-	}
+	fill_btab(btab, tid, NW * 32);
 
 	const bool tl_luma = hl < 8;
 	const int tl_by = tl_luma ? (hl >> 1) * 4 : (hl & 1) * 4;
@@ -695,20 +687,7 @@ vp8_mb_lockstep(const Vp8ImgDesc* __restrict__ descs, int n_images, int line_px,
 	uint8_t* tf_u = tf_y + 4 * line_px;
 	uint8_t* tf_v = tf_u + 2 * line_px;
 
-	if (RECON) {
-		for (int i = threadIdx.x; i < kBtabWords; i += blockDim.x) {
-			const int h = i / 176, m = (i % 176) / 16, p = i % 16, base = h * 16;
-			uint32_t a = 0, b = 0, c = 0, kind = 0;
-			if (m == 0) kind = 2;
-			else if (m == 1) { a = 5 - (p >> 2); b = 7 + (p & 3); c = 6; kind = 1; }
-			else if (m == 10) kind = 3;
-			else {
-				const int tap = c_bpred_taps[m * 16 + p], t0 = tap & 15;
-				a = t0; b = t0 + 1; c = (tap & 16) ? t0 : t0 + 2;
-			}
-			btab[i] = (base + a) | ((base + b) << 8) | ((base + c) << 16) | (VP8P_KIND_CODE(kind) << 24);
-		}
-	}
+	if (RECON) fill_btab(btab, threadIdx.x, blockDim.x);
 	if (warp == 0 && lane < 2) ctl[lane] = 0;
 	__syncthreads();
 
@@ -840,6 +819,27 @@ cudaError_t allow_smem(K k, size_t smem) {
 	return cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, limit);
 }
 
+// Launch configuration of `grid` 16-warp CTAs in clusters of `cluster`; cfg.attrs points into the object, so it is
+// neither copied nor moved.
+struct ClusterLaunch {
+	cudaLaunchConfig_t cfg{};
+	cudaLaunchAttribute attr[1];
+	ClusterLaunch(int grid, int cluster, size_t smem, cudaStream_t st) {
+		cfg.gridDim = dim3(grid);
+		cfg.blockDim = dim3(16 * 32);
+		cfg.dynamicSmemBytes = smem;
+		cfg.stream = st;
+		attr[0].id = cudaLaunchAttributeClusterDimension;
+		attr[0].val.clusterDim.x = (unsigned)cluster;
+		attr[0].val.clusterDim.y = 1;
+		attr[0].val.clusterDim.z = 1;
+		cfg.attrs = attr;
+		cfg.numAttrs = 1;
+	}
+	ClusterLaunch(const ClusterLaunch&) = delete;
+	ClusterLaunch& operator=(const ClusterLaunch&) = delete;
+};
+
 template <int NW, bool RECON, bool FILTER>
 int launch_lockstep_t(const Vp8ImgDesc* descs, int n, int line_px, int grid, int groups, size_t smem, uint8_t* scratch, cudaStream_t st) {
 	auto k = vp8_mb_lockstep<NW, RECON, FILTER>;
@@ -862,19 +862,8 @@ int launch_pairs_t(const Vp8ImgDesc* descs, int n, int line_px, int grid, size_t
 	auto k = vp8_mb_pairs<16, RECON, FILTER, true, false>;
 	cudaError_t e = allow_smem(k, smem);
 	if (e != cudaSuccess) return (int)e;
-	cudaLaunchConfig_t cfg{};
-	cfg.gridDim = dim3(grid);
-	cfg.blockDim = dim3(16 * 32);
-	cfg.dynamicSmemBytes = smem;
-	cfg.stream = st;
-	cudaLaunchAttribute attr[1];
-	attr[0].id = cudaLaunchAttributeClusterDimension;
-	attr[0].val.clusterDim.x = (unsigned)cluster;
-	attr[0].val.clusterDim.y = 1;
-	attr[0].val.clusterDim.z = 1;
-	cfg.attrs = attr;
-	cfg.numAttrs = 1;
-	e = cudaLaunchKernelEx(&cfg, k, descs, n, line_px, scratch);
+	const ClusterLaunch cl(grid, cluster, smem, st);
+	e = cudaLaunchKernelEx(&cl.cfg, k, descs, n, line_px, scratch);
 	if (e != cudaSuccess) return (int)e;
 	return (int)cudaGetLastError();
 }
@@ -886,19 +875,8 @@ int launch_split(bool filter, const Vp8ImgDesc* descs, int n, int line_px, int g
 	auto k = filter ? vp8_mb_split<true> : vp8_mb_split<false>;
 	cudaError_t e = allow_smem(k, smem);
 	if (e != cudaSuccess) return (int)e;
-	cudaLaunchConfig_t cfg{};
-	cfg.gridDim = dim3(grid);
-	cfg.blockDim = dim3(16 * 32);
-	cfg.dynamicSmemBytes = smem;
-	cfg.stream = st;
-	cudaLaunchAttribute attr[1];
-	attr[0].id = cudaLaunchAttributeClusterDimension;
-	attr[0].val.clusterDim.x = (unsigned)cluster;
-	attr[0].val.clusterDim.y = 1;
-	attr[0].val.clusterDim.z = 1;
-	cfg.attrs = attr;
-	cfg.numAttrs = 1;
-	e = cudaLaunchKernelEx(&cfg, k, descs, n, line_px, scratch);
+	const ClusterLaunch cl(grid, cluster, smem, st);
+	e = cudaLaunchKernelEx(&cl.cfg, k, descs, n, line_px, scratch);
 	if (e != cudaSuccess) return (int)e;
 	return (int)cudaGetLastError();
 }
@@ -915,19 +893,9 @@ int occupancy_pairs_t(size_t smem) {
 template <typename K>
 int max_clusters_of(K k, size_t smem, int cluster) {
 	if (allow_smem(k, smem) != cudaSuccess) return 0;
-	cudaLaunchConfig_t cfg{};
-	cfg.gridDim = dim3(cluster);
-	cfg.blockDim = dim3(16 * 32);
-	cfg.dynamicSmemBytes = smem;
-	cudaLaunchAttribute attr[1];
-	attr[0].id = cudaLaunchAttributeClusterDimension;
-	attr[0].val.clusterDim.x = (unsigned)cluster;
-	attr[0].val.clusterDim.y = 1;
-	attr[0].val.clusterDim.z = 1;
-	cfg.attrs = attr;
-	cfg.numAttrs = 1;
+	const ClusterLaunch cl(cluster, cluster, smem, nullptr);
 	int n = 0;
-	if (cudaOccupancyMaxActiveClusters(&n, k, &cfg) != cudaSuccess) {
+	if (cudaOccupancyMaxActiveClusters(&n, k, &cl.cfg) != cudaSuccess) {
 		(void)cudaGetLastError();
 		return 0;
 	}
