@@ -1,10 +1,11 @@
 import sys, json, time
-sys.path.insert(0,'/root/repo')
 from pathlib import Path
+ROOT = Path(__file__).resolve().parent.parent
+sys.path.insert(0, str(ROOT))
 import webp_decoder_b200 as W
 from webp_decoder_b200 import parse as P
 files=["noise_1920x1080_q75.webp","rgbgrad_1920x1080_q75.webp","checker_1920x1080_q75.webp","diag_1920x1080_q75.webp"]
-pf=P.parse_batch([Path('/root/repo/bench_data/'+f).read_bytes() for f in files], pinned=True)
+pf=P.parse_batch([(ROOT / 'bench_data' / f).read_bytes() for f in files], pinned=True)
 ctx=W.Context(0)
 for name,sel in [("mix",[0,1,2,3]),("noise",[0]),("rgbgrad",[1]),("checker",[2]),("diag",[3])]:
     order=[sel[i%len(sel)] for i in range(1024)]

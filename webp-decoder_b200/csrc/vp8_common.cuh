@@ -79,15 +79,17 @@ __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wai
 
 // Store 4 pixels at (ox, oy) of an output plane, honouring the crop (negative coordinates are outside too).
 // The byte-wise tail is rare (frame borders, unaligned strides): kept out of line so that it is not replicated at every
-// store site (the kernels are instruction-cache bound).
+// store site (the kernels are instruction-cache bound). Both stores are predicated rather than behind an early return, so
+// the lanes do not diverge around them; the address is formed on every lane but used only inside the plane.
 __device__ __noinline__ void put_bytes(uint8_t* d, uint32_t v, uint32_t n) {
 	for (uint32_t k = 0; k < n; k++) d[k] = (uint8_t)(v >> (8 * k));
 }
 __device__ __forceinline__ void put_word(const OutPlane& o, int ox, int oy, uint32_t v) {
-	if ((uint32_t)oy >= o.h || (uint32_t)ox >= o.w) return;
+	const bool in = ((uint32_t)oy < o.h) & ((uint32_t)ox < o.w);
+	const bool word = in & o.word_ok & ((uint32_t)ox + 4 <= o.w);
 	uint8_t* d = o.p + (size_t)oy * o.stride + ox;
-	if (o.word_ok && (uint32_t)ox + 4 <= o.w) st_pix32(d, v);
-	else put_bytes(d, v, min(4u, o.w - (uint32_t)ox));
+	if (word) st_pix32(d, v);
+	if (in & !word) put_bytes(d, v, min(4u, o.w - (uint32_t)ox));
 }
 
 // ------------------------------------------------------------------------------------------------ transforms
