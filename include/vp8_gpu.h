@@ -145,6 +145,18 @@ int vp8_gpu_rgb(vp8_gpu_ctx* ctx, vp8_gpu_batch* b);
  * EFBIG for an image whose scanlines exceed 0x7FFFFFFF bytes (the reference's own limit). */
 int vp8_gpu_png(vp8_gpu_ctx* ctx, vp8_gpu_batch* b);
 
+/* Compressed -png files (default 0: off, the reference's bytes). With on != 0 every -png door of this context - vp8_gpu_png +
+ * vp8_gpu_download_png, vp8_gpu_decode_png, VP8_GPU_OUT_PNG through vp8_gpu_decode_compact / vp8_gpu_decode_webp - writes
+ * what any PNG reader decodes to the same pixels, but smaller: every scanline carries the PNG filter (0..4) whose filtered
+ * bytes have the least sum of min(v, 256 - v), and the filtered stream is cut into the stored writer's 65535-byte pieces, each
+ * one a fixed-Huffman deflate block of run-length tokens (matches at distance 1) closed by an empty stored block, or - when
+ * that is not shorter - the stored block itself. So no file is longer than its stored version, and vp8_gpu_png_bytes /
+ * vp8_gpu_decode_bytes / vp8_gpu_decode_webp_bytes remain the capacity to provide. Filtering, encoding, checksums and the
+ * layout are done on the device (vp8_pngz.cu); the files of a batch lie back to back, in dst as well (always read
+ * offsets[] and sizes[]), and the pipelined calls move only their bytes and each file's length over the link.
+ * yuv420_write_png_fd and vp8_gpu_png_frame always emit the reference's bytes. */
+int vp8_gpu_set_png_deflate(vp8_gpu_ctx* ctx, int on);
+
 enum { VP8_GPU_TIGHT = 0, VP8_GPU_PADDED = 1 };
 
 /* One pass over an uploaded batch: reconstruction, fused with the loop filter when filtered != 0.

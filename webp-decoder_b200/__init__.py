@@ -50,7 +50,7 @@ EXPORTS = [
     "vp8_gpu_last_launch_config", "vp8_gpu_frame_params", "vp8_gpu_kernel_time", "vp8_gpu_rgb_time",
     "vp8_gpu_decode_i420", "vp8_gpu_decode_ppm", "vp8_gpu_decode_bytes", "vp8_gpu_set_kernel",
     "vp8_gpu_png_bound", "vp8_gpu_png_frame", "vp8_gpu_set_transport",
-    "vp8_gpu_png", "vp8_gpu_png_bytes", "vp8_gpu_download_png", "vp8_gpu_decode_png", "vp8_gpu_png_time",
+    "vp8_gpu_png", "vp8_gpu_png_bytes", "vp8_gpu_download_png", "vp8_gpu_decode_png", "vp8_gpu_png_time", "vp8_gpu_set_png_deflate",
     "vp8_gpu_set_cluster", "vp8_gpu_set_cluster_split", "vp8_gpu_last_split", "vp8_gpu_last_cluster", "vp8_gpu_last_groups", "vp8_gpu_last_segments",
     "vp8_gpu_decode_compact", "vp8_gpu_decode_webp", "vp8_gpu_decode_webp_bytes", "vp8_gpu_last_call_profile", "vp8_gpu_bind_host", "vp8_gpu_last_transport", "vp8_gpu_last_dense_frames",
     # encoder in-loop reconstruction (include/vp8_enc.h)
@@ -115,6 +115,7 @@ def load_library() -> C.CDLL:
     L.vp8_gpu_download_png.argtypes = [vp, vp, vp, sz, vp, vp]
     L.vp8_gpu_decode_png.argtypes = [vp, pp, pp, C.c_int, vp, sz, vp, vp, C.c_int]
     L.vp8_gpu_png_time.argtypes = [vp, C.POINTER(C.c_double), C.POINTER(C.c_int)]
+    L.vp8_gpu_set_png_deflate.argtypes = [vp, C.c_int]
     L.vp8_gpu_download_images.argtypes = [vp, vp, vp]
     L.vp8_gpu_download_padded.argtypes = [vp, vp, C.c_int, vp, vp, vp]
     L.vp8_gpu_batch_size.argtypes = [vp]
@@ -268,6 +269,12 @@ class Context:
         """compact: True / False, or "auto" (chosen chunk by chunk, the library's default)."""
         mode = 2 if compact == "auto" else int(bool(compact))
         _check(self._L.vp8_gpu_set_transport(self._h, mode, host_threads), "vp8_gpu_set_transport")
+
+    def set_png_deflate(self, on: bool):
+        """Compressed -png files from every -png call of this context (per-row PNG filters, run-length fixed-Huffman
+        deflate, all on the device; never longer than the stored files) - or, off (the default), the reference's bytes.
+        The files then lie back to back: read offsets / sizes."""
+        _check(self._L.vp8_gpu_set_png_deflate(self._h, int(bool(on))), "vp8_gpu_set_png_deflate")
 
     def last_dense_frames(self):
         """Frames of the last pipelined call that crossed dense inside compact chunks (vp8_gpu_last_dense_frames)."""

@@ -16,7 +16,7 @@ from pathlib import Path
 HERE = Path(__file__).resolve().parent
 CSRC = HERE / "csrc"
 LIB = HERE / "libvp8gpu.so"
-SOURCES = [CSRC / "vp8_pairs.cu", CSRC / "vp8_rgb.cu", CSRC / "vp8_png.cu", CSRC / "vp8_gpu.cu", CSRC / "vp8_enc.cu", CSRC / "vp8_parse.cpp"]
+SOURCES = [CSRC / "vp8_pairs.cu", CSRC / "vp8_rgb.cu", CSRC / "vp8_png.cu", CSRC / "vp8_pngz.cu", CSRC / "vp8_gpu.cu", CSRC / "vp8_enc.cu", CSRC / "vp8_parse.cpp"]
 HEADERS = sorted(list(CSRC.glob("*.h")) + list(CSRC.glob("*.cuh")) + list(CSRC.glob("*.inc")) + list((HERE.parent / "include").glob("*.h")))
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 

@@ -71,6 +71,16 @@ struct Vp8PngDesc {
 	uint32_t pad_;
 };
 
+// Work item of the compressed-PNG kernels (vp8_pngz.cu): one RGB24 image in, a filtered, run-length deflated -png file out.
+struct Vp8PngzDesc {
+	const uint8_t* rgb;    // tight RGB24
+	uint32_t width, height;
+	uint32_t first_row;    // scanlines of the images before this one
+	uint32_t first_piece;  // pieces (vp8_pngz_pieces) of the images before this one
+	uint8_t head[44];      // vp8_pngz_fill_desc; the finish kernel writes the file's IDAT length over bytes 33..36
+	uint32_t pad_;
+};
+
 enum Vp8KernelMode {
 	VP8_K_RECON = 0,        // m06 only: unfiltered pixels out
 	VP8_K_RECON_FILTER = 1, // m06+m07 fused: filtered pixels out, single pass
@@ -109,3 +119,13 @@ size_t vp8_png_accum_bytes(void);
 size_t vp8_png_tables_bytes(void);
 void vp8_png_tables(void* dst);
 void vp8_png_fill_desc(Vp8PngDesc* d, const void* tables);
+// Compressed -png files (vp8_pngz.cu), written back to back into out_dev: file i starts at the sum of the lengths of the files
+// before it. work_dev: vp8_pngz_work_bytes() of device memory, where the kernels leave each file's length (vp8_pngz_lens:
+// n_images uint32). tables_dev: vp8_png_tables() on the device. vp8_pngz_fill_desc completes a descriptor whose width /
+// height are set; first_row / first_piece = running sums of height / vp8_pngz_pieces().
+int vp8_launch_pngz(const Vp8PngzDesc* descs_dev, int n_images, uint32_t total_rows, uint32_t total_pieces, const void* tables_dev, void* work_dev,
+                    uint8_t* out_dev, void* stream);
+size_t vp8_pngz_work_bytes(int n_images, uint32_t total_rows, uint32_t total_pieces);
+const uint32_t* vp8_pngz_lens(const void* work_dev, int n_images, uint32_t total_rows, uint32_t total_pieces);
+uint32_t vp8_pngz_pieces(uint32_t width, uint32_t height);
+void vp8_pngz_fill_desc(Vp8PngzDesc* d, const void* tables);

@@ -162,6 +162,9 @@ struct vp8_gpu_ctx {
 	std::vector<std::pair<cudaEvent_t, cudaEvent_t>> timed_rgb; // same for the m08 launches
 	std::vector<std::pair<cudaEvent_t, cudaEvent_t>> timed_png; // same for the m09 launches
 	void* d_png_tables = nullptr;                               // checksum tables of the m09 kernels (first vp8_gpu_png)
+	bool png_deflate = false;                                   // -png files filtered and run-length deflated (vp8_gpu_set_png_deflate)
+	uint32_t* zlens = nullptr;                                  // pinned: per-file lengths of a pipelined deflate call, one per frame
+	size_t zlens_cap = 0;
 	std::vector<std::pair<cudaEvent_t, cudaEvent_t>> spare;
 	cudaStream_t pipe[4] = {nullptr, nullptr, nullptr, nullptr}; // chunk pipeline of vp8_gpu_decode_*
 	cudaEvent_t pipe_ev = nullptr;
@@ -232,6 +235,12 @@ struct vp8_gpu_batch {
 	void* d_pngacc = nullptr;
 	uint32_t png_ctas = 0;
 	bool pngdesc_up = false, have_png = false;
+	Vp8PngzDesc* d_pngzdesc = nullptr; // compressed -png (vp8_pngz.cu): descriptors and the launch's scratch
+	void* d_pngzwork = nullptr;
+	size_t pngz_work_bytes = 0;
+	uint32_t pngz_rows = 0, pngz_pieces = 0;
+	bool pngzdesc_up = false;
+	bool png_z = false; // d_png holds compressed files, back to back (the last vp8_gpu_png ran with deflate on)
 	int max_mb_cols = 0;
 	PlaneState state = PLANES_NONE;
 	bool filtered = false, have_rgb = false, have_coeffs = true;
@@ -571,6 +580,8 @@ void batch_destroy(vp8_gpu_ctx* c, vp8_gpu_batch* b, bool known_idle = false) {
 	dev_release(c, b->d_png, b->png_bytes);
 	dev_release(c, b->d_pngdesc, sizeof(Vp8PngDesc) * b->n);
 	dev_release(c, b->d_pngacc, vp8_png_accum_bytes() * b->n);
+	dev_release(c, b->d_pngzdesc, sizeof(Vp8PngzDesc) * b->n);
+	dev_release(c, b->d_pngzwork, b->pngz_work_bytes);
 	dev_release(c, b->d_scratch, b->scratch_bytes);
 	delete b;
 }
@@ -1423,6 +1434,7 @@ void vp8_gpu_destroy(vp8_gpu_ctx* c) {
 		if (c->bounce_ev[i]) cudaEventDestroy(c->bounce_ev[i]);
 	}
 	if (c->d_png_tables) cudaFree(c->d_png_tables);
+	if (c->zlens) cudaFreeHost(c->zlens);
 	for (auto* v : {&c->timed, &c->timed_rgb, &c->timed_png, &c->spare})
 		for (auto& ev : *v) {
 			cudaEventDestroy(ev.first);
@@ -1477,6 +1489,12 @@ int vp8_gpu_set_cluster(vp8_gpu_ctx* c, int ctas_per_image) {
 	if (!c || (ctas_per_image != 0 && ctas_per_image != 1 && ctas_per_image != 2 && ctas_per_image != 4 && ctas_per_image != 8))
 		return fail(EINVAL, "bad cluster size");
 	c->tune_cluster = ctas_per_image;
+	return 0;
+}
+
+int vp8_gpu_set_png_deflate(vp8_gpu_ctx* c, int on) {
+	if (!c) return fail(EINVAL, "no context");
+	c->png_deflate = on != 0;
 	return 0;
 }
 
@@ -1633,11 +1651,13 @@ static int png_layout(vp8_gpu_batch* b) {
 	b->png_ctas = (uint32_t)ctas;
 	return 0;
 }
+static int push_pngz_descs(vp8_gpu_ctx* c, vp8_gpu_batch* b);
 static int push_png_descs(vp8_gpu_ctx* c, vp8_gpu_batch* b) {
 	if (png_layout(b)) return -1;
 	if (png_tables_ready(c)) return -1;
 	if (!b->d_rgb && dev_alloc(c, b->rgb_bytes, (void**)&b->d_rgb)) return -1;
 	if (!b->d_png && dev_alloc(c, b->png_bytes, (void**)&b->d_png)) return -1;
+	if (c->png_deflate) return push_pngz_descs(c, b);
 	if (!b->d_pngdesc && dev_alloc(c, sizeof(Vp8PngDesc) * b->n, (void**)&b->d_pngdesc)) return -1;
 	if (!b->d_pngacc && dev_alloc(c, vp8_png_accum_bytes() * b->n, &b->d_pngacc)) return -1;
 	if (b->pngdesc_up) return 0;
@@ -1666,18 +1686,53 @@ static int push_png_descs(vp8_gpu_ctx* c, vp8_gpu_batch* b) {
 	return 0;
 }
 
+// Compressed -png (vp8_pngz.cu): the files go back to back into the same arena, which holds them since none is longer than
+// its stored version.
+static int push_pngz_descs(vp8_gpu_ctx* c, vp8_gpu_batch* b) {
+	if (b->pngzdesc_up) return 0;
+	std::vector<Vp8PngzDesc> h(b->n);
+	uint64_t rows = 0, pieces = 0;
+	for (int i = 0; i < b->n; i++) {
+		const FrameMeta& m = b->meta[i];
+		Vp8PngzDesc& d = h[i];
+		memset(&d, 0, sizeof(d));
+		d.rgb = b->d_rgb + m.rgb_off + kPpmSlot;
+		d.width = m.width;
+		d.height = m.height;
+		d.first_row = (uint32_t)rows;
+		d.first_piece = (uint32_t)pieces;
+		rows += m.height;
+		pieces += vp8_pngz_pieces(m.width, m.height);
+		if (i && h[i - 1].width == d.width && h[i - 1].height == d.height) memcpy(d.head, h[i - 1].head, sizeof(d.head));
+		else vp8_pngz_fill_desc(&d, png_host_tables());
+	}
+	if (rows > 0x7FFFFFFFull || pieces > 0x7FFFFFFFull) return fail(EFBIG, "batch too large for one PNG launch");
+	b->pngz_rows = (uint32_t)rows;
+	b->pngz_pieces = (uint32_t)pieces;
+	b->pngz_work_bytes = vp8_pngz_work_bytes(b->n, b->pngz_rows, b->pngz_pieces);
+	if (!b->d_pngzdesc && dev_alloc(c, sizeof(Vp8PngzDesc) * b->n, (void**)&b->d_pngzdesc)) return -1;
+	if (!b->d_pngzwork && dev_alloc(c, b->pngz_work_bytes, &b->d_pngzwork)) return -1;
+	if (push_table(c, b->d_pngzdesc, h.data(), sizeof(Vp8PngzDesc) * b->n, b->stream)) return -1;
+	b->pngzdesc_up = true;
+	return 0;
+}
+static const uint32_t* pngz_lens_dev(const vp8_gpu_batch* b) { return vp8_pngz_lens(b->d_pngzwork, b->n, b->pngz_rows, b->pngz_pieces); }
+
 int vp8_gpu_png(vp8_gpu_ctx* c, vp8_gpu_batch* b) {
 	if (!c || !b) return fail(EINVAL, "bad arguments");
 	if (!b->have_rgb) return fail(EINVAL, "run vp8_gpu_rgb first");
 	CU(cudaSetDevice(c->device));
 	if (push_png_descs(c, b)) return -1;
+	const bool z = c->png_deflate;
 	TimedPair ev;
 	if (begin_timed(c, b->stream, &ev)) return -1;
-	const int rc = vp8_launch_png(b->d_pngdesc, b->n, b->png_ctas, c->d_png_tables, b->d_pngacc, b->stream);
+	const int rc = z ? vp8_launch_pngz(b->d_pngzdesc, b->n, b->pngz_rows, b->pngz_pieces, c->d_png_tables, b->d_pngzwork, b->d_png, b->stream)
+	                 : vp8_launch_png(b->d_pngdesc, b->n, b->png_ctas, c->d_png_tables, b->d_pngacc, b->stream);
 	if (end_timed(c, c->timed_png, ev, b->stream)) return -1;
 	if (rc) return fail(EIO, "png launch", (cudaError_t)rc);
-	c->launches += 2;
+	c->launches += z ? 5 : 2;
 	b->have_png = true;
+	b->png_z = z;
 	return 0;
 }
 
@@ -1686,7 +1741,19 @@ size_t vp8_gpu_png_bytes(vp8_gpu_batch* b) { return b && !png_layout(b) ? b->png
 int vp8_gpu_download_png(vp8_gpu_ctx* c, vp8_gpu_batch* b, uint8_t* dst, size_t cap, size_t* offsets, size_t* sizes) {
 	if (!c || !b || !dst) return fail(EINVAL, "bad arguments");
 	if (!b->have_png) return fail(EINVAL, "run vp8_gpu_png first");
-	return download_out(c, b, VP8_GPU_OUT_PNG, dst, cap, offsets, sizes);
+	if (!b->png_z) return download_out(c, b, VP8_GPU_OUT_PNG, dst, cap, offsets, sizes);
+	// compressed: the files' lengths first, then their bytes in one copy
+	if (cap < b->png_bytes) return fail(EINVAL, "destination too small");
+	CU(cudaSetDevice(c->device));
+	std::vector<uint32_t> lens(b->n);
+	if (download(c, b->stream, lens.data(), (const uint8_t*)pngz_lens_dev(b), sizeof(uint32_t) * b->n)) return -1;
+	size_t at = 0;
+	for (int i = 0; i < b->n; i++) {
+		if (offsets) offsets[i] = at;
+		if (sizes) sizes[i] = lens[i];
+		at += lens[i];
+	}
+	return download(c, b->stream, dst, b->d_png, at);
 }
 
 size_t vp8_gpu_i420_bytes(const vp8_gpu_batch* b) { return b ? b->tight_bytes : 0; }
@@ -2194,6 +2261,19 @@ static int decode_pipelined(vp8_gpu_ctx* c, const FrameGeom* geom, int n, const 
 		off[i + 1] = off[i] + out_slot_bytes(w, h, format);
 	}
 	if (cap < off[n]) return fail(EINVAL, "destination too small");
+	// Compressed -png: a chunk's files have their length only once its kernels ran. Its lengths (4 bytes a file) come back into
+	// pinned memory first, and its download - ONE copy of its files, packed behind those of the chunk before - is enqueued one
+	// chunk later, so that the host has made the next chunk before it waits for them.
+	const bool deflate = want_png && c->png_deflate;
+	if (deflate && c->zlens_cap < (size_t)n) {
+		if (c->zlens) cudaFreeHost(c->zlens);
+		c->zlens = nullptr;
+		c->zlens_cap = 0;
+		CU(cudaHostAlloc((void**)&c->zlens, sizeof(uint32_t) * n, cudaHostAllocDefault));
+		c->zlens_cap = n;
+	}
+	std::vector<size_t> zoff(deflate ? n : 0);
+	size_t zpos = 0;
 	for (auto& p : c->pipe)
 		if (!p) CU(cudaStreamCreateWithFlags(&p, cudaStreamNonBlocking));
 	if (!c->pipe_ev) CU(cudaEventCreateWithFlags(&c->pipe_ev, cudaEventDisableTiming));
@@ -2208,6 +2288,8 @@ static int decode_pipelined(vp8_gpu_ctx* c, const FrameGeom* geom, int n, const 
 	struct Chunk {
 		vp8_gpu_batch* b = nullptr;
 		cudaEvent_t up = nullptr, done = nullptr;
+		cudaEvent_t lens = nullptr; // deflate: its kernels and its file lengths' copy are done
+		int first = 0, cnt = 0;
 	};
 	Chunk ring[kDepth];
 	cudaEvent_t ev_kernel = nullptr;
@@ -2223,14 +2305,27 @@ static int decode_pipelined(vp8_gpu_ctx* c, const FrameGeom* geom, int n, const 
 		ch.b = nullptr;
 	};
 	rc = make_event(&ev_kernel);
-	for (int i = 0; i < kDepth && !rc; i++) rc = make_event(&ring[i].up) || make_event(&ring[i].done);
+	for (int i = 0; i < kDepth && !rc; i++) rc = make_event(&ring[i].up) || make_event(&ring[i].done) || make_event(&ring[i].lens);
+	Chunk* pending = nullptr; // deflate: the chunk whose download is not enqueued yet
+	auto download_pending = [&]() -> int {
+		Chunk* ch = pending;
+		pending = nullptr;
+		if (!ch) return 0;
+		CU(cudaEventSynchronize(ch->lens));
+		const size_t at = zpos;
+		for (int j = 0; j < ch->cnt; j++) zoff[ch->first + j] = zpos, zpos += c->zlens[ch->first + j];
+		CU(cudaStreamWaitEvent(c->pipe[3], ch->lens, 0));
+		if (download(c, c->pipe[3], dst + at, ch->b->d_png, zpos - at, false)) return -1;
+		CU(cudaEventRecord(ch->done, c->pipe[3]));
+		return 0;
+	};
 	const auto t_p0 = std::chrono::steady_clock::now();
 	c->trace_compact_ms = c->trace_retire_ms = c->trace_malloc_ms = 0;
 	c->trace_dense_frames = 0;
 	c->trace_mallocs = c->trace_frees = 0;
 	cudaStream_t s_up = c->pipe[0], s_down = c->pipe[3];
 	// VP8_GPU_TRACE=2: device-side timeline, four timed events per chunk (upload start/end, kernels end, download end)
-	const bool timeline = getenv("VP8_GPU_TRACE") && atoi(getenv("VP8_GPU_TRACE")) >= 2;
+	const bool timeline = !deflate && getenv("VP8_GPU_TRACE") && atoi(getenv("VP8_GPU_TRACE")) >= 2;
 	std::vector<cudaEvent_t> tl;
 	std::vector<double> tl_host;
 	auto mark = [&](cudaStream_t s) {
@@ -2278,6 +2373,20 @@ static int decode_pipelined(vp8_gpu_ctx* c, const FrameGeom* geom, int n, const 
 		if (!rc && want_png) rc = vp8_gpu_png(c, b);
 		if (rc) break;
 		mark(s_run);
+		if (deflate) {
+			ch.first = first;
+			ch.cnt = cnt;
+			c->d2h += sizeof(uint32_t) * cnt;
+			if (cudaMemcpyAsync(c->zlens + first, pngz_lens_dev(b), sizeof(uint32_t) * cnt, cudaMemcpyDeviceToHost, s_run) != cudaSuccess ||
+			    cudaEventRecord(ch.lens, s_run) != cudaSuccess) {
+				rc = fail(EIO, "pipeline lengths", cudaGetLastError());
+				break;
+			}
+			rc = download_pending(); // the chunk before this one
+			pending = &ch;
+			if (rc) break;
+			continue;
+		}
 		if (cudaEventRecord(ev_kernel, s_run) != cudaSuccess || cudaStreamWaitEvent(s_down, ev_kernel, 0) != cudaSuccess) {
 			rc = fail(EIO, "pipeline events", cudaGetLastError());
 			break;
@@ -2287,6 +2396,7 @@ static int decode_pipelined(vp8_gpu_ctx* c, const FrameGeom* geom, int n, const 
 		if (!rc && cudaEventRecord(ch.done, s_down) != cudaSuccess) rc = fail(EIO, "pipeline events", cudaGetLastError());
 		mark(s_down);
 	}
+	if (!rc) rc = download_pending(); // the last chunk
 	const int saved = errno;
 	const auto t_e0 = std::chrono::steady_clock::now();
 	for (auto& p : c->pipe) cudaStreamSynchronize(p);
@@ -2294,6 +2404,7 @@ static int decode_pipelined(vp8_gpu_ctx* c, const FrameGeom* geom, int n, const 
 		if (ch.b) batch_destroy(c, ch.b, true);
 		if (ch.up) cudaEventDestroy(ch.up);
 		if (ch.done) cudaEventDestroy(ch.done);
+		if (ch.lens) cudaEventDestroy(ch.lens);
 	}
 	if (ev_kernel) cudaEventDestroy(ev_kernel);
 	if (timeline && !rc) {
@@ -2319,7 +2430,14 @@ static int decode_pipelined(vp8_gpu_ctx* c, const FrameGeom* geom, int n, const 
 		errno = saved;
 		return -1;
 	}
-	for (int i = 0; i < n; i++) report_slot(dst, off[i], geom[i].width, geom[i].height, format, i, offsets, sizes);
+	for (int i = 0; i < n; i++) {
+		if (!deflate) {
+			report_slot(dst, off[i], geom[i].width, geom[i].height, format, i, offsets, sizes);
+			continue;
+		}
+		if (offsets) offsets[i] = zoff[i];
+		if (sizes) sizes[i] = c->zlens[i];
+	}
 	return 0;
 }
 

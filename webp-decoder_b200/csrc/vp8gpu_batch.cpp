@@ -1,8 +1,10 @@
 // vp8gpu_batch - batch front end over libvp8gpu.so: the reference CLI's -yuv / -yuvf / -ppm / -png sub-commands
 // (reference src/main.c:556-842) for MANY files at once, on one or several GPUs.
 //
-//   vp8gpu_batch -yuv|-yuvf|-ppm|-png <out_dir> [--devices 0,1,..] [--device N] [--threads T] [--chunk C] file.webp ...
+//   vp8gpu_batch -yuv|-yuvf|-ppm|-png <out_dir> [--deflate] [--devices 0,1,..] [--device N] [--threads T] [--chunk C] file.webp ...
 //
+// --deflate (with -png only): compressed .png files - per-row PNG filters and run-length deflate, framed on the device
+// (vp8_gpu_set_png_deflate) - instead of the reference's stored-deflate bytes.
 // The files are dealt to the GPUs longest-first by macroblock count (frames are independent units: no exchange between
 // GPUs). Per GPU one host thread runs the whole pipeline for its share: container + header + token parsing on T / #GPUs
 // parser threads straight into the compact wire format in pinned memory (vp8_parse_batch_compact), one pipelined GPU
@@ -79,7 +81,7 @@ struct Job {
 
 // Everything one GPU does for its share of the files. Returns the number of failed files.
 static int run_share(int device, int slot, int n_devices, std::vector<Job*>& jobs, const std::string& mode, const std::string& out_dir,
-                     int threads, int chunk) {
+                     int threads, int chunk, bool deflate) {
 	const int n = (int)jobs.size();
 	if (n == 0) return 0;
 	vp8_gpu_ctx* ctx = nullptr;
@@ -89,6 +91,7 @@ static int run_share(int device, int slot, int n_devices, std::vector<Job*>& job
 	}
 	if (n_devices > 1) vp8_gpu_bind_host(ctx, slot, 0); // this thread, its parser threads and its pinned memory next to the GPU
 	vp8_gpu_set_transport(ctx, 2, threads);
+	vp8_gpu_set_png_deflate(ctx, deflate);
 	int failed = 0;
 	// ---- parse on host threads (m01 + m02 + m05) straight into one pinned arena, compact wire format
 	size_t arena_bytes = 0;
@@ -153,7 +156,7 @@ static int run_share(int device, int slot, int n_devices, std::vector<Job*>& job
 
 int main(int argc, char** argv) {
 	if (argc < 4) {
-		fprintf(stderr, "usage: %s -yuv|-yuvf|-ppm|-png <out_dir> [--devices 0,1,..] [--threads T] [--chunk C] file.webp ...\n", argv[0]);
+		fprintf(stderr, "usage: %s -yuv|-yuvf|-ppm|-png <out_dir> [--deflate] [--devices 0,1,..] [--threads T] [--chunk C] file.webp ...\n", argv[0]);
 		return 2;
 	}
 	const std::string mode = argv[1], out_dir = argv[2];
@@ -162,6 +165,7 @@ int main(int argc, char** argv) {
 		return 2;
 	}
 	int threads = (int)std::thread::hardware_concurrency(), chunk = 0;
+	bool deflate = false;
 	std::vector<int> devices;
 	std::vector<const char*> paths;
 	for (int i = 3; i < argc; i++) {
@@ -169,9 +173,14 @@ int main(int argc, char** argv) {
 			for (char* tok = strtok(argv[++i], ","); tok; tok = strtok(nullptr, ",")) devices.push_back(atoi(tok));
 		} else if (!strcmp(argv[i], "--threads") && i + 1 < argc) threads = atoi(argv[++i]);
 		else if (!strcmp(argv[i], "--chunk") && i + 1 < argc) chunk = atoi(argv[++i]);
+		else if (!strcmp(argv[i], "--deflate")) deflate = true;
 		else paths.push_back(argv[i]);
 	}
 	if (paths.empty()) return 2;
+	if (deflate && mode != "-png") {
+		fprintf(stderr, "error: --deflate needs -png\n");
+		return 2;
+	}
 	if (devices.empty()) devices.push_back(0);
 	mkdir(out_dir.c_str(), 0755);
 
@@ -207,7 +216,7 @@ int main(int argc, char** argv) {
 	std::vector<std::thread> workers;
 	const int per = std::max(1, threads / nd);
 	for (int d = 0; d < nd; d++)
-		workers.emplace_back([&, d] { gpu_failed += run_share(devices[d], d, nd, share[d], mode, out_dir, per, chunk); });
+		workers.emplace_back([&, d] { gpu_failed += run_share(devices[d], d, nd, share[d], mode, out_dir, per, chunk, deflate); });
 	for (auto& t : workers) t.join();
 	return (failed + gpu_failed.load()) ? 1 : 0;
 }
