@@ -331,58 +331,94 @@ void orc_frame_params(const Vp8DecodedFrame* f, int16_t dq[4][6], uint8_t lf[4][
 	}
 }
 
-enum { EDGE_MB = 0, EDGE_INNER = 1, EDGE_SIMPLE = 2 };
+enum { EDGE_MB = ORC_LF_MB, EDGE_INNER = ORC_LF_INNER, EDGE_SIMPLE = ORC_LF_SIMPLE };
+
+/* Where the positions of one edge are counted: counts == NULL counts nothing (orc_loopfilter_padded). */
+typedef struct {
+	uint64_t* counts;
+	int dir, plane, parity; /* parity: of the macroblock row below a horizontal macroblock edge, else -1 */
+} LfSite;
+
+static void tally(const LfSite* at, int cell) {
+	if (at->counts) at->counts[cell]++;
+}
+
+static void tally_outcome(const LfSite* at, int kind, int outcome) {
+	tally(at, ORC_LF_OUTCOME_CELL(kind, at->dir, at->plane, outcome));
+	if (at->parity >= 0) tally(at, ORC_LF_PARITY_CELL(at->parity, outcome));
+}
+
+/* clip255, adding to *n when it clips */
+static uint8_t clip255_n(int v, int* n) {
+	*n += v < 0 || v > 255;
+	return clip255(v);
+}
 
 /* Filter one position across an edge. q points at q0, s is the step across the edge.
  * kind EDGE_MB    : reference filter_mb_*_edge body   (vp8_loopfilter.c:106-117,129-140)
  * kind EDGE_INNER : reference filter_subblock_*_edge  (vp8_loopfilter.c:119-127,142-150)
  * kind EDGE_SIMPLE: reference filter_*_edge_simple    (vp8_loopfilter.c:152-164), lim = total limit
  * with thresholds :24-56 and kernels :58-104. */
-static void filter_pos(uint8_t* q, ptrdiff_t s, int kind, int lim, int interior, int hev_thr) {
+static void filter_pos(uint8_t* q, ptrdiff_t s, int kind, int lim, int interior, int hev_thr, const LfSite* at) {
 	int p1 = q[-2 * s], p0 = q[-s], q0 = q[0], q1 = q[s];
-	if (2 * iabs(p0 - q0) + (iabs(p1 - q1) >> 1) > lim) return;
+	int clips = 0;
+	if (2 * iabs(p0 - q0) + (iabs(p1 - q1) >> 1) > lim) {
+		tally_outcome(at, kind, ORC_LF_FAIL_EDGE);
+		return;
+	}
 	int hev = 0;
 	if (kind != EDGE_SIMPLE) {
 		int p3 = q[-4 * s], p2 = q[-3 * s], q2 = q[2 * s], q3 = q[3 * s];
 		if (iabs(p3 - p2) > interior || iabs(p2 - p1) > interior || iabs(p1 - p0) > interior ||
-		    iabs(q3 - q2) > interior || iabs(q2 - q1) > interior || iabs(q1 - q0) > interior)
-			return;
-		hev = iabs(p1 - p0) > hev_thr || iabs(q1 - q0) > hev_thr;
-		if (kind == EDGE_MB && !hev) {
-			int w = sclamp(sclamp(p1 - q1) + 3 * (q0 - p0));
-			int a = (27 * w + 63) >> 7, b = (18 * w + 63) >> 7, c = (9 * w + 63) >> 7;
-			q[-s] = clip255(p0 + a);
-			q[0] = clip255(q0 - a);
-			q[-2 * s] = clip255(p1 + b);
-			q[s] = clip255(q1 - b);
-			q[-3 * s] = clip255(p2 + c);
-			q[2 * s] = clip255(q2 - c);
+		    iabs(q3 - q2) > interior || iabs(q2 - q1) > interior || iabs(q1 - q0) > interior) {
+			tally_outcome(at, kind, ORC_LF_FAIL_INTERIOR);
 			return;
 		}
+		tally(at, ORC_LF_HEV_CELL(kind, hev_thr));
+		hev = iabs(p1 - p0) > hev_thr || iabs(q1 - q0) > hev_thr;
+		tally_outcome(at, kind, hev ? ORC_LF_HEV : ORC_LF_NO_HEV);
+		if (kind == EDGE_MB && !hev) {
+			int w0 = sclamp(p1 - q1) + 3 * (q0 - p0), w = sclamp(w0);
+			int a = (27 * w + 63) >> 7, b = (18 * w + 63) >> 7, c = (9 * w + 63) >> 7;
+			q[-s] = clip255_n(p0 + a, &clips);
+			q[0] = clip255_n(q0 - a, &clips);
+			q[-2 * s] = clip255_n(p1 + b, &clips);
+			q[s] = clip255_n(q1 - b, &clips);
+			q[-3 * s] = clip255_n(p2 + c, &clips);
+			q[2 * s] = clip255_n(q2 - c, &clips);
+			if (w != w0) tally(at, ORC_LF_SAT_CELL(kind, ORC_LF_SAT_W));
+			if (clips) tally(at, ORC_LF_SAT_CELL(kind, ORC_LF_SAT_CLIP));
+			return;
+		}
+	} else {
+		tally_outcome(at, kind, ORC_LF_SIMPLE_APPLIED);
 	}
 	/* "common" 4-tap adjustment; outer taps used for simple, MB+hev and inner+hev */
 	int outer = (kind != EDGE_INNER) || hev;
 	int a = 3 * (q0 - p0);
 	if (outer) a += sclamp(p1 - q1);
+	if (sclamp(a) != a) tally(at, ORC_LF_SAT_CELL(kind, ORC_LF_SAT_A));
 	a = sclamp(a);
+	if (a + 4 > 127 || a + 3 > 127) tally(at, ORC_LF_SAT_CELL(kind, ORC_LF_SAT_A_ROUND));
 	int f1 = sclamp(a + 4) >> 3, f2 = sclamp(a + 3) >> 3;
-	q[0] = clip255(q0 - f1);
-	q[-s] = clip255(p0 + f2);
+	q[0] = clip255_n(q0 - f1, &clips);
+	q[-s] = clip255_n(p0 + f2, &clips);
 	if (!outer) {
 		int h = (f1 + 1) >> 1;
-		q[s] = clip255(q1 - h);
-		q[-2 * s] = clip255(p1 + h);
+		q[s] = clip255_n(q1 - h, &clips);
+		q[-2 * s] = clip255_n(p1 + h, &clips);
 	}
+	if (clips) tally(at, ORC_LF_SAT_CELL(kind, ORC_LF_SAT_CLIP));
 }
 
 /* n positions along an edge: walk = step along the edge, across = step across it. */
 static void filter_edge(uint8_t* q, ptrdiff_t walk, ptrdiff_t across, int n, int kind, int lim, int interior,
-                        int hev_thr) {
-	for (int i = 0; i < n; i++) filter_pos(q + i * walk, across, kind, lim, interior, hev_thr);
+                        int hev_thr, const LfSite* at) {
+	for (int i = 0; i < n; i++) filter_pos(q + i * walk, across, kind, lim, interior, hev_thr, at);
 }
 
 /* Reference vp8_loopfilter_apply_keyframe (vp8_loopfilter.c:201-283). */
-int orc_loopfilter_padded(const Vp8DecodedFrame* f, uint8_t* y, uint8_t* u, uint8_t* v) {
+int orc_loopfilter_census(const Vp8DecodedFrame* f, uint8_t* y, uint8_t* u, uint8_t* v, uint64_t* counts) {
 	if (!f || !y || !u || !v) {
 		errno = EINVAL;
 		return -1;
@@ -390,6 +426,9 @@ int orc_loopfilter_padded(const Vp8DecodedFrame* f, uint8_t* y, uint8_t* u, uint
 	const uint32_t cols = f->mb_cols, rows = f->mb_rows;
 	const ptrdiff_t sy = (ptrdiff_t)cols * 16, sc = (ptrdiff_t)cols * 8;
 	for (uint32_t my = 0; my < rows; my++) {
+		const LfSite vy = {counts, ORC_LF_VERT, ORC_LF_Y, -1}, vc = {counts, ORC_LF_VERT, ORC_LF_UV, -1};
+		const LfSite hy = {counts, ORC_LF_HORZ, ORC_LF_Y, -1}, hc = {counts, ORC_LF_HORZ, ORC_LF_UV, -1};
+		const LfSite ty = {counts, ORC_LF_HORZ, ORC_LF_Y, (int)(my & 1)}, tc = {counts, ORC_LF_HORZ, ORC_LF_UV, (int)(my & 1)};
 		for (uint32_t mx = 0; mx < cols; mx++) {
 			const size_t mb = (size_t)my * cols + mx;
 			MbFilter m = mb_filter_params(f, mb);
@@ -400,37 +439,43 @@ int orc_loopfilter_padded(const Vp8DecodedFrame* f, uint8_t* y, uint8_t* u, uint
 
 			if (f->lf_use_simple) {
 				const int lim_mb = 2 * (m.level + 2) + m.interior, lim_in = 2 * m.level + m.interior;
-				if (mx) filter_edge(Y, sy, 1, 16, EDGE_SIMPLE, lim_mb, 0, 0);
+				if (mx) filter_edge(Y, sy, 1, 16, EDGE_SIMPLE, lim_mb, 0, 0, &vy);
 				if (inner)
-					for (int e = 4; e < 16; e += 4) filter_edge(Y + e, sy, 1, 16, EDGE_SIMPLE, lim_in, 0, 0);
-				if (my) filter_edge(Y, 1, sy, 16, EDGE_SIMPLE, lim_mb, 0, 0);
+					for (int e = 4; e < 16; e += 4) filter_edge(Y + e, sy, 1, 16, EDGE_SIMPLE, lim_in, 0, 0, &vy);
+				if (my) filter_edge(Y, 1, sy, 16, EDGE_SIMPLE, lim_mb, 0, 0, &ty);
 				if (inner)
-					for (int e = 4; e < 16; e += 4) filter_edge(Y + e * sy, 1, sy, 16, EDGE_SIMPLE, lim_in, 0, 0);
+					for (int e = 4; e < 16; e += 4) filter_edge(Y + e * sy, 1, sy, 16, EDGE_SIMPLE, lim_in, 0, 0, &hy);
 				continue;
 			}
 			const int lim_mb = 2 * (m.level + 2) + m.interior, lim_in = 2 * m.level + m.interior;
 			if (mx) {
-				filter_edge(Y, sy, 1, 16, EDGE_MB, lim_mb, m.interior, m.hev_thr);
-				for (int k = 0; k < 2; k++) filter_edge(C[k], sc, 1, 8, EDGE_MB, lim_mb, m.interior, m.hev_thr);
+				filter_edge(Y, sy, 1, 16, EDGE_MB, lim_mb, m.interior, m.hev_thr, &vy);
+				for (int k = 0; k < 2; k++) filter_edge(C[k], sc, 1, 8, EDGE_MB, lim_mb, m.interior, m.hev_thr, &vc);
 			}
 			if (inner) {
-				for (int e = 4; e < 16; e += 4) filter_edge(Y + e, sy, 1, 16, EDGE_INNER, lim_in, m.interior, m.hev_thr);
-				for (int k = 0; k < 2; k++) filter_edge(C[k] + 4, sc, 1, 8, EDGE_INNER, lim_in, m.interior, m.hev_thr);
+				for (int e = 4; e < 16; e += 4) filter_edge(Y + e, sy, 1, 16, EDGE_INNER, lim_in, m.interior, m.hev_thr, &vy);
+				for (int k = 0; k < 2; k++) filter_edge(C[k] + 4, sc, 1, 8, EDGE_INNER, lim_in, m.interior, m.hev_thr, &vc);
 			}
 			if (my) {
-				filter_edge(Y, 1, sy, 16, EDGE_MB, lim_mb, m.interior, m.hev_thr);
-				for (int k = 0; k < 2; k++) filter_edge(C[k], 1, sc, 8, EDGE_MB, lim_mb, m.interior, m.hev_thr);
+				filter_edge(Y, 1, sy, 16, EDGE_MB, lim_mb, m.interior, m.hev_thr, &ty);
+				for (int k = 0; k < 2; k++) filter_edge(C[k], 1, sc, 8, EDGE_MB, lim_mb, m.interior, m.hev_thr, &tc);
 			}
 			if (inner) {
 				for (int e = 4; e < 16; e += 4)
-					filter_edge(Y + e * sy, 1, sy, 16, EDGE_INNER, lim_in, m.interior, m.hev_thr);
+					filter_edge(Y + e * sy, 1, sy, 16, EDGE_INNER, lim_in, m.interior, m.hev_thr, &hy);
 				for (int k = 0; k < 2; k++)
-					filter_edge(C[k] + 4 * sc, 1, sc, 8, EDGE_INNER, lim_in, m.interior, m.hev_thr);
+					filter_edge(C[k] + 4 * sc, 1, sc, 8, EDGE_INNER, lim_in, m.interior, m.hev_thr, &hc);
 			}
 		}
 	}
 	return 0;
 }
+
+int orc_loopfilter_padded(const Vp8DecodedFrame* f, uint8_t* y, uint8_t* u, uint8_t* v) {
+	return orc_loopfilter_census(f, y, u, v, NULL);
+}
+
+size_t orc_loopfilter_census_cells(void) { return ORC_LF_CELLS; }
 
 /* Reconstruct (+ filter) into padded scratch planes, crop to a tight I420 buffer.
  * Reference vp8_reconstruct_keyframe_yuv_internal (vp8_recon.c:423-712). */

@@ -180,7 +180,8 @@ def test_cluster_mode_one_image_over_several_ctas(gpu_ctx, oracle, ctas, split):
     gpu_ctx.set_cluster(ctas, split)
     try:
         frames = [fuzz_frame(600 + s, 400 + 64 * s, 1100 + 200 * s, density=0.15, lf_level=20 + s, lf_use_simple=0) for s in range(3)]
-        frames.append(fuzz_frame(610, 64, 4000, density=0.2))          # 250 macroblock rows, 4 columns
+        # 250 macroblock rows, 4 columns: the only frame that gives rows to CTAs 4..8; pinned so that it really filters
+        frames.append(fuzz_frame(610, 64, 4000, density=0.2, lf_level=40, lf_delta_enabled=0, lf_use_simple=0))
         frames.append(fuzz_frame(611, 2500, 600, density=0.1, lf_use_simple=1, lf_level=33))
         kfs, ds = [f.header() for f in frames], [f.cstruct() for f in frames]
         for filtered in (False, True):

@@ -226,18 +226,43 @@ class Checker:
     def rgb(self, i420: np.ndarray, w: int, h: int) -> np.ndarray: ...
 
 
+# orc_loopfilter_census cells (oracle/vp8_oracle.h): one named field per cell block, the labels of each axis below
+LF_AXES = {
+    "kind": ("mb", "inner", "simple"),
+    "dir": ("vert", "horz"),
+    "plane": ("y", "uv"),
+    "outcome": ("fail_edge", "fail_interior", "no_hev", "hev", "simple"),
+    "sat": ("w", "a", "a_round", "clip"),
+    "hev_thr": (0, 1, 2),
+    "parity": ("even", "odd"),
+}
+LF_FIELDS = {"outcome": ("kind", "dir", "plane", "outcome"), "sat": ("kind", "sat"), "hev_thr": ("kind", "hev_thr"),
+             "parity": ("parity", "outcome")}
+LF_CENSUS = np.dtype([(k, np.uint64, tuple(len(LF_AXES[a]) for a in axes)) for k, axes in LF_FIELDS.items()])
+
+
+def census_sum(censuses):
+    """Cell-wise sum of loopfilter_census results."""
+    flat = sum(np.asarray(c).reshape(1).view(np.uint64) for c in censuses)
+    return flat.view(LF_CENSUS)[0]
+
+
 class Oracle(Checker):
-    """oracle/liboracle.so: our C restatement."""
+    """oracle/liboracle.so: our C restatement (or a library built from a copy of its source: so)."""
     name = "oracle"
 
-    def __init__(self):
-        so = ORACLE_DIR / "liboracle.so"
-        if not so.exists():
-            build_oracle()
+    def __init__(self, so=None):
+        if so is None:
+            so = ORACLE_DIR / "liboracle.so"
+            if not so.exists():
+                build_oracle()
         L = self.lib = C.CDLL(str(so))
         L.orc_decode_i420.argtypes = [C.POINTER(DecodedFrame), C.c_uint32, C.c_uint32, C.c_int, C.c_void_p]
         L.orc_recon_padded.argtypes = [C.POINTER(DecodedFrame)] + [C.c_void_p] * 3
         L.orc_loopfilter_padded.argtypes = [C.POINTER(DecodedFrame)] + [C.c_void_p] * 3
+        L.orc_loopfilter_census.argtypes = [C.POINTER(DecodedFrame)] + [C.c_void_p] * 4
+        L.orc_loopfilter_census_cells.restype = C.c_size_t
+        assert L.orc_loopfilter_census_cells() * 8 == LF_CENSUS.itemsize
         L.orc_i420_to_rgb.argtypes = [C.c_void_p] * 3 + [C.c_uint32] * 4 + [C.c_void_p]
         L.orc_i420_to_rgb.restype = None
         L.orc_ppm.argtypes = [C.c_void_p, C.c_uint32, C.c_uint32, C.c_void_p]
@@ -272,6 +297,14 @@ class Oracle(Checker):
     def loopfilter_padded(self, fr, y, u, v):
         d = fr.cstruct()
         assert self.lib.orc_loopfilter_padded(C.byref(d), y.ctypes.data, u.ctypes.data, v.ctypes.data) == 0
+
+    def loopfilter_census(self, fr):
+        """Counts of the loop filter's arms over one frame (recon_padded, then the filter): a record of dtype LF_CENSUS."""
+        y, u, v = self.recon_padded(fr)
+        out = np.zeros((), LF_CENSUS)
+        d = fr.cstruct()
+        assert self.lib.orc_loopfilter_census(C.byref(d), y.ctypes.data, u.ctypes.data, v.ctypes.data, out.ctypes.data) == 0
+        return out
 
     def rgb(self, i420, w, h):
         cw, ch = (w + 1) // 2, (h + 1) // 2
