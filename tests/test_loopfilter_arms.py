@@ -1,8 +1,8 @@
 """The loop filter's arms, reached on purpose.
 
 Whether a filter position is modified, and by which arm, depends on the pixels, and the fuzz frames are mostly dense
-random content on which most positions fail the edge or the interior limit. The frames here are built recipe by
-recipe so that every arm of the filter runs many times: both hev outcomes of macroblock and inner edges, the simple
+random content on which most positions fail the edge or the interior limit. The stress set (vp8fix.stress_frame) is
+built recipe by recipe so that every arm of the filter runs many times: both hev outcomes of macroblock and inner edges, the simple
 filter, the clamps of w and a, clip255 at 0 and 255, every hev threshold, skipped inner edges next to filtered ones.
 - CPU: the oracle's arm census (orc_loopfilter_census) of the set stays above a stated floor in every reachable cell,
   and twelve one-line mutants of the oracle's filter each change some output byte of the set.
@@ -13,77 +13,8 @@ import subprocess
 import numpy as np
 import pytest
 
-from vp8fix import LF_AXES, ORACLE_DIR, Frame, Oracle, census_sum, compute_has_coeff, default_params
-
-
-# ------------------------------------------------------------------------------------------------- filter-stress frames
-def stress_frame(recipe: str, seed: int, width: int, height: int) -> Frame:
-    """A frame whose reconstruction drives the loop filter into particular arms. Content is made of i16 macroblocks
-    with Y2 DC/AC (flat 4x4 blocks: steps at block edges), one low-frequency luma AC term per block (ramps: hev),
-    textured macroblocks (dense coefficients: interior-limit failures) and macroblocks without coefficients."""
-    rng = np.random.default_rng(seed)
-    n = ((width + 15) // 16) * ((height + 15) // 16)
-    p = default_params(q_index=int(rng.integers(0, 8)), lf_level=int(rng.integers(20, 64)))
-    # Y2 DC / Y2 AC / luma AC bounds, share of B_PRED, textured and empty macroblocks, Y2 DC offset of every macroblock
-    y2dc, y2ac, ac, bpred, tex, empty, bias = 60, 0, 0, 0.0, 0.0, 0.1, 0
-    if recipe == "smooth":      # small steps between flat blocks: the 27/18/9 arm
-        y2dc, y2ac = 40, 6
-    elif recipe == "ramp":      # gradients inside the blocks: hev, at the levels where the hev threshold changes
-        y2dc, ac = 40, 12
-        p["lf_level"] = int(rng.choice([15, 16, 39, 40, 63]))
-    elif recipe == "steps63":   # large steps, the widest limits: w and a saturate
-        y2dc, y2ac, ac = 400, 30, 4
-        p.update(lf_level=63, lf_sharpness=0)
-    elif recipe == "extremes":  # content pushed to 0 or 255 with texture next to it: clip255 clips
-        y2dc, y2ac, ac, tex, bias = 300, 40, 10, 0.3, int(rng.choice([-600, 600]))
-        p.update(lf_level=63, lf_sharpness=0)
-    elif recipe == "textured":  # smooth macroblocks next to textured partners, every sharpness: interior limit
-        y2dc, ac, tex = 60, 8, 0.5
-        p.update(lf_sharpness=int(rng.integers(0, 8)), lf_level=int(rng.integers(8, 40)))
-    elif recipe == "simple":
-        y2dc, y2ac, ac, tex = 60, 8, 8, 0.2
-        p.update(lf_use_simple=1, lf_level=int(rng.integers(10, 64)), lf_sharpness=int(rng.integers(0, 8)))
-    elif recipe == "segments":  # per-segment levels (some 0), B_PRED mode delta, B_PRED without coefficients
-        y2dc, y2ac, ac, tex, bpred, empty = 60, 8, 8, 0.2, 0.4, 0.3
-        p.update(segmentation_enabled=1, segmentation_abs=int(rng.integers(0, 2)), lf_delta_enabled=1, lf_sharpness=4,
-                 lf_ref_delta=[int(rng.integers(-10, 10)), 0, 0, 0], lf_mode_delta=[int(rng.integers(-20, 21)), 0, 0, 0])
-        p["seg_lf_level"] = [0, 15, 40, 63] if p["segmentation_abs"] else [-63, -5, 0, 20]
-    else:
-        raise ValueError(recipe)
-    a = {
-        "segment_id": rng.integers(0, 4, n).astype(np.uint8),
-        "skip_coeff": np.zeros(n, np.uint8),
-        "ymode": np.where(rng.random(n) < bpred, 4, rng.integers(0, 4, n)).astype(np.uint8),
-        "uv_mode": rng.integers(0, 4, n).astype(np.uint8),
-        "bmode": rng.integers(0, 10, n * 16).astype(np.uint8),
-    }
-    y2 = np.zeros((n, 16), np.int16)
-    y2[:, 0] = bias + rng.integers(-y2dc, y2dc + 1, n)
-    y2[:, 1:] = rng.integers(-y2ac, y2ac + 1, (n, 15)) * (rng.random((n, 15)) < 0.3)
-    yy = np.zeros((n, 16, 16), np.int16)
-    yy[:, :, 0] = rng.integers(-y2dc // 4, y2dc // 4 + 1, (n, 16))  # DC of B_PRED blocks (compute_has_coeff clears it for i16)
-    term = np.where(rng.random((n, 16)) < 0.5, 1, 4)                  # first horizontal or first vertical AC term
-    np.put_along_axis(yy, term[..., None], rng.integers(-ac, ac + 1, (n, 16, 1)), axis=2)
-    t = rng.random(n) < tex
-    yy[t] = rng.integers(-60, 61, (int(t.sum()), 16, 16))
-    uv = [np.zeros((n, 4, 16), np.int16) for _ in range(2)]
-    for c in uv:
-        c[:, :, 0] = rng.integers(-20, 21, (n, 4))
-        c[t] = rng.integers(-40, 41, (int(t.sum()), 4, 16))
-    e = rng.random(n) < empty
-    y2[e], yy[e], uv[0][e], uv[1][e] = 0, 0, 0, 0
-    a.update(coeff_y2=y2.reshape(-1), coeff_y=yy.reshape(-1), coeff_u=uv[0].reshape(-1), coeff_v=uv[1].reshape(-1))
-    a["has_coeff"] = compute_has_coeff(a, n)
-    return Frame(width, height, p, a)
-
-
-RECIPES = ("smooth", "ramp", "steps63", "extremes", "textured", "simple", "segments")
-# widths that are not a multiple of 16, single macroblock columns and rows, a frame wider than 1000 px
-SIZES = ((160, 96), (100, 72), (16, 200), (9, 130), (300, 16), (200, 12), (1040, 40), (96, 160))
-# 512 macroblock rows, 2 columns: the 8 CTAs x 16 warps of a fused cluster of 8 deal 2-row pairs round-robin, so every
-# CTA gets rows and every warp takes a second pair (more than 2 * 255 rows); every 16-row band must really filter
-TALL = ("ramp", 999, 24, 8192)
-STRESS = tuple((r, 100 * i + j, *SIZES[(4 * i + j) % len(SIZES)]) for i, r in enumerate(RECIPES) for j in range(4)) + (TALL,)
+from vp8fix import (LF_AXES, ORACLE_DIR, SHAPES, STRESS, TALL, Oracle, census_sum, expected_launch, first_difference, launch_of,
+                    reset_shape, set_shape, shape_batches, stress_frame)
 
 
 @pytest.fixture(scope="module")
@@ -213,18 +144,6 @@ def test_every_filter_mutant_changes_the_stress_set(oracle, stress, tmp_path):
 
 
 # ---------------------------------------------------------------------------------------- GPU: every wavefront shape
-DEFAULT_KERNEL = 3  # what a fresh context runs (vp8_gpu.h: vp8_gpu_set_kernel)
-
-# (kernel, warps, images per SM, CTAs per image, split) -> expected last_launch_config of the fused decode
-SHAPES = [(2, w, 0, 1, False) for w in (4, 8, 16)]  # vp8_mb_pairs<NW, ..., LS=false>
-# kernel 3 + 8 warps + images_per_cta == 0 is the 8-warp lockstep-small pairs shape, vp8_mb_pairs<8, ..., LS=true>; no
-# field of the launch config reports LS itself
-SHAPES += [(3, 8, 0, 1, False)]
-# g = 1: vp8_mb_pairs<4>; g >= 2: vp8_mb_lockstep with g images per CTA
-SHAPES += [(3, 4, g, 1, False) for g in range(1, 8)]
-SHAPES += [(3, 16, 0, c, False) for c in (2, 4, 8)] + [(3, 16, 0, c, True) for c in (4, 8)]
-
-
 @pytest.fixture(scope="module")
 def oracle_out(oracle, stress):
     """The oracle's I420 (unfiltered, filtered) and padded planes (reconstructed + filtered) of every stress frame."""
@@ -236,48 +155,22 @@ def oracle_out(oracle, stress):
     return out
 
 
-def first_difference(f, got, want, padded=False):
-    """plane / x / y / macroblock of the first differing byte of an I420 buffer, or of padded (y, u, v) planes."""
-    if padded:
-        planes = list(zip("yuv", got, want))
-    else:
-        w, h, cw, ch = f.width, f.height, (f.width + 1) // 2, (f.height + 1) // 2
-        cut = lambda b: (b[:w * h].reshape(h, w), b[w * h:w * h + cw * ch].reshape(ch, cw), b[w * h + cw * ch:].reshape(ch, cw))
-        planes = list(zip("yuv", cut(got), cut(want)))
-    for name, g, wnt in planes:
-        bad = np.argwhere(g != wnt)
-        if len(bad):
-            y, x = (int(v) for v in bad[0])
-            mb = 16 if name == "y" else 8
-            return f"plane {name} x={x} y={y} macroblock ({x // mb}, {y // mb}): got {g[y, x]} want {wnt[y, x]}"
-    return "no difference"
-
-
 @pytest.mark.gpu
 @pytest.mark.parametrize("kernel,warps,per_sm,ctas,split", SHAPES)
 def test_every_wavefront_shape_on_the_stress_set(gpu_ctx, stress, oracle_out, kernel, warps, per_sm, ctas, split):
     """Fused recon + filter (filtered and not) and the staged recon() -> filter() in one launch shape, against the oracle.
     Clusters run in batches of up to 7 frames that each hold the tall frame, so that they stay clusters (as many as are
     resident at once) and every CTA of a cluster gets filtered rows."""
-    idx = list(range(len(stress)))
-    if ctas > 1:
-        small = idx[:-1]
-        batches = [small[i:i + 6] + [idx[-1]] for i in range(0, len(small), 6)]
-    else:
-        batches = [idx]
-    gpu_ctx.set_kernel(kernel)
-    gpu_ctx.set_tuning(warps, per_sm)
-    gpu_ctx.set_cluster(ctas, split)
+    shape = (kernel, warps, per_sm, ctas, split)
+    set_shape(gpu_ctx, shape)
     try:
-        for batch in batches:
+        for batch in shape_batches(len(stress), len(stress) - 1, ctas):
             frames = [stress[i] for i in batch]
             kfs, ds = [f.header() for f in frames], [f.cstruct() for f in frames]
-            shape = (kernel, warps, per_sm, ctas, split)
             for filtered in (False, True):
                 outs = gpu_ctx.decode_i420(kfs, ds, filtered=filtered)
                 cfg = gpu_ctx.last_launch_config()
-                assert (cfg["warps_per_image"], cfg["ctas_per_image"], cfg["split"]) == (warps, ctas, split), (shape, cfg)
-                assert cfg["images_per_cta"] == (per_sm if per_sm >= 2 else 0), (shape, cfg)
+                assert launch_of(cfg) == expected_launch(shape), (shape, cfg)
                 for i, f, o in zip(batch, frames, outs):
                     want = oracle_out[i][filtered]
                     assert np.array_equal(o, want), (f"shape {shape} filtered={filtered} recipe {STRESS[i][0]} "
@@ -287,8 +180,7 @@ def test_every_wavefront_shape_on_the_stress_set(gpu_ctx, stress, oracle_out, ke
             try:
                 gpu_ctx.filter(b)
                 cfg = gpu_ctx.last_launch_config()
-                assert (cfg["warps_per_image"], cfg["ctas_per_image"], cfg["split"]) == (warps, ctas, False), (shape, cfg)
-                assert cfg["images_per_cta"] == (per_sm if per_sm >= 2 else 0), (shape, cfg)
+                assert launch_of(cfg) == expected_launch(shape, staged_filter=True), (shape, cfg)
                 for k, (i, f) in enumerate(zip(batch, frames)):
                     got, want = gpu_ctx.download_padded(b, k), oracle_out[i]["padded"]
                     assert all(np.array_equal(g, w) for g, w in zip(got, want)), (
@@ -297,6 +189,4 @@ def test_every_wavefront_shape_on_the_stress_set(gpu_ctx, stress, oracle_out, ke
             finally:
                 b.free()
     finally:
-        gpu_ctx.set_cluster(0, True)
-        gpu_ctx.set_tuning(0, 0)
-        gpu_ctx.set_kernel(DEFAULT_KERNEL)
+        reset_shape(gpu_ctx)

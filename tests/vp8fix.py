@@ -199,6 +199,76 @@ def fuzz_frame(seed: int, width: int, height: int, *, density: float = 0.2, amp:
     return Frame(width, height, p, a)
 
 
+def stress_frame(recipe: str, seed: int, width: int, height: int) -> Frame:
+    """A frame whose reconstruction drives the loop filter into particular arms. Content is made of i16 macroblocks
+    with Y2 DC/AC (flat 4x4 blocks: steps at block edges), one low-frequency luma AC term per block (ramps: hev),
+    textured macroblocks (dense coefficients: interior-limit failures) and macroblocks without coefficients."""
+    rng = np.random.default_rng(seed)
+    n = ((width + 15) // 16) * ((height + 15) // 16)
+    p = default_params(q_index=int(rng.integers(0, 8)), lf_level=int(rng.integers(20, 64)))
+    # Y2 DC / Y2 AC / luma AC bounds, share of B_PRED, textured and empty macroblocks, Y2 DC offset of every macroblock
+    y2dc, y2ac, ac, bpred, tex, empty, bias = 60, 0, 0, 0.0, 0.0, 0.1, 0
+    if recipe == "smooth":      # small steps between flat blocks: the 27/18/9 arm
+        y2dc, y2ac = 40, 6
+    elif recipe == "ramp":      # gradients inside the blocks: hev, at the levels where the hev threshold changes
+        y2dc, ac = 40, 12
+        p["lf_level"] = int(rng.choice([15, 16, 39, 40, 63]))
+    elif recipe == "steps63":   # large steps, the widest limits: w and a saturate
+        y2dc, y2ac, ac = 400, 30, 4
+        p.update(lf_level=63, lf_sharpness=0)
+    elif recipe == "extremes":  # content pushed to 0 or 255 with texture next to it: clip255 clips
+        y2dc, y2ac, ac, tex, bias = 300, 40, 10, 0.3, int(rng.choice([-600, 600]))
+        p.update(lf_level=63, lf_sharpness=0)
+    elif recipe == "textured":  # smooth macroblocks next to textured partners, every sharpness: interior limit
+        y2dc, ac, tex = 60, 8, 0.5
+        p.update(lf_sharpness=int(rng.integers(0, 8)), lf_level=int(rng.integers(8, 40)))
+    elif recipe == "simple":
+        y2dc, y2ac, ac, tex = 60, 8, 8, 0.2
+        p.update(lf_use_simple=1, lf_level=int(rng.integers(10, 64)), lf_sharpness=int(rng.integers(0, 8)))
+    elif recipe == "segments":  # per-segment levels (some 0), B_PRED mode delta, B_PRED without coefficients
+        y2dc, y2ac, ac, tex, bpred, empty = 60, 8, 8, 0.2, 0.4, 0.3
+        p.update(segmentation_enabled=1, segmentation_abs=int(rng.integers(0, 2)), lf_delta_enabled=1, lf_sharpness=4,
+                 lf_ref_delta=[int(rng.integers(-10, 10)), 0, 0, 0], lf_mode_delta=[int(rng.integers(-20, 21)), 0, 0, 0])
+        p["seg_lf_level"] = [0, 15, 40, 63] if p["segmentation_abs"] else [-63, -5, 0, 20]
+    else:
+        raise ValueError(recipe)
+    a = {
+        "segment_id": rng.integers(0, 4, n).astype(np.uint8),
+        "skip_coeff": np.zeros(n, np.uint8),
+        "ymode": np.where(rng.random(n) < bpred, 4, rng.integers(0, 4, n)).astype(np.uint8),
+        "uv_mode": rng.integers(0, 4, n).astype(np.uint8),
+        "bmode": rng.integers(0, 10, n * 16).astype(np.uint8),
+    }
+    y2 = np.zeros((n, 16), np.int16)
+    y2[:, 0] = bias + rng.integers(-y2dc, y2dc + 1, n)
+    y2[:, 1:] = rng.integers(-y2ac, y2ac + 1, (n, 15)) * (rng.random((n, 15)) < 0.3)
+    yy = np.zeros((n, 16, 16), np.int16)
+    yy[:, :, 0] = rng.integers(-y2dc // 4, y2dc // 4 + 1, (n, 16))  # DC of B_PRED blocks (compute_has_coeff clears it for i16)
+    term = np.where(rng.random((n, 16)) < 0.5, 1, 4)                  # first horizontal or first vertical AC term
+    np.put_along_axis(yy, term[..., None], rng.integers(-ac, ac + 1, (n, 16, 1)), axis=2)
+    t = rng.random(n) < tex
+    yy[t] = rng.integers(-60, 61, (int(t.sum()), 16, 16))
+    uv = [np.zeros((n, 4, 16), np.int16) for _ in range(2)]
+    for c in uv:
+        c[:, :, 0] = rng.integers(-20, 21, (n, 4))
+        c[t] = rng.integers(-40, 41, (int(t.sum()), 4, 16))
+    e = rng.random(n) < empty
+    y2[e], yy[e], uv[0][e], uv[1][e] = 0, 0, 0, 0
+    a.update(coeff_y2=y2.reshape(-1), coeff_y=yy.reshape(-1), coeff_u=uv[0].reshape(-1), coeff_v=uv[1].reshape(-1))
+    a["has_coeff"] = compute_has_coeff(a, n)
+    return Frame(width, height, p, a)
+
+
+RECIPES = ("smooth", "ramp", "steps63", "extremes", "textured", "simple", "segments")
+# widths that are not a multiple of 16, single macroblock columns and rows, a frame wider than 1000 px
+SIZES = ((160, 96), (100, 72), (16, 200), (9, 130), (300, 16), (200, 12), (1040, 40), (96, 160))
+# 512 macroblock rows, 2 columns: the 8 CTAs x 16 warps of a fused cluster of 8 deal 2-row pairs round-robin, so every
+# CTA gets rows and every warp takes a second pair (more than 2 * 255 rows); every 16-row band must really filter
+TALL = ("ramp", 999, 24, 8192)
+# the loop-filter stress set (tests/test_loopfilter_arms.py), its tall frame last
+STRESS = tuple((r, 100 * i + j, *SIZES[(4 * i + j) % len(SIZES)]) for i, r in enumerate(RECIPES) for j in range(4)) + (TALL,)
+
+
 def compute_has_coeff(a, n):
     """has_coeff as the host token parser defines it (reference vp8_tokens.c:331-339,604): any decoded
     coefficient of the macroblock non-zero. Y2 only counts where it is coded (ymode != B_PRED), and for
@@ -212,6 +282,70 @@ def compute_has_coeff(a, n):
     nz = (y2 != 0).any(1) | (yy != 0).any((1, 2)) | (a["coeff_u"].reshape(n, 64) != 0).any(1) | \
         (a["coeff_v"].reshape(n, 64) != 0).any(1)
     return nz.astype(np.uint8)
+
+
+def first_difference(f, got, want, padded=False):
+    """plane / x / y / macroblock of the first differing byte of an I420 buffer, or of padded (y, u, v) planes."""
+    if padded:
+        planes = list(zip("yuv", got, want))
+    else:
+        w, h, cw, ch = f.width, f.height, (f.width + 1) // 2, (f.height + 1) // 2
+        cut = lambda b: (b[:w * h].reshape(h, w), b[w * h:w * h + cw * ch].reshape(ch, cw), b[w * h + cw * ch:].reshape(ch, cw))
+        planes = list(zip("yuv", cut(got), cut(want)))
+    for name, g, wnt in planes:
+        bad = np.argwhere(g != wnt)
+        if len(bad):
+            y, x = (int(v) for v in bad[0])
+            mb = 16 if name == "y" else 8
+            return f"plane {name} x={x} y={y} macroblock ({x // mb}, {y // mb}): got {g[y, x]} want {wnt[y, x]}"
+    return "no difference"
+
+
+# ---------------------------------------------------------------------------- wavefront kernel shapes
+DEFAULT_KERNEL = 3  # what a fresh context runs (vp8_gpu.h: vp8_gpu_set_kernel)
+
+# (kernel, warps, images per SM, CTAs per image, split): set_kernel / set_tuning / set_cluster of a context
+SHAPES = [(2, w, 0, 1, False) for w in (4, 8, 16)]  # vp8_mb_pairs<NW, ..., LS=false>
+# kernel 3 + 8 warps + images_per_cta == 0 is the 8-warp lockstep-small pairs shape, vp8_mb_pairs<8, ..., LS=true>; no
+# field of the launch config reports LS itself
+SHAPES += [(3, 8, 0, 1, False)]
+# g = 1: vp8_mb_pairs<4>; g >= 2: vp8_mb_lockstep with g images per CTA
+SHAPES += [(3, 4, g, 1, False) for g in range(1, 8)]
+SHAPES += [(3, 16, 0, c, False) for c in (2, 4, 8)] + [(3, 16, 0, c, True) for c in (4, 8)]
+
+
+def set_shape(ctx, shape):
+    kernel, warps, per_sm, ctas, split = shape
+    ctx.set_kernel(kernel)
+    ctx.set_tuning(warps, per_sm)
+    ctx.set_cluster(ctas, split)
+
+
+def reset_shape(ctx):
+    ctx.set_cluster(0, True)
+    ctx.set_tuning(0, 0)
+    ctx.set_kernel(DEFAULT_KERNEL)
+
+
+def expected_launch(shape, staged_filter=False):
+    """(warps_per_image, ctas_per_image, split, images_per_cta) that last_launch_config reports for a launch in `shape`
+    (the stand-alone filter never runs the split flavour)."""
+    kernel, warps, per_sm, ctas, split = shape
+    return warps, ctas, split and not staged_filter, per_sm if per_sm >= 2 else 0
+
+
+def launch_of(cfg):
+    return cfg["warps_per_image"], cfg["ctas_per_image"], cfg["split"], cfg["images_per_cta"]
+
+
+def shape_batches(n, tall, ctas):
+    """Index batches of n frames for one shape: all at once, or for clusters batches of up to 7 frames that each hold
+    frame `tall` (enough macroblock rows that every CTA of the cluster gets some; at most 7 frames, so that all the
+    clusters are resident at once and the planner keeps the cluster size)."""
+    if ctas <= 1:
+        return [list(range(n))]
+    rest = [i for i in range(n) if i != tall]
+    return [rest[i:i + 6] + [tall] for i in range(0, len(rest), 6)]
 
 
 # ---------------------------------------------------------------------------- CPU checkers

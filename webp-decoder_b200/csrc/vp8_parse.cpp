@@ -269,13 +269,16 @@ struct CompactSink {
 	uint32_t cur = 0, blocks = 0;
 	alignas(32) int16_t y2[16];
 	bool y2_nz = false;
+	bool failed = false; // a granule did not fit: [pos, end) lies past the capacity, nothing more is written
 
 	bool room() {
+		if (failed) return false;
 		if (end - pos >= vp8c::kMbWorst + 32) return true; // done() zeroes one slot ahead
 		if (!cursor) return false;
 		pos = cursor->fetch_add(vp8c::kGranule);
 		end = pos + vp8c::kGranule;
-		return end <= capacity;
+		failed = end > capacity;
+		return !failed;
 	}
 	bool begin_ok = true;
 	void begin_mb(size_t i) {
