@@ -213,6 +213,20 @@ int vp8_gpu_decode_webp(vp8_gpu_ctx* ctx, const uint8_t* const* files, const siz
                         uint8_t* dst, size_t cap, size_t* offsets, size_t* sizes, int chunk);
 size_t vp8_gpu_decode_webp_bytes(const uint8_t* const* files, const size_t* file_sizes, int n, int ppm);
 
+/* Lossy WebP with alpha: .webp bytes in, dwebp's -pam files out ("P7\nWIDTH <w>\nHEIGHT <h>\nDEPTH 4\nMAXVAL 255\n
+ * TUPLTYPE RGB_ALPHA\nENDHDR\n" + w * h * 4 bytes RGBA, not premultiplied). Accepts simple files (alpha 255) and the extended
+ * layout VP8X [+ ALPH] + 'VP8 ' under the container rules of vp8_parse_webp_info (include/vp8_parse.h). The RGB is exactly what
+ * the -ppm output of vp8_gpu_decode_webp gives for the same 'VP8 ' chunk. Same pipelining, chunking, processing order (always
+ * read offsets[]) and errors as vp8_gpu_decode_webp: a file that fails to parse fails the call with its errno. The parser
+ * threads also decode each ALPH payload (raw, or VP8L: the green channel of its image stream) into the chunk's pinned arena,
+ * so the plane travels with the chunk's one upload; the alpha filter is undone on the device and the RGBA pixels are written
+ * by the m08 kernel's 4-byte flavour. The VP8L decode counts as host work in vp8_gpu_last_call_profile. The existing calls are
+ * unchanged: vp8_gpu_decode_webp and its relatives still reject an extended file with EINVAL.
+ * vp8_gpu_decode_webp_rgba_bytes gives the capacity needed (0 if a file is not accepted). */
+int vp8_gpu_decode_webp_rgba(vp8_gpu_ctx* ctx, const uint8_t* const* files, const size_t* file_sizes, int n, uint8_t* dst, size_t cap,
+                             size_t* offsets, size_t* sizes, int chunk);
+size_t vp8_gpu_decode_webp_rgba_bytes(const uint8_t* const* files, const size_t* file_sizes, int n);
+
 /* Where a pipelined call of this context spent its host time (milliseconds, last call): total, host work on the chunks
  * (compaction of dense frames / gather / parsing), waiting for staging slots and retiring chunks. */
 int vp8_gpu_last_call_profile(const vp8_gpu_ctx* ctx, double* total_ms, double* host_work_ms, double* wait_ms);
@@ -245,6 +259,8 @@ int vp8_gpu_kernel_time(vp8_gpu_ctx* ctx, double* total_ms, int* launches);
 /* Same for the m08 (RGB) launches of vp8_gpu_rgb / vp8_gpu_decode_ppm, and for the m09 launch pairs of vp8_gpu_png. */
 int vp8_gpu_rgb_time(vp8_gpu_ctx* ctx, double* total_ms, int* launches);
 int vp8_gpu_png_time(vp8_gpu_ctx* ctx, double* total_ms, int* launches);
+/* Same for the launches of vp8_gpu_decode_webp_rgba: the alpha unfilter kernel and the RGBA flavour of m08. */
+int vp8_gpu_alpha_time(vp8_gpu_ctx* ctx, double* total_ms, int* launches);
 
 /* Host-side per-frame parameter derivation, exported so tests can pin it against the oracle:
  * dq[4][6] = {y1dc,y1ac,uvdc,uvac,y2dc,y2ac} per segment (vp8_recon.c:57-76);

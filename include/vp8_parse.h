@@ -83,6 +83,22 @@ int vp8_parse_batch_compact(const uint8_t* const* files, const size_t* sizes, in
  * (base = new_start, head_off = 0). */
 void vp8_compact_rebase(Vp8CompactFrame* f, void* new_start);
 
+/* ---------------------------------------------------------------- lossy files with alpha (webp_alpha.cpp)
+ * Every call above keeps the reference's rules and rejects the extended layout with EINVAL. The two calls below, and
+ * vp8_gpu_decode_webp_rgba (vp8_gpu.h), also accept it (RFC 9649): 'VP8X' first, at most one 'ALPH' before the 'VP8 '
+ * chunk, 'ICCP' / 'EXIF' / 'XMP ' and unknown chunks skipped; the VP8X canvas must equal the frame size (EINVAL). The
+ * animation flag, 'ANIM' / 'ANMF' and 'VP8L' images give ENOTSUP. An ALPH header with reserved bits set, compression > 1
+ * or pre-processing > 1 is EINVAL; the pre-processing hint is otherwise ignored (no alpha dithering, as libwebp by
+ * default). A VP8L-compressed plane that is truncated, uses incomplete or over-subscribed codes, copies from before the
+ * start or has bad transform parameters is EINVAL.
+ *
+ * Frame size of a simple or extended file, and whether it carries an ALPH chunk. */
+int vp8_parse_webp_info(const uint8_t* file, size_t size, uint32_t* width, uint32_t* height, int* has_alpha);
+
+/* The file's alpha plane, unfiltered, width * height bytes into alpha[0 .. cap): what the RGBA output carries as its 4th
+ * byte. A file without ALPH gives 255 everywhere. Decoded and unfiltered on the calling thread. */
+int vp8_parse_alpha(const uint8_t* file, size_t size, uint8_t* alpha, size_t cap);
+
 #ifdef __cplusplus
 }
 #endif

@@ -53,6 +53,7 @@ EXPORTS = [
     "vp8_gpu_png", "vp8_gpu_png_bytes", "vp8_gpu_download_png", "vp8_gpu_decode_png", "vp8_gpu_png_time", "vp8_gpu_set_png_deflate",
     "vp8_gpu_set_cluster", "vp8_gpu_set_cluster_split", "vp8_gpu_last_split", "vp8_gpu_last_cluster", "vp8_gpu_last_groups", "vp8_gpu_last_segments",
     "vp8_gpu_decode_compact", "vp8_gpu_decode_webp", "vp8_gpu_decode_webp_bytes", "vp8_gpu_last_call_profile", "vp8_gpu_bind_host", "vp8_gpu_last_transport", "vp8_gpu_last_dense_frames",
+    "vp8_gpu_decode_webp_rgba", "vp8_gpu_decode_webp_rgba_bytes", "vp8_gpu_alpha_time", "vp8_parse_webp_info", "vp8_parse_alpha",
     # encoder in-loop reconstruction (include/vp8_enc.h)
     "enc_vp8_encode_dc_pred_inloop", "enc_vp8_encode_i16x16_uv_sad_inloop", "enc_vp8_encode_i16x16_sad_inloop",
     "enc_vp8_encode_bpred_uv_sad_inloop", "vp8_gpu_enc_i16_inloop", "vp8_gpu_enc_bpred_inloop", "vp8_gpu_enc_mb_total",
@@ -135,6 +136,10 @@ def load_library() -> C.CDLL:
     L.vp8_gpu_decode_webp.argtypes = [vp, pp, vp, C.c_int, C.c_int, C.c_int, vp, sz, vp, vp, C.c_int]
     L.vp8_gpu_decode_webp_bytes.argtypes = [pp, vp, C.c_int, C.c_int]
     L.vp8_gpu_decode_webp_bytes.restype = sz
+    L.vp8_gpu_decode_webp_rgba.argtypes = [vp, pp, vp, C.c_int, vp, sz, vp, vp, C.c_int]
+    L.vp8_gpu_decode_webp_rgba_bytes.argtypes = [pp, vp, C.c_int]
+    L.vp8_gpu_decode_webp_rgba_bytes.restype = sz
+    L.vp8_gpu_alpha_time.argtypes = [vp, C.POINTER(C.c_double), C.POINTER(C.c_int)]
     L.vp8_gpu_last_call_profile.argtypes = [vp, C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(C.c_double)]
     L.vp8_gpu_bind_host.argtypes = [vp, C.c_int, C.c_int]
     L.vp8_gpu_last_transport.argtypes = [vp, C.POINTER(C.c_int), C.POINTER(C.c_int)]
@@ -401,6 +406,19 @@ class Context:
     def decode_webp_bytes(self, files: "WebpFiles", ppm: bool = False) -> int:
         return int(self._L.vp8_gpu_decode_webp_bytes(files.ptrs, files.sizes, files.n, _fmt(ppm)))
 
+    def decode_webp_rgba_into(self, files: "WebpFiles", out: np.ndarray, chunk: int = 0):
+        """vp8_gpu_decode_webp_rgba: .webp bytes in (simple, or VP8X with an ALPH chunk), dwebp's -pam files out (RGBA,
+        alpha 255 for files without one); frame i is out[offsets[i]:offsets[i]+sizes[i]]. Returns (offsets, sizes)."""
+        assert out.dtype == np.uint8 and out.flags.c_contiguous
+        offs, sizes = np.zeros(files.n, np.uint64), np.zeros(files.n, np.uint64)
+        _check(self._L.vp8_gpu_decode_webp_rgba(self._h, files.ptrs, files.sizes, files.n, out.ctypes.data, out.nbytes, offs.ctypes.data,
+                                                sizes.ctypes.data, chunk), "vp8_gpu_decode_webp_rgba")
+        return offs, sizes
+
+    def decode_webp_rgba_bytes(self, files: "WebpFiles") -> int:
+        """Capacity decode_webp_rgba_into needs (0 if a file is not accepted)."""
+        return int(self._L.vp8_gpu_decode_webp_rgba_bytes(files.ptrs, files.sizes, files.n))
+
     def last_call_profile(self):
         t, h, w = C.c_double(), C.c_double(), C.c_double()
         _check(self._L.vp8_gpu_last_call_profile(self._h, C.byref(t), C.byref(h), C.byref(w)), "vp8_gpu_last_call_profile")
@@ -473,6 +491,12 @@ class Context:
         """(total_ms, launch pairs) of the m09 launches (vp8_png_frame + vp8_png_finish) since the previous call."""
         ms, n = C.c_double(), C.c_int()
         _check(self._L.vp8_gpu_png_time(self._h, C.byref(ms), C.byref(n)), "vp8_gpu_png_time")
+        return ms.value, n.value
+
+    def alpha_time(self):
+        """(total_ms, launches) of the alpha unfilter and RGBA launches of decode_webp_rgba_into since the previous call."""
+        ms, n = C.c_double(), C.c_int()
+        _check(self._L.vp8_gpu_alpha_time(self._h, C.byref(ms), C.byref(n)), "vp8_gpu_alpha_time")
         return ms.value, n.value
 
     def last_launch_config(self):

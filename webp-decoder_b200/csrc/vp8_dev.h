@@ -57,7 +57,15 @@ struct Vp8RgbDesc {
 	uint8_t* rgb;
 	uint32_t width, height;
 	uint32_t stride_y, stride_uv;
-	uint32_t pad_[2];
+	const uint8_t* alpha; // RGBA flavour: the unfiltered alpha plane (width x height, tight), or null for alpha 255
+};
+
+// Work item of the alpha unfilter kernel (vp8_alpha.cu): one filtered ALPH plane, tight, unfiltered in place.
+struct Vp8AlphaDesc {
+	uint8_t* plane;
+	uint32_t width, height;
+	uint32_t method; // 1 horizontal, 2 vertical, 3 gradient (0: nothing to do)
+	uint32_t pad_;
 };
 
 // Work item of the PNG framing kernels (vp8_png.cu): one RGB24 image in, the reference's -png file out.
@@ -107,8 +115,11 @@ int vp8_launch_lockstep(int mode, const Vp8ImgDesc* descs_dev, int n_images, int
                         void* stream);
 int vp8_lockstep_smem_bytes(int groups, int max_mb_cols);
 int vp8_lockstep_max_groups(int max_mb_cols); // how many groups fit in the shared memory of one SM for this frame width (0: none)
-// m08 (vp8_rgb.cu). tiles_per_image: host array, vp8_rgb_tiles() of every image.
-int vp8_launch_rgb(const Vp8RgbDesc* descs_dev, int n_images, const uint32_t* tiles_per_image, void* stream);
+// m08 (vp8_rgb.cu). tiles_per_image: host array, vp8_rgb_tiles() of every image. rgba != 0: 4-byte pixels, the 4th byte from
+// the descriptor's alpha plane (255 without one).
+int vp8_launch_rgb(const Vp8RgbDesc* descs_dev, int n_images, const uint32_t* tiles_per_image, int rgba, void* stream);
+// Alpha unfilter (vp8_alpha.cu): one CTA per plane.
+int vp8_launch_alpha_unfilter(const Vp8AlphaDesc* descs_dev, int n_planes, void* stream);
 uint32_t vp8_rgb_tiles(uint32_t width, uint32_t height);
 // m09 (vp8_png.cu). Host side: vp8_png_tables() builds the checksum tables (copy vp8_png_tables_bytes() to the device once),
 // vp8_png_fill_desc() completes a descriptor whose width / height are set; first_cta = running sum of vp8_png_ctas().

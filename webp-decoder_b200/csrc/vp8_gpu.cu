@@ -55,6 +55,8 @@ constexpr size_t kAlign = 256;
 constexpr size_t kBounceBytes = 32u << 20;
 constexpr int kCompactMinThreads = 8; // automatic transport of dense frames: compact when the context has at least this many host threads
 constexpr int kPpmSlot = 32; // header slot in front of each RGB image; RGB starts 32 bytes into the slot
+constexpr int kPamSlot = 128; // same for the -pam header of vp8_gpu_decode_webp_rgba (at most 73 bytes)
+constexpr int kOutPam = 3;    // internal output format of vp8_gpu_decode_webp_rgba; never a value of the `ppm` arguments
 constexpr uint64_t kArenaMagic = 0x564138415245414eull; // stats_opaque[21] of frames whose arrays vp8_parse carved from ONE block
                                                         // ([22] = base address, [23] = bytes); same constant in vp8_parse.cpp
 
@@ -161,6 +163,7 @@ struct vp8_gpu_ctx {
 	std::vector<std::pair<cudaEvent_t, cudaEvent_t>> timed; // recorded, not yet read
 	std::vector<std::pair<cudaEvent_t, cudaEvent_t>> timed_rgb; // same for the m08 launches
 	std::vector<std::pair<cudaEvent_t, cudaEvent_t>> timed_png; // same for the m09 launches
+	std::vector<std::pair<cudaEvent_t, cudaEvent_t>> timed_alpha; // same for the alpha unfilter and RGBA launches
 	void* d_png_tables = nullptr;                               // checksum tables of the m09 kernels (first vp8_gpu_png)
 	bool png_deflate = false;                                   // -png files filtered and run-length deflated (vp8_gpu_set_png_deflate)
 	uint32_t* zlens = nullptr;                                  // pinned: per-file lengths of a pipelined deflate call, one per frame
@@ -204,7 +207,9 @@ struct FrameMeta {
 	bool has_seg, has_hc;
 	size_t tight_off;   // tight I420 (Y|U|V) within d_tight
 	size_t pad_off[3];  // padded planes within d_pad
-	size_t rgb_off;     // slot within d_rgb (RGB at +kPpmSlot)
+	size_t rgb_off;     // slot within d_rgb (RGB at +kPpmSlot, RGBA at +kPamSlot)
+	size_t alpha_off = SIZE_MAX; // RGBA batches: the frame's alpha plane within d_in (filtered until the unfilter kernel ran)
+	uint32_t alpha_method = 0;   // its ALPH filter
 	int16_t dq[4][6];
 	uint8_t lf[4][2][4];
 	uint8_t lf_simple;
@@ -241,6 +246,9 @@ struct vp8_gpu_batch {
 	uint32_t pngz_rows = 0, pngz_pieces = 0;
 	bool pngzdesc_up = false;
 	bool png_z = false; // d_png holds compressed files, back to back (the last vp8_gpu_png ran with deflate on)
+	bool rgba = false;  // d_rgb holds -pam slots: RGBA at kPamSlot (vp8_gpu_decode_webp_rgba)
+	Vp8AlphaDesc* d_alphadesc = nullptr; // the planes the unfilter kernel works on
+	int n_alpha = 0;
 	int max_mb_cols = 0;
 	PlaneState state = PLANES_NONE;
 	bool filtered = false, have_rgb = false, have_coeffs = true;
@@ -498,11 +506,16 @@ DenseArrays dense_arrays(const Vp8DecodedFrame* f, bool need_coeffs, bool has_se
 // Every output holds frame after frame, each in a 256-byte aligned slot: the batch arenas and the caller's buffer of a
 // pipelined call alike. A PPM slot has kPpmSlot bytes of header room in front of the RGB.
 int ppm_header(char* buf, uint32_t w, uint32_t h) { return snprintf(buf, 32, "P6\n%u %u\n255\n", w, h); }
+// dwebp's -pam header
+int pam_header(char* buf, uint32_t w, uint32_t h) {
+	return snprintf(buf, kPamSlot, "P7\nWIDTH %u\nHEIGHT %u\nDEPTH 4\nMAXVAL 255\nTUPLTYPE RGB_ALPHA\nENDHDR\n", w, h);
+}
 
 // Bytes of a frame's slot that its output in `format` takes.
 size_t out_bytes(size_t w, size_t h, int format) {
 	return format == VP8_GPU_OUT_PNG   ? vp8_png_file_bytes((uint32_t)w, (uint32_t)h)
 	       : format == VP8_GPU_OUT_PPM ? kPpmSlot + w * h * 3
+	       : format == kOutPam         ? kPamSlot + w * h * 4
 	                                   : w * h + 2 * ((w + 1) / 2) * ((h + 1) / 2);
 }
 size_t out_slot_bytes(size_t w, size_t h, int format) { return align_up(out_bytes(w, h, format)); }
@@ -513,11 +526,12 @@ bool png_fits(uint64_t w, uint64_t h) { return (3 * w + 1) * h <= 0x7FFFFFFFull;
 // Frame i's file in its downloaded slot at dst + slot: offsets[i] / sizes[i], and the PPM header in front of the RGB.
 void report_slot(uint8_t* dst, size_t slot, uint32_t w, uint32_t h, int format, int i, size_t* offsets, size_t* sizes) {
 	size_t at = slot, bytes = out_bytes(w, h, format);
-	if (format == VP8_GPU_OUT_PPM) {
-		char hdr[32];
-		const int hl = ppm_header(hdr, w, h);
-		at += kPpmSlot - hl;
-		bytes -= kPpmSlot - hl;
+	if (format == VP8_GPU_OUT_PPM || format == kOutPam) {
+		char hdr[kPamSlot];
+		const int room = format == kOutPam ? kPamSlot : kPpmSlot;
+		const int hl = format == kOutPam ? pam_header(hdr, w, h) : ppm_header(hdr, w, h);
+		at += room - hl;
+		bytes -= room - hl;
 		memcpy(dst + at, hdr, hl);
 	}
 	if (offsets) offsets[i] = at;
@@ -526,7 +540,7 @@ void report_slot(uint8_t* dst, size_t slot, uint32_t w, uint32_t h, int format, 
 
 // Frame i's slot in the batch's arena of `format`.
 size_t slot_off(const vp8_gpu_batch* b, int i, int format) {
-	return format == VP8_GPU_OUT_PNG ? b->png_off[i] : format == VP8_GPU_OUT_PPM ? b->meta[i].rgb_off : b->meta[i].tight_off;
+	return format == VP8_GPU_OUT_PNG ? b->png_off[i] : format == VP8_GPU_OUT_PPM || format == kOutPam ? b->meta[i].rgb_off : b->meta[i].tight_off;
 }
 
 // The batch's arena of `format`: device block, size, and the bytes up to the end of the last frame (what a download copies).
@@ -538,7 +552,7 @@ OutArena out_arena(const vp8_gpu_batch* b, int format) {
 	const FrameMeta& last = b->meta.back();
 	const size_t used = slot_off(b, b->n - 1, format) + out_bytes(last.width, last.height, format);
 	if (format == VP8_GPU_OUT_PNG) return {b->d_png, b->png_bytes, used};
-	if (format == VP8_GPU_OUT_PPM) return {b->d_rgb, b->rgb_bytes, used};
+	if (format == VP8_GPU_OUT_PPM || format == kOutPam) return {b->d_rgb, b->rgb_bytes, used};
 	return {b->d_tight, b->tight_bytes, used};
 }
 
@@ -559,7 +573,7 @@ void out_layout(vp8_gpu_batch* b) {
 		m.tight_off = tight;
 		tight += out_slot_bytes(m.width, m.height, VP8_GPU_OUT_I420);
 		m.rgb_off = rgb;
-		rgb += out_slot_bytes(m.width, m.height, VP8_GPU_OUT_PPM);
+		rgb += out_slot_bytes(m.width, m.height, b->rgba ? kOutPam : VP8_GPU_OUT_PPM);
 		b->max_mb_cols = std::max<int>(b->max_mb_cols, m.mb_cols);
 	}
 	b->tight_bytes = tight;
@@ -583,6 +597,7 @@ void batch_destroy(vp8_gpu_ctx* c, vp8_gpu_batch* b, bool known_idle = false) {
 	dev_release(c, b->d_pngzdesc, sizeof(Vp8PngzDesc) * b->n);
 	dev_release(c, b->d_pngzwork, b->pngz_work_bytes);
 	dev_release(c, b->d_scratch, b->scratch_bytes);
+	dev_release(c, b->d_alphadesc, sizeof(Vp8AlphaDesc) * b->n_alpha);
 	delete b;
 }
 
@@ -1067,13 +1082,13 @@ int rgb_of_host_image(vp8_gpu_ctx* c, const Yuv420Image* img, std::vector<uint8_
 	for (uint32_t r = 0; r < ch && !rc; r++) rc = up.put(dv + (size_t)r * cw, img->v + (size_t)r * img->stride_uv, cw);
 	if (!rc) rc = up.flush();
 	if (!rc) {
-		Vp8RgbDesc d{dy, du, dv, d_rgb, w, h, w, cw, {0, 0}};
+		Vp8RgbDesc d{dy, du, dv, d_rgb, w, h, w, cw, nullptr};
 		cudaError_t e = cudaMemcpyAsync(d_desc, &d, sizeof(d), cudaMemcpyHostToDevice, c->stream);
 		if (e != cudaSuccess) rc = fail(EIO, "descriptor upload", e);
 	}
 	if (!rc) {
 		const uint32_t tiles = vp8_rgb_tiles(w, h);
-		const int lrc = vp8_launch_rgb(d_desc, 1, &tiles, c->stream);
+		const int lrc = vp8_launch_rgb(d_desc, 1, &tiles, 0, c->stream);
 		if (lrc) rc = fail(EIO, "rgb launch", (cudaError_t)lrc);
 		else c->launches++;
 	}
@@ -1435,7 +1450,7 @@ void vp8_gpu_destroy(vp8_gpu_ctx* c) {
 	}
 	if (c->d_png_tables) cudaFree(c->d_png_tables);
 	if (c->zlens) cudaFreeHost(c->zlens);
-	for (auto* v : {&c->timed, &c->timed_rgb, &c->timed_png, &c->spare})
+	for (auto* v : {&c->timed, &c->timed_rgb, &c->timed_png, &c->timed_alpha, &c->spare})
 		for (auto& ev : *v) {
 			cudaEventDestroy(ev.first);
 			cudaEventDestroy(ev.second);
@@ -1590,7 +1605,8 @@ static int push_rgb_descs(vp8_gpu_ctx* c, vp8_gpu_batch* b, int state) {
 		d.v = p.v;
 		d.stride_y = p.stride_y;
 		d.stride_uv = p.stride_uv;
-		d.rgb = b->d_rgb + m.rgb_off + kPpmSlot;
+		d.rgb = b->d_rgb + m.rgb_off + (b->rgba ? kPamSlot : kPpmSlot);
+		d.alpha = m.alpha_off != SIZE_MAX ? b->d_in + m.alpha_off : nullptr;
 	}
 	if (push_table(c, b->d_rgbdesc, h.data(), sizeof(Vp8RgbDesc) * b->n, b->stream)) return -1;
 	b->rgbdesc_key = state;
@@ -1602,11 +1618,34 @@ static int push_rgb_descs(vp8_gpu_ctx* c, vp8_gpu_batch* b, int state) {
 // i.e. behind the arenas of the next chunks the host has queued meanwhile: the first kernels then start 10 ms late
 // (VP8_GPU_TRACE=2 timeline, profiles/README.md r2).
 static int push_png_descs(vp8_gpu_ctx* c, vp8_gpu_batch* b);
+// Work items of the alpha unfilter kernel: the frames whose ALPH plane is filtered (method 0 needs no launch).
+static int push_alpha_descs(vp8_gpu_ctx* c, vp8_gpu_batch* b) {
+	std::vector<Vp8AlphaDesc> h;
+	for (const FrameMeta& m : b->meta)
+		if (m.alpha_off != SIZE_MAX && m.alpha_method) h.push_back({b->d_in + m.alpha_off, m.width, m.height, m.alpha_method, 0});
+	if (h.empty() || b->d_alphadesc) return 0;
+	b->n_alpha = (int)h.size();
+	if (dev_alloc(c, sizeof(Vp8AlphaDesc) * h.size(), (void**)&b->d_alphadesc)) return -1;
+	return push_table(c, b->d_alphadesc, h.data(), sizeof(Vp8AlphaDesc) * h.size(), b->stream);
+}
 static int push_tables_ahead(vp8_gpu_ctx* c, vp8_gpu_batch* b, int filtered, int format) {
 	if (ensure_planes(c, b, VP8_GPU_TIGHT)) return -1;
 	if (push_descs(c, b, wavefront_mode(b, filtered), VP8_GPU_TIGHT)) return -1;
 	if (format != VP8_GPU_OUT_I420 && push_rgb_descs(c, b, PLANES_TIGHT)) return -1;
+	if (format == kOutPam) return push_alpha_descs(c, b);
 	return format == VP8_GPU_OUT_PNG ? push_png_descs(c, b) : 0;
+}
+
+// The alpha planes of an RGBA batch unfiltered in place (vp8_alpha.cu), before vp8_gpu_rgb reads them.
+static int alpha_unfilter(vp8_gpu_ctx* c, vp8_gpu_batch* b) {
+	if (!b->n_alpha) return 0;
+	TimedPair ev;
+	if (begin_timed(c, b->stream, &ev)) return -1;
+	const int rc = vp8_launch_alpha_unfilter(b->d_alphadesc, b->n_alpha, b->stream);
+	if (end_timed(c, c->timed_alpha, ev, b->stream)) return -1;
+	if (rc) return fail(EIO, "alpha unfilter launch", (cudaError_t)rc);
+	c->launches++;
+	return 0;
 }
 
 int vp8_gpu_rgb(vp8_gpu_ctx* c, vp8_gpu_batch* b) {
@@ -1618,8 +1657,8 @@ int vp8_gpu_rgb(vp8_gpu_ctx* c, vp8_gpu_batch* b) {
 	for (int i = 0; i < b->n; i++) tiles[i] = vp8_rgb_tiles(b->meta[i].width, b->meta[i].height);
 	TimedPair ev;
 	if (begin_timed(c, b->stream, &ev)) return -1;
-	const int rc = vp8_launch_rgb(b->d_rgbdesc, b->n, tiles.data(), b->stream);
-	if (end_timed(c, c->timed_rgb, ev, b->stream)) return -1;
+	const int rc = vp8_launch_rgb(b->d_rgbdesc, b->n, tiles.data(), b->rgba, b->stream);
+	if (end_timed(c, b->rgba ? c->timed_alpha : c->timed_rgb, ev, b->stream)) return -1;
 	if (rc) return fail(EIO, "rgb launch", (cudaError_t)rc);
 	c->launches += (b->n + 65534) / 65535;
 	b->have_rgb = true;
@@ -1945,6 +1984,7 @@ size_t compact_frame(const Vp8DecodedFrame* f, uint8_t* arena, std::atomic<size_
 // What the pipeline needs to know about frame i before its chunk is built.
 struct FrameGeom {
 	uint32_t width, height;
+	bool alpha = false; // vp8_gpu_decode_webp_rgba: the file has an ALPH chunk
 };
 
 // Per-frame parameters of a compact batch entry from the frame's scalars; head / packed = offsets inside the device arena.
@@ -2003,12 +2043,13 @@ void pool_run(vp8_gpu_ctx* c, int threads, const std::function<void()>& work) {
 // Either returns -1 with errno set on failure, and the batch is destroyed.
 int compact_chunk(vp8_gpu_ctx* c, const FrameGeom* g, int n, size_t packed, size_t in_bytes, bool staged, int slot, cudaStream_t st,
                   const std::function<int(vp8_gpu_batch*)>& queue, const std::function<int(vp8_gpu_batch*, uint8_t*, size_t*)>& fill,
-                  vp8_gpu_batch** out) {
+                  vp8_gpu_batch** out, bool rgba = false) {
 	if (packed / 32 > 0xffffffffull) return fail(EINVAL, "compact chunk exceeds the 32-bit block index; use a smaller chunk");
 	vp8_gpu_batch* b = new (std::nothrow) vp8_gpu_batch;
 	if (!b) return fail(ENOMEM, "batch");
 	b->n = n;
 	b->stream = st;
+	b->rgba = rgba;
 	b->meta.resize(n);
 	for (int i = 0; i < n; i++) {
 		FrameMeta& m = b->meta[i];
@@ -2237,6 +2278,55 @@ int batch_create_webp(vp8_gpu_ctx* c, const uint8_t* const* files, const size_t*
 	    out);
 }
 
+// (d) .webp files for RGBA output: as (c), and the worker that parses a file with an ALPH chunk also decodes its FILTERED alpha
+// plane (raw bytes, or the green channel of a VP8L stream: webp_alpha.cpp) into the same staging slot, taking the space from the
+// same cursor, so the plane crosses with the chunk's one upload; the unfilter kernel finishes it on the device.
+int batch_create_webp_rgba(vp8_gpu_ctx* c, const uint8_t* const* files, const size_t* sizes, const FrameGeom* g, int n, int slot,
+                           cudaStream_t st, vp8_gpu_batch** out) {
+	size_t in = 0;
+	for (int i = 0; i < n; i++) {
+		in += vp8c::shared_bound((size_t)((g[i].width + 15) / 16) * ((g[i].height + 15) / 16));
+		if (g[i].alpha) in += align_up((size_t)g[i].width * g[i].height, 32);
+	}
+	return compact_chunk(
+	    c, g, n, in, in, true, slot, st, nullptr,
+	    [&](vp8_gpu_batch* b, uint8_t* stage, size_t* used) {
+		    std::atomic<size_t> cursor{0};
+		    std::atomic<int> next{0}, bad{0}, bad_errno{0};
+		    std::vector<int> order(n);
+		    for (int i = 0; i < n; i++) order[i] = i;
+		    std::stable_sort(order.begin(), order.end(), [&](int a, int b2) { return sizes[a] > sizes[b2]; });
+		    pool_run(c, pool_threads(c, n), [&]() {
+			    for (int k; (k = next.fetch_add(1)) < n;) {
+				    const int i = order[k];
+				    WebpParts p;
+				    Vp8KeyFrameHeader kf;
+				    Vp8CompactFrame cf;
+				    int rc = webp_locate(files[i], sizes[i], &p);
+				    if (!rc && (p.width != g[i].width || p.height != g[i].height || (p.alph != nullptr) != g[i].alpha)) rc = (errno = EINVAL, -1);
+				    if (!rc) rc = vp8_parse_payload_shared(p.vp8, p.vp8_size, &kf, &cf, stage, in, &cursor);
+				    if (!rc && p.alph) {
+					    const size_t px = (size_t)p.width * p.height, at = cursor.fetch_add(align_up(px, 32));
+					    if (at + px > in) rc = (errno = ENOSPC, -1);
+					    else if (!(rc = webp_alpha_filtered(&p, stage + at))) {
+						    b->meta[i].alpha_off = at;
+						    b->meta[i].alpha_method = (uint32_t)p.alpha_filter;
+					    }
+				    }
+				    if (rc) {
+					    if (!bad.fetch_add(1)) bad_errno = errno ? errno : EINVAL;
+					    continue;
+				    }
+				    compact_meta(b->meta[i], &cf.f, cf.head_off, cf.packed_off);
+			    }
+		    });
+		    if (bad.load()) return fail(bad_errno.load(), "a .webp file of the chunk failed to parse");
+		    *used = cursor.load();
+		    return 0;
+	    },
+	    out, /*rgba*/ true);
+}
+
 // Chunked pipeline: chunk k's host->device copies, kernels and device->host copy run on internal streams, so the
 // copy engines (one per direction) and the SMs work on different chunks at the same time. Blocking: returns when
 // dst holds every frame. Output layout = the layout of one big batch (frame i at offsets[i], 256-byte aligned).
@@ -2369,7 +2459,8 @@ static int decode_pipelined(vp8_gpu_ctx* c, const FrameGeom* geom, int n, const 
 		}
 		b->stream = s_run; // kernels (and the descriptor upload) of this chunk
 		rc = vp8_gpu_run(c, b, filtered, VP8_GPU_TIGHT);
-		if (!rc && (want_ppm || want_png)) rc = vp8_gpu_rgb(c, b);
+		if (!rc && format == kOutPam) rc = alpha_unfilter(c, b);
+		if (!rc && (want_ppm || want_png || format == kOutPam)) rc = vp8_gpu_rgb(c, b);
 		if (!rc && want_png) rc = vp8_gpu_png(c, b);
 		if (rc) break;
 		mark(s_run);
@@ -2584,6 +2675,44 @@ size_t vp8_gpu_decode_webp_bytes(const uint8_t* const* files, const size_t* file
 	return total;
 }
 
+// Geometry probe of the RGBA door: frame size and whether an ALPH chunk is there (container rules of webp_locate).
+static int rgba_geometry(const uint8_t* const* files, const size_t* file_sizes, int n, std::vector<FrameGeom>& g) {
+	g.resize(n);
+	for (int i = 0; i < n; i++) {
+		WebpParts p;
+		if (webp_locate(files[i], file_sizes[i], &p)) return fail(errno ? errno : EINVAL, "not a lossy WebP key frame (simple, or VP8X with optional ALPH)");
+		g[i] = {p.width, p.height, p.alph != nullptr};
+	}
+	return 0;
+}
+
+int vp8_gpu_decode_webp_rgba(vp8_gpu_ctx* c, const uint8_t* const* files, const size_t* file_sizes, int n, uint8_t* dst, size_t cap,
+                             size_t* offsets, size_t* sizes, int chunk) {
+	if (!c || !files || !file_sizes || !dst || n <= 0) return fail(EINVAL, "bad arguments");
+	std::vector<FrameGeom> g;
+	if (rgba_geometry(files, file_sizes, n, g)) return -1;
+	return in_processing_order(g, n, offsets, sizes, [&](const FrameGeom* gp, const std::vector<int>& idx, size_t* op, size_t* sp) {
+		std::vector<const uint8_t*> fp(n);
+		std::vector<size_t> fs(n);
+		for (int j = 0; j < n; j++) fp[j] = files[idx[j]], fs[j] = file_sizes[idx[j]];
+		return decode_pipelined(
+		    c, gp, n,
+		    [&](int first, int cnt, int slot, cudaStream_t s_up, bool, vp8_gpu_batch** out) {
+			    return batch_create_webp_rgba(c, fp.data() + first, fs.data() + first, gp + first, cnt, slot, s_up, out);
+		    },
+		    1, kOutPam, dst, cap, op, sp, chunk, /*ramp*/ false);
+	});
+}
+
+size_t vp8_gpu_decode_webp_rgba_bytes(const uint8_t* const* files, const size_t* file_sizes, int n) {
+	if (!files || !file_sizes || n <= 0) return 0;
+	std::vector<FrameGeom> g;
+	if (rgba_geometry(files, file_sizes, n, g)) return 0;
+	size_t total = 0;
+	for (const FrameGeom& f : g) total += out_slot_bytes(f.width, f.height, kOutPam);
+	return total;
+}
+
 int vp8_gpu_last_transport(const vp8_gpu_ctx* c, int* dense_chunks, int* compact_chunks) {
 	if (!c) return fail(EINVAL, "null context");
 	if (dense_chunks) *dense_chunks = c->last_dense_chunks;
@@ -2718,6 +2847,7 @@ static int drain_timed(vp8_gpu_ctx* c, std::vector<std::pair<cudaEvent_t, cudaEv
 int vp8_gpu_kernel_time(vp8_gpu_ctx* c, double* total_ms, int* launches) { return c ? drain_timed(c, c->timed, total_ms, launches) : fail(EINVAL, "null context"); }
 int vp8_gpu_rgb_time(vp8_gpu_ctx* c, double* total_ms, int* launches) { return c ? drain_timed(c, c->timed_rgb, total_ms, launches) : fail(EINVAL, "null context"); }
 int vp8_gpu_png_time(vp8_gpu_ctx* c, double* total_ms, int* launches) { return c ? drain_timed(c, c->timed_png, total_ms, launches) : fail(EINVAL, "null context"); }
+int vp8_gpu_alpha_time(vp8_gpu_ctx* c, double* total_ms, int* launches) { return c ? drain_timed(c, c->timed_alpha, total_ms, launches) : fail(EINVAL, "null context"); }
 
 // ================================================================================================ C-ABI: reference module interfaces
 

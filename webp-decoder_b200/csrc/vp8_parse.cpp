@@ -742,3 +742,18 @@ int vp8_parse_webp_shared(const uint8_t* file, size_t size, Vp8KeyFrameHeader* k
 	if (find_vp8_chunk(file, size, &payload, &psize)) return -1;
 	return parse_payload_compact(payload, psize, kf, cf, base, capacity, cursor, 0);
 }
+
+int vp8_parse_payload_shared(const uint8_t* payload, size_t psize, Vp8KeyFrameHeader* kf, Vp8CompactFrame* cf, uint8_t* base, size_t capacity,
+                             std::atomic<size_t>* cursor) {
+	return parse_payload_compact(payload, psize, kf, cf, base, capacity, cursor, 0);
+}
+
+int vp8_simple_chunk(const uint8_t* file, size_t size, const uint8_t** payload, size_t* psize) { return find_vp8_chunk(file, size, payload, psize); }
+
+int vp8_frame_size(const uint8_t* payload, size_t size, uint32_t* width, uint32_t* height) {
+	Vp8KeyFrameHeader kf;
+	if (read_frame_header(payload, size, &kf)) return -1;
+	*width = kf.width;
+	*height = kf.height;
+	return 0;
+}

@@ -18,6 +18,8 @@ constexpr int kRgbThreads = 128;
 
 __device__ __forceinline__ uint32_t pack_uv(uint32_t u, uint32_t v) { return u | (v << 16); }
 
+// kRgba: the same tiles stored as 4-byte pixels, the 4th byte from the frame's alpha plane (vp8_gpu_decode_webp_rgba)
+template <bool kRgba>
 __global__ void __launch_bounds__(kRgbThreads) vp8_i420_to_rgb(const Vp8RgbDesc* __restrict__ descs) {
 	const Vp8RgbDesc d = descs[blockIdx.y];
 	const uint32_t w = d.width, h = d.height, cw = (w + 1) >> 1, ch = (h + 1) >> 1;
@@ -92,6 +94,45 @@ __global__ void __launch_bounds__(kRgbThreads) vp8_i420_to_rgb(const Vp8RgbDesc*
 	uint32_t top[12], bot[12];
 	rgbk::tile_rgb(t, top, bot);
 
+	if constexpr (kRgba) {
+#pragma unroll
+		for (int row = 0; row < 2; row++) {
+			if (!(row ? has_bot : has_top)) continue;
+			const uint32_t* o = row ? bot : top;
+			const size_t at = (size_t)(2 * p - 1 + row) * w + px0;
+			uint32_t a4[4] = {0xffffffffu, 0xffffffffu, 0xffffffffu, 0xffffffffu};
+			if (d.alpha) {
+				const uint8_t* ap = d.alpha + at;
+				if (full && (reinterpret_cast<uintptr_t>(ap) & 15) == 0) {
+					const uint4 v = __ldg(reinterpret_cast<const uint4*>(ap));
+					a4[0] = v.x; a4[1] = v.y; a4[2] = v.z; a4[3] = v.w;
+				} else {
+#pragma unroll
+					for (int q = 0; q < 4; q++) {
+						uint32_t v = 0;
+						for (int k = 0; k < 4; k++) v |= (uint32_t)__ldg(ap + min(4 * q + k, (int)(w - px0) - 1)) << (8 * k);
+						a4[q] = v;
+					}
+				}
+			}
+			uint32_t px[16];
+#pragma unroll
+			for (int q = 0; q < 4; q++) rgbk::rgba_quad(o + 3 * q, a4[q], px + 4 * q);
+			uint8_t* dst = d.rgb + at * 4;
+			if (full && (reinterpret_cast<uintptr_t>(dst) & 15) == 0) {
+				uint4* d4 = reinterpret_cast<uint4*>(dst);
+#pragma unroll
+				for (int i = 0; i < 4; i++) __stcs(d4 + i, make_uint4(px[4 * i], px[4 * i + 1], px[4 * i + 2], px[4 * i + 3]));
+			} else {
+				uint32_t* d1 = reinterpret_cast<uint32_t*>(dst); // slots and rows of 4-byte pixels are always 4-byte aligned
+				const uint32_t n = min((uint32_t)rgbk::kTilePx, w - px0);
+#pragma unroll
+				for (int i = 0; i < 16; i++)
+					if ((uint32_t)i < n) __stcs(d1 + i, px[i]);
+			}
+		}
+		return;
+	}
 	const size_t row_bytes = (size_t)w * 3;
 #pragma unroll
 	for (int row = 0; row < 2; row++) {
@@ -120,7 +161,7 @@ __global__ void __launch_bounds__(kRgbThreads) vp8_i420_to_rgb(const Vp8RgbDesc*
 } // namespace
 
 // grid.y carries the image index (at most 65535 per launch), grid.x the tiles of the largest image of the slice
-int vp8_launch_rgb(const Vp8RgbDesc* descs_dev, int n_images, const uint32_t* tiles_per_image, void* stream) {
+int vp8_launch_rgb(const Vp8RgbDesc* descs_dev, int n_images, const uint32_t* tiles_per_image, int rgba, void* stream) {
 	constexpr int kSlice = 65535;
 	for (int first = 0; first < n_images; first += kSlice) {
 		const int cnt = n_images - first < kSlice ? n_images - first : kSlice;
@@ -128,7 +169,8 @@ int vp8_launch_rgb(const Vp8RgbDesc* descs_dev, int n_images, const uint32_t* ti
 		for (int i = 0; i < cnt; i++) most = tiles_per_image[first + i] > most ? tiles_per_image[first + i] : most;
 		if (!most) continue;
 		dim3 grid((most + kRgbThreads - 1) / kRgbThreads, (unsigned)cnt);
-		vp8_i420_to_rgb<<<grid, kRgbThreads, 0, (cudaStream_t)stream>>>(descs_dev + first);
+		if (rgba) vp8_i420_to_rgb<true><<<grid, kRgbThreads, 0, (cudaStream_t)stream>>>(descs_dev + first);
+		else vp8_i420_to_rgb<false><<<grid, kRgbThreads, 0, (cudaStream_t)stream>>>(descs_dev + first);
 		const cudaError_t e = cudaGetLastError();
 		if (e != cudaSuccess) return (int)e;
 	}

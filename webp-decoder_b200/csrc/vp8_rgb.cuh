@@ -124,4 +124,13 @@ VP8_RGB_FN void tile_rgb(const Tile& t, uint32_t (&top)[12], uint32_t (&bot)[12]
 	}
 }
 
+// Four pixels of tile_rgb's output (three RGB24 words) and their four alpha bytes (one word, pixel k in byte k) -> four RGBA
+// words, for the RGBA flavour of the kernel.
+VP8_RGB_FN void rgba_quad(const uint32_t* rgb3, uint32_t alpha4, uint32_t* out4) {
+	out4[0] = perm(rgb3[0], alpha4, 0x4210);                            // R0 G0 B0 A0
+	out4[1] = perm(perm(rgb3[0], rgb3[1], 0x0543), alpha4, 0x5210);      // R1 G1 B1 A1
+	out4[2] = perm(perm(rgb3[1], rgb3[2], 0x0432), alpha4, 0x6210);      // R2 G2 B2 A2
+	out4[3] = perm(rgb3[2], alpha4, 0x7321);                            // R3 G3 B3 A3
+}
+
 } // namespace rgbk

@@ -1,7 +1,7 @@
 // vp8gpu_batch - batch front end over libvp8gpu.so: the reference CLI's -yuv / -yuvf / -ppm / -png sub-commands
 // (reference src/main.c:556-842) for MANY files at once, on one or several GPUs.
 //
-//   vp8gpu_batch -yuv|-yuvf|-ppm|-png <out_dir> [--deflate] [--devices 0,1,..] [--device N] [--threads T] [--chunk C] file.webp ...
+//   vp8gpu_batch -yuv|-yuvf|-ppm|-png|-pam <out_dir> [--deflate] [--devices 0,1,..] [--device N] [--threads T] [--chunk C] file.webp ...
 //
 // --deflate (with -png only): compressed .png files - per-row PNG filters and run-length deflate, framed on the device
 // (vp8_gpu_set_png_deflate) - instead of the reference's stored-deflate bytes.
@@ -9,6 +9,8 @@
 // GPUs). Per GPU one host thread runs the whole pipeline for its share: container + header + token parsing on T / #GPUs
 // parser threads straight into the compact wire format in pinned memory (vp8_parse_batch_compact), one pipelined GPU
 // call (vp8_gpu_decode_compact), outputs written as <out_dir>/<stem>.<ext>.
+// -pam writes dwebp's RGBA -pam files and also takes lossy files with alpha (VP8X + ALPH); it goes through the .webp call
+// (vp8_gpu_decode_webp_rgba), whose parser threads read the files themselves.
 // Exit status 0 when every file decoded, 1 otherwise (one line per failed file on stderr, like the reference CLI).
 #include <errno.h>
 #include <fcntl.h>
@@ -93,6 +95,28 @@ static int run_share(int device, int slot, int n_devices, std::vector<Job*>& job
 	vp8_gpu_set_transport(ctx, 2, threads);
 	vp8_gpu_set_png_deflate(ctx, deflate);
 	int failed = 0;
+	if (mode == "-pam") {
+		std::vector<const uint8_t*> fp(n);
+		std::vector<size_t> fs(n), offs(n), sizes(n);
+		for (int k = 0; k < n; k++) fp[k] = jobs[k]->bytes.data(), fs[k] = jobs[k]->bytes.size();
+		const size_t cap = vp8_gpu_decode_webp_rgba_bytes(fp.data(), fs.data(), n);
+		uint8_t* out = cap ? (uint8_t*)vp8_gpu_host_alloc(cap) : nullptr;
+		if (!out || vp8_gpu_decode_webp_rgba(ctx, fp.data(), fs.data(), n, out, cap, offs.data(), sizes.data(), chunk)) {
+			complain("error: decode failed: %s%s\n", vp8_gpu_last_error());
+			failed = n;
+		} else {
+			for (int k = 0; k < n; k++) {
+				const std::string path = out_dir + "/" + stem_of(jobs[k]->path) + ".pam";
+				if (!write_file(path, out + offs[k], sizes[k])) {
+					complain("error: %s: write failed\n", path.c_str());
+					failed++;
+				}
+			}
+		}
+		if (out) vp8_gpu_host_free(out);
+		vp8_gpu_destroy(ctx);
+		return failed;
+	}
 	// ---- parse on host threads (m01 + m02 + m05) straight into one pinned arena, compact wire format
 	size_t arena_bytes = 0;
 	for (Job* j : jobs) arena_bytes += (vp8_parse_compact_bytes(j->w, j->h) + 255) / 256 * 256;
@@ -156,11 +180,11 @@ static int run_share(int device, int slot, int n_devices, std::vector<Job*>& job
 
 int main(int argc, char** argv) {
 	if (argc < 4) {
-		fprintf(stderr, "usage: %s -yuv|-yuvf|-ppm|-png <out_dir> [--deflate] [--devices 0,1,..] [--threads T] [--chunk C] file.webp ...\n", argv[0]);
+		fprintf(stderr, "usage: %s -yuv|-yuvf|-ppm|-png|-pam <out_dir> [--deflate] [--devices 0,1,..] [--threads T] [--chunk C] file.webp ...\n", argv[0]);
 		return 2;
 	}
 	const std::string mode = argv[1], out_dir = argv[2];
-	if (mode != "-yuv" && mode != "-yuvf" && mode != "-ppm" && mode != "-png") {
+	if (mode != "-yuv" && mode != "-yuvf" && mode != "-ppm" && mode != "-png" && mode != "-pam") {
 		fprintf(stderr, "error: unknown sub-command %s\n", mode.c_str());
 		return 2;
 	}
@@ -190,7 +214,10 @@ int main(int argc, char** argv) {
 	int failed = 0;
 	for (size_t i = 0; i < paths.size(); i++) {
 		jobs[i].path = paths[i];
-		if (!read_file(paths[i], jobs[i].bytes) || vp8_parse_webp_size(jobs[i].bytes.data(), jobs[i].bytes.size(), &jobs[i].w, &jobs[i].h)) {
+		const bool ok = read_file(paths[i], jobs[i].bytes) &&
+		                !(mode == "-pam" ? vp8_parse_webp_info(jobs[i].bytes.data(), jobs[i].bytes.size(), &jobs[i].w, &jobs[i].h, nullptr)
+		                                 : vp8_parse_webp_size(jobs[i].bytes.data(), jobs[i].bytes.size(), &jobs[i].w, &jobs[i].h));
+		if (!ok) {
 			fprintf(stderr, "error: %s: not a supported simple lossy WebP (RIFF/WEBP + single VP8 chunk)\n", paths[i]);
 			failed++;
 		} else {

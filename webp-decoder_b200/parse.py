@@ -40,6 +40,8 @@ def bind(L):
     L.vp8_parse_batch_compact.argtypes = [vp, vp, C.c_int, C.c_int, vp, vp, vp, sz, vp, vp]
     L.vp8_compact_rebase.argtypes = [vp, vp]
     L.vp8_compact_rebase.restype = None
+    L.vp8_parse_webp_info.argtypes = [vp, sz, C.POINTER(C.c_uint32), C.POINTER(C.c_uint32), C.POINTER(C.c_int)]
+    L.vp8_parse_alpha.argtypes = [vp, sz, vp, sz]
     _L = L
 
 
@@ -99,6 +101,30 @@ def webp_size(data: bytes):
         e = C.get_errno()
         raise OSError(e, "not a simple lossy WebP key frame")
     return w.value, h.value
+
+
+def webp_info(data: bytes):
+    """(width, height, has_alpha) of a simple or extended (VP8X) lossy file (vp8_parse_webp_info)."""
+    w, h, a = C.c_uint32(), C.c_uint32(), C.c_int()
+    buf = (C.c_uint8 * len(data)).from_buffer_copy(data)
+    if _lib().vp8_parse_webp_info(buf, len(data), C.byref(w), C.byref(h), C.byref(a)) != 0:
+        e = C.get_errno()
+        raise OSError(e, f"not a lossy WebP key frame: {os.strerror(e)}")
+    return w.value, h.value, bool(a.value)
+
+
+def alpha_plane(data: bytes):
+    """The unfiltered alpha plane of a .webp file as an (h, w) uint8 array, decoded on the host (vp8_parse_alpha); None for a
+    file without an ALPH chunk."""
+    w, h, has_alpha = webp_info(data)
+    if not has_alpha:
+        return None
+    out = np.empty((h, w), np.uint8)
+    buf = (C.c_uint8 * len(data)).from_buffer_copy(data)
+    if _lib().vp8_parse_alpha(buf, len(data), out.ctypes.data, out.nbytes) != 0:
+        e = C.get_errno()
+        raise OSError(e, f"alpha plane: {os.strerror(e)}")
+    return out
 
 
 def parse_batch(files, threads: int | None = None, pinned: bool = False) -> ParsedFrames:
