@@ -1,9 +1,10 @@
-// parse_arena_check.cpp - host check of the shared-arena parse (vp8_parse_webp_shared, vp8_parse.cpp): a frame whose packed
-// blocks need several 64 KiB granules is parsed into an arena of `capacity` bytes that is followed, in the same allocation,
-// by a canary region of shared_bound(mb) bytes - as far as a parse that ignored its capacity could write. Every capacity
-// that cannot hold the frame must fail with ENOSPC and leave the canary as it was; the first one that can must give the
-// same masks, first-block addresses and blocks as the standalone parse (vp8_parse_webp_compact), and so must two frames
-// that share one cursor in an arena of exactly their summed bounds. Built and run by tests/test_compact_shapes.py.
+// parse_arena_check.cpp - host check of the shared-arena parse (vp8_simple_chunk + vp8_parse_payload_shared, vp8_parse.cpp):
+// a frame whose packed blocks need several 64 KiB granules is parsed into an arena of `capacity` bytes that is followed, in
+// the same allocation, by a canary region of shared_bound(mb) bytes - as far as a parse that ignored its capacity could
+// write. Every capacity that cannot hold the frame must fail with ENOSPC and leave the canary as it was; the first one that
+// can must give the same masks, first-block addresses and blocks as the standalone parse (vp8_parse_webp_compact), and so
+// must two frames that share one cursor in an arena of exactly their summed bounds. Built and run by
+// tests/test_compact_shapes.py.
 // Usage: parse_arena_check <file.webp> <other.webp>; prints "ok <granules> <blocks>" or the first failure.
 #include <errno.h>
 #include <stdio.h>
@@ -36,6 +37,15 @@ static std::vector<uint8_t> read_file(const char* path) {
 	if (fread(d.data(), 1, d.size(), f) != d.size()) d.clear();
 	fclose(f);
 	return d;
+}
+
+// The shared-arena parse of a simple .webp file: its 'VP8 ' payload, parsed into [base, base + capacity) from *cursor.
+static int parse_shared(const std::vector<uint8_t>& file, Vp8KeyFrameHeader* kf, Vp8CompactFrame* cf, uint8_t* base, size_t capacity,
+                        std::atomic<size_t>* cursor) {
+	const uint8_t* payload;
+	size_t psize;
+	if (vp8_simple_chunk(file.data(), file.size(), &payload, &psize)) return -1;
+	return vp8_parse_payload_shared(payload, psize, kf, cf, base, capacity, cursor);
 }
 
 static size_t mb_count(const Vp8CompactFrame& cf) { return (size_t)cf.f.mb_cols * cf.f.mb_rows; }
@@ -102,7 +112,7 @@ int main(int argc, char** argv) {
 		std::atomic<size_t> cursor{0};
 		Vp8CompactFrame cf;
 		errno = 0;
-		const int rc = vp8_parse_webp_shared(file.data(), file.size(), &kf, &cf, buf, cap, &cursor);
+		const int rc = parse_shared(file, &kf, &cf, buf, cap, &cursor);
 		const int e = errno;
 		size_t ok = 0;
 		while (ok < bound && buf[cap + ok] == kCanary) ok++;
@@ -126,8 +136,8 @@ int main(int argc, char** argv) {
 	memset(buf + cap2, kCanary, bound);
 	std::atomic<size_t> cursor{0};
 	Vp8CompactFrame a, b;
-	CHECK(vp8_parse_webp_shared(file.data(), file.size(), &kf, &a, buf, cap2, &cursor) == 0, "first frame of a shared arena: errno %d", errno);
-	CHECK(vp8_parse_webp_shared(other.data(), other.size(), &kf, &b, buf, cap2, &cursor) == 0, "second frame of a shared arena: errno %d", errno);
+	CHECK(parse_shared(file, &kf, &a, buf, cap2, &cursor) == 0, "first frame of a shared arena: errno %d", errno);
+	CHECK(parse_shared(other, &kf, &b, buf, cap2, &cursor) == 0, "second frame of a shared arena: errno %d", errno);
 	CHECK(cursor.load() <= cap2, "cursor %zu past the capacity %zu", cursor.load(), cap2);
 	CHECK(same_frame(a, buf, ref, ref_packed, "shared arena, first frame"), " ");
 	CHECK(same_frame(b, buf, ref2, ref2.base + ref2.packed_off, "shared arena, second frame"), " ");

@@ -256,9 +256,9 @@ def parse_arena_check(tmp_path_factory):
 
 
 def test_shared_arena_parse_stops_at_its_capacity(parse_arena_check):
-    """vp8_parse_webp_shared with capacities from just past the frame's head up to its bound: every one that cannot hold
-    the frame (8 granules) fails with ENOSPC and writes nothing past the capacity; the rest, and two frames sharing a
-    cursor at exactly their summed bounds, give the standalone parse's masks and blocks."""
+    """vp8_simple_chunk + vp8_parse_payload_shared with capacities from just past the frame's head up to its bound: every
+    one that cannot hold the frame (8 granules) fails with ENOSPC and writes nothing past the capacity; the rest, and two
+    frames sharing a cursor at exactly their summed bounds, give the standalone parse's masks and blocks."""
     webp = GOLDEN / "webp"
     r = subprocess.run([str(parse_arena_check), str(webp / "ref_generated_gen_noise_400x416_q10.webp"),
                         str(webp / "enc_noise_200x120_q75_i16_lf.webp")], capture_output=True, text=True)

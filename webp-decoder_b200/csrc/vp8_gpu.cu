@@ -62,6 +62,14 @@ constexpr uint64_t kArenaMagic = 0x564138415245414eull; // stats_opaque[21] of f
 
 inline size_t align_up(size_t v, size_t a = kAlign) { return (v + a - 1) / a * a; }
 
+// a[idx[0]], ..., a[idx[n - 1]]: a pipelined chunk's share of the caller's arrays
+template <class T>
+std::vector<T> gather(const T* a, const int* idx, int n) {
+	std::vector<T> v(n);
+	for (int j = 0; j < n; j++) v[j] = a[idx[j]];
+	return v;
+}
+
 bool is_pinned(const void* p) {
 	cudaPointerAttributes a;
 	if (cudaPointerGetAttributes(&a, p) != cudaSuccess) {
@@ -1058,79 +1066,6 @@ int png_tables_ready(vp8_gpu_ctx* c) {
 	return 0;
 }
 
-// RGB24 of a host I420 image through the device (m08 kernel only) - or, as_png, the -png file of it (m08 + m09 kernels).
-int rgb_of_host_image(vp8_gpu_ctx* c, const Yuv420Image* img, std::vector<uint8_t>& rgb, bool as_png = false) {
-	const uint32_t w = img->width, h = img->height, cw = (w + 1) / 2, ch = (h + 1) / 2;
-	const size_t ysz = (size_t)w * h, csz = (size_t)cw * ch, total = align_up(ysz) + 2 * align_up(csz);
-	const size_t rgb_bytes = ysz * 3;
-	uint8_t *d_in = nullptr, *d_rgb = nullptr;
-	Vp8RgbDesc* d_desc = nullptr;
-	if (dev_alloc(c, total, (void**)&d_in)) return -1;
-	if (dev_alloc(c, rgb_bytes, (void**)&d_rgb) || dev_alloc(c, sizeof(Vp8RgbDesc), (void**)&d_desc)) {
-		dev_release(c, d_in, total);
-		dev_release(c, d_rgb, rgb_bytes);
-		return -1;
-	}
-	int rc = 0;
-	Uploader up{c, c->stream};
-	uint8_t* dy = d_in;
-	uint8_t* du = d_in + align_up(ysz);
-	uint8_t* dv = du + align_up(csz);
-	// tighten strides on the way in
-	for (uint32_t r = 0; r < h && !rc; r++) rc = up.put(dy + (size_t)r * w, img->y + (size_t)r * img->stride_y, w);
-	for (uint32_t r = 0; r < ch && !rc; r++) rc = up.put(du + (size_t)r * cw, img->u + (size_t)r * img->stride_uv, cw);
-	for (uint32_t r = 0; r < ch && !rc; r++) rc = up.put(dv + (size_t)r * cw, img->v + (size_t)r * img->stride_uv, cw);
-	if (!rc) rc = up.flush();
-	if (!rc) {
-		Vp8RgbDesc d{dy, du, dv, d_rgb, w, h, w, cw, nullptr};
-		cudaError_t e = cudaMemcpyAsync(d_desc, &d, sizeof(d), cudaMemcpyHostToDevice, c->stream);
-		if (e != cudaSuccess) rc = fail(EIO, "descriptor upload", e);
-	}
-	if (!rc) {
-		const uint32_t tiles = vp8_rgb_tiles(w, h);
-		const int lrc = vp8_launch_rgb(d_desc, 1, &tiles, 0, c->stream);
-		if (lrc) rc = fail(EIO, "rgb launch", (cudaError_t)lrc);
-		else c->launches++;
-	}
-	if (!rc && as_png) {
-		if (!png_fits(w, h)) rc = fail(EFBIG, "image too large for a single IDAT");
-		const size_t file_len = rc ? 0 : vp8_png_file_bytes(w, h), png_bytes = align_up(file_len), side = 256 + vp8_png_accum_bytes();
-		uint8_t *d_png = nullptr, *d_side = nullptr; // side block: descriptor, then the accumulators
-		if (!rc) rc = png_tables_ready(c);
-		if (!rc && (dev_alloc(c, png_bytes, (void**)&d_png) || dev_alloc(c, side, (void**)&d_side))) rc = -1;
-		if (!rc) {
-			Vp8PngDesc pd;
-			memset(&pd, 0, sizeof(pd));
-			pd.rgb = d_rgb;
-			pd.out = d_png;
-			pd.width = w;
-			pd.height = h;
-			vp8_png_fill_desc(&pd, png_host_tables());
-			if (push_table(c, d_side, &pd, sizeof(pd), c->stream)) rc = -1;
-		}
-		if (!rc) {
-			const int lrc = vp8_launch_png((const Vp8PngDesc*)d_side, 1, vp8_png_ctas(w, h), c->d_png_tables, d_side + 256, c->stream);
-			if (lrc) rc = fail(EIO, "png launch", (cudaError_t)lrc);
-			else c->launches += 2;
-		}
-		if (!rc) {
-			rgb.resize(file_len);
-			rc = download(c, c->stream, rgb.data(), d_png, file_len);
-		}
-		cudaStreamSynchronize(c->stream);
-		dev_release(c, d_png, png_bytes);
-		dev_release(c, d_side, side);
-	} else if (!rc) {
-		rgb.resize(rgb_bytes);
-		rc = download(c, c->stream, rgb.data(), d_rgb, rgb_bytes);
-	}
-	cudaStreamSynchronize(c->stream);
-	dev_release(c, d_in, total);
-	dev_release(c, d_rgb, rgb_bytes);
-	dev_release(c, d_desc, sizeof(Vp8RgbDesc));
-	return rc;
-}
-
 // ------------------------------------------------------------------------------------------------ PNG framing
 // Stored-deflate PNG as the reference frames it (yuv2rgb_png.c:208-364): signature, IHDR, a single IDAT holding
 // a zlib stream of stored blocks of at most 65535 bytes over filter-0 scanlines, Adler-32, IEND.
@@ -1870,7 +1805,8 @@ int vp8_gpu_download_images(vp8_gpu_ctx* c, vp8_gpu_batch* b, Yuv420Image* out) 
 //   (a) compact_frame(): host threads drop the all-zero blocks of dense Vp8DecodedFrames (the reference's contract);
 //   (b) frames the parser already emitted compact (vp8_parse_webp_compact): moved as they are, no host pass at all
 //       when they sit in pinned memory;
-//   (c) .webp bytes: host threads parse straight into the pinned arena (vp8_parse_webp_shared).
+//   (c) .webp bytes: host threads parse each file's 'VP8 ' payload (webp_locate) straight into the pinned arena
+//       (vp8_parse_payload_shared), and for RGBA output its ALPH plane beside it.
 using vp8c::kGranule;
 
 // One macroblock: appends its non-zero 4x4 blocks (32 bytes each) at out, returns the presence mask; *bytes = appended.
@@ -2243,46 +2179,12 @@ int batch_create_precompact(vp8_gpu_ctx* c, const Vp8CompactFrame* const* fr, in
 	    out);
 }
 
-// (c) .webp bytes in: the worker threads parse straight into the pinned staging slot (one image per thread at a time).
-int batch_create_webp(vp8_gpu_ctx* c, const uint8_t* const* files, const size_t* sizes, const FrameGeom* g, int n, int slot, cudaStream_t st,
-                      vp8_gpu_batch** out) {
-	size_t in = 0;
-	for (int i = 0; i < n; i++) in += vp8c::shared_bound((size_t)((g[i].width + 15) / 16) * ((g[i].height + 15) / 16));
-	return compact_chunk(
-	    c, g, n, in, in, true, slot, st, nullptr,
-	    [&](vp8_gpu_batch* b, uint8_t* stage, size_t* used) {
-		    std::atomic<size_t> cursor{0};
-		    std::atomic<int> next{0}, bad{0}, bad_errno{0};
-		    const int threads = pool_threads(c, n);
-		    // parse time goes with the file size and differs by two orders of magnitude between files: longest first, so that the
-		    // chunk does not end with one thread on a big file and the others idle
-		    std::vector<int> order(n);
-		    for (int i = 0; i < n; i++) order[i] = i;
-		    std::stable_sort(order.begin(), order.end(), [&](int a, int b2) { return sizes[a] > sizes[b2]; });
-		    pool_run(c, threads, [&]() {
-			    for (int k; (k = next.fetch_add(1)) < n;) {
-				    const int i = order[k];
-				    Vp8KeyFrameHeader kf;
-				    Vp8CompactFrame cf;
-				    if (vp8_parse_webp_shared(files[i], sizes[i], &kf, &cf, stage, in, &cursor) || kf.width != g[i].width || kf.height != g[i].height) {
-					    if (!bad.fetch_add(1)) bad_errno = errno ? errno : EINVAL;
-					    continue;
-				    }
-				    compact_meta(b->meta[i], &cf.f, cf.head_off, cf.packed_off);
-			    }
-		    });
-		    if (bad.load()) return fail(bad_errno.load(), "a .webp file of the chunk failed to parse");
-		    *used = cursor.load();
-		    return 0;
-	    },
-	    out);
-}
-
-// (d) .webp files for RGBA output: as (c), and the worker that parses a file with an ALPH chunk also decodes its FILTERED alpha
-// plane (raw bytes, or the green channel of a VP8L stream: webp_alpha.cpp) into the same staging slot, taking the space from the
-// same cursor, so the plane crosses with the chunk's one upload; the unfilter kernel finishes it on the device.
-int batch_create_webp_rgba(vp8_gpu_ctx* c, const uint8_t* const* files, const size_t* sizes, const FrameGeom* g, int n, int slot,
-                           cudaStream_t st, vp8_gpu_batch** out) {
+// (c) .webp files in: the worker threads locate each file's 'VP8 ' payload (webp_locate) and parse it straight into the pinned
+// staging slot (one image per thread at a time). For RGBA output, the worker that parses a file with an ALPH chunk also decodes
+// its FILTERED alpha plane (raw bytes, or the green channel of a VP8L stream: webp_alpha.cpp) into the same staging slot, taking
+// the space from the same cursor, so the plane crosses with the chunk's one upload; the unfilter kernel finishes it on the device.
+int batch_create_webp(vp8_gpu_ctx* c, const uint8_t* const* files, const size_t* sizes, const FrameGeom* g, int n, bool rgba, int slot,
+                      cudaStream_t st, vp8_gpu_batch** out) {
 	size_t in = 0;
 	for (int i = 0; i < n; i++) {
 		in += vp8c::shared_bound((size_t)((g[i].width + 15) / 16) * ((g[i].height + 15) / 16));
@@ -2293,6 +2195,8 @@ int batch_create_webp_rgba(vp8_gpu_ctx* c, const uint8_t* const* files, const si
 	    [&](vp8_gpu_batch* b, uint8_t* stage, size_t* used) {
 		    std::atomic<size_t> cursor{0};
 		    std::atomic<int> next{0}, bad{0}, bad_errno{0};
+		    // parse time goes with the file size and differs by two orders of magnitude between files: longest first, so that the
+		    // chunk does not end with one thread on a big file and the others idle
 		    std::vector<int> order(n);
 		    for (int i = 0; i < n; i++) order[i] = i;
 		    std::stable_sort(order.begin(), order.end(), [&](int a, int b2) { return sizes[a] > sizes[b2]; });
@@ -2324,17 +2228,44 @@ int batch_create_webp_rgba(vp8_gpu_ctx* c, const uint8_t* const* files, const si
 		    *used = cursor.load();
 		    return 0;
 	    },
-	    out, /*rgba*/ true);
+	    out, rgba);
 }
 
 // Chunked pipeline: chunk k's host->device copies, kernels and device->host copy run on internal streams, so the
 // copy engines (one per direction) and the SMs work on different chunks at the same time. Blocking: returns when
-// dst holds every frame. Output layout = the layout of one big batch (frame i at offsets[i], 256-byte aligned).
-// make_chunk(first, count, staging slot, upload stream, link_idle, &batch) builds and uploads one chunk; link_idle says
-// whether everything queued on the upload stream so far has already left the host.
-using ChunkMaker = std::function<int(int, int, int, cudaStream_t, bool, vp8_gpu_batch**)>;
+// dst holds every frame. Output layout = the layout of one big batch of the frames in processing order (processing_order), each
+// in a 256-byte aligned slot; offsets[i] / sizes[i] are reported for the caller's frame i. geom is in the caller's order.
+// make_chunk(idx, count, staging slot, upload stream, &batch) builds and uploads one chunk: the caller's frames idx[0..count).
+using ChunkMaker = std::function<int(const int*, int, int, cudaStream_t, vp8_gpu_batch**)>;
 
 static int out_format(int ppm) { return ppm == VP8_GPU_OUT_PNG ? VP8_GPU_OUT_PNG : ppm ? VP8_GPU_OUT_PPM : VP8_GPU_OUT_I420; }
+
+// A chunk's kernels take as long as its biggest frame needs (one frame is a dependency chain, spread over a cluster at best),
+// so a call whose frames differ a lot in size processes them biggest first: the 4K frames share the first chunks, each on a
+// cluster of several SMs, instead of putting their latency into every chunk. Returns the caller's indices in processing order.
+static std::vector<int> processing_order(const FrameGeom* g, int n) {
+	size_t lo = ~(size_t)0, hi = 0;
+	std::vector<int> ord(n);
+	for (int i = 0; i < n; i++) {
+		const size_t px = (size_t)g[i].width * g[i].height;
+		lo = std::min(lo, px);
+		hi = std::max(hi, px);
+		ord[i] = i;
+	}
+	if (n >= 2 && hi >= 2 * lo)
+		std::stable_sort(ord.begin(), ord.end(), [&](int a, int b) { return (size_t)g[a].width * g[a].height > (size_t)g[b].width * g[b].height; });
+	return ord;
+}
+
+// Bytes of a pipelined call's output: every frame's slot; 0 when a -png frame does not fit one IDAT.
+static size_t out_total_bytes(const FrameGeom* g, int n, int format) {
+	size_t total = 0;
+	for (int i = 0; i < n; i++) {
+		if (format == VP8_GPU_OUT_PNG && !png_fits(g[i].width, g[i].height)) return 0;
+		total += out_slot_bytes(g[i].width, g[i].height, format);
+	}
+	return total;
+}
 
 static int decode_pipelined(vp8_gpu_ctx* c, const FrameGeom* geom, int n, const ChunkMaker& make_chunk, int filtered, int format,
                             uint8_t* dst, size_t cap, size_t* offsets, size_t* sizes, int chunk, bool ramp = true) {
@@ -2344,12 +2275,10 @@ static int decode_pipelined(vp8_gpu_ctx* c, const FrameGeom* geom, int n, const 
 			if (!png_fits(geom[i].width, geom[i].height)) return fail(EFBIG, "image too large for a single IDAT");
 	CU(cudaSetDevice(c->device));
 	if (chunk <= 0) chunk = 64;
-	// global layout
+	// global layout: slot j holds the caller's frame ord[j]
+	const std::vector<int> ord = processing_order(geom, n);
 	std::vector<size_t> off(n + 1, 0);
-	for (int i = 0; i < n; i++) {
-		const size_t w = geom[i].width, h = geom[i].height;
-		off[i + 1] = off[i] + out_slot_bytes(w, h, format);
-	}
+	for (int j = 0; j < n; j++) off[j + 1] = off[j] + out_slot_bytes(geom[ord[j]].width, geom[ord[j]].height, format);
 	if (cap < off[n]) return fail(EINVAL, "destination too small");
 	// Compressed -png: a chunk's files have their length only once its kernels ran. Its lengths (4 bytes a file) come back into
 	// pinned memory first, and its download - ONE copy of its files, packed behind those of the chunk before - is enqueued one
@@ -2445,8 +2374,7 @@ static int decode_pipelined(vp8_gpu_ctx* c, const FrameGeom* geom, int n, const 
 		c->trace_retire_ms += std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_r0).count();
 		vp8_gpu_batch* b = nullptr;
 		if (timeline) tl_host.push_back(std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_p0).count());
-		const bool link_idle = k == 0 || cudaEventQuery(ring[(k - 1) % kDepth].up) == cudaSuccess;
-		rc = make_chunk(first, cnt, slot, s_up, link_idle, &b);
+		rc = make_chunk(ord.data() + first, cnt, slot, s_up, &b);
 		if (rc) break;
 		ch.b = b;
 		b->stream = s_up;
@@ -2521,57 +2449,17 @@ static int decode_pipelined(vp8_gpu_ctx* c, const FrameGeom* geom, int n, const 
 		errno = saved;
 		return -1;
 	}
-	for (int i = 0; i < n; i++) {
+	for (int j = 0; j < n; j++) {
+		const int i = ord[j];
 		if (!deflate) {
-			report_slot(dst, off[i], geom[i].width, geom[i].height, format, i, offsets, sizes);
+			report_slot(dst, off[j], geom[i].width, geom[i].height, format, i, offsets, sizes);
 			continue;
 		}
-		if (offsets) offsets[i] = zoff[i];
-		if (sizes) sizes[i] = c->zlens[i];
+		if (offsets) offsets[i] = zoff[j];
+		if (sizes) sizes[i] = c->zlens[j];
 	}
 	return 0;
 }
-
-// A chunk's kernels take as long as its biggest frame needs (one frame is a dependency chain, spread over a cluster at best),
-// so a call whose frames differ a lot in size processes them biggest first: the 4K frames share the first chunks, each on a
-// cluster of several SMs, instead of putting their latency into every chunk. Returns the processing order; empty = as given.
-static std::vector<int> processing_order(const FrameGeom* g, int n) {
-	size_t lo = ~(size_t)0, hi = 0;
-	for (int i = 0; i < n; i++) {
-		const size_t px = (size_t)g[i].width * g[i].height;
-		lo = std::min(lo, px);
-		hi = std::max(hi, px);
-	}
-	if (n < 2 || hi < 2 * lo) return {};
-	std::vector<int> ord(n);
-	for (int i = 0; i < n; i++) ord[i] = i;
-	std::stable_sort(ord.begin(), ord.end(), [&](int a, int b) { return (size_t)g[a].width * g[a].height > (size_t)g[b].width * g[b].height; });
-	return ord;
-}
-
-// Runs `call(geometry, index map, offsets, sizes)` on the frames in processing order and hands offsets / sizes back in the
-// caller's order. idx[j] = caller's index of the j-th processed frame.
-extern "C++" {
-template <class Call>
-static int in_processing_order(std::vector<FrameGeom>& g, int n, size_t* offsets, size_t* sizes, Call call) {
-	std::vector<int> ord = processing_order(g.data(), n);
-	if (ord.empty()) {
-		ord.resize(n);
-		for (int i = 0; i < n; i++) ord[i] = i;
-		return call(g.data(), ord, offsets, sizes);
-	}
-	std::vector<FrameGeom> gp(n);
-	for (int j = 0; j < n; j++) gp[j] = g[ord[j]];
-	std::vector<size_t> op(n), sp(n);
-	const int rc = call(gp.data(), ord, op.data(), sp.data());
-	if (rc) return rc;
-	for (int j = 0; j < n; j++) {
-		if (offsets) offsets[ord[j]] = op[j];
-		if (sizes) sizes[ord[j]] = sp[j];
-	}
-	return 0;
-}
-} // extern "C++"
 
 // The reference's contract: dense Vp8DecodedFrames in host memory. Which transport carries them is a host question: the
 // compact one needs every frame's 6.7 MB (1080p) read by host threads and then moves a third of the bytes, the dense one
@@ -2592,19 +2480,16 @@ static int decode_dense(vp8_gpu_ctx* c, const Vp8KeyFrameHeader* const* kf, cons
 	const int threads = c->host_threads > 0 ? c->host_threads : (int)std::min(32u, std::max(1u, std::thread::hardware_concurrency()));
 	const bool compact = c->transport_mode == 1 || (c->transport_mode == 2 && threads >= kCompactMinThreads);
 	c->last_dense_chunks = c->last_compact_chunks = 0;
-	return in_processing_order(g, n, offsets, sizes, [&](const FrameGeom* gp, const std::vector<int>& idx, size_t* op, size_t* sp) {
-		std::vector<const Vp8KeyFrameHeader*> kfp(n);
-		std::vector<const Vp8DecodedFrame*> frp(n);
-		for (int j = 0; j < n; j++) kfp[j] = kf[idx[j]], frp[j] = frames[idx[j]];
-		return decode_pipelined(
-		    c, gp, n,
-		    [&](int first, int cnt, int slot, cudaStream_t s_up, bool, vp8_gpu_batch** out) {
-			    (compact ? c->last_compact_chunks : c->last_dense_chunks)++;
-			    return compact ? batch_create_compact(c, kfp.data() + first, frp.data() + first, cnt, slot, s_up, out)
-			                   : batch_create(c, kfp.data() + first, frp.data() + first, cnt, true, out, s_up, true);
-		    },
-		    filtered, format, dst, cap, op, sp, chunk);
-	});
+	return decode_pipelined(
+	    c, g.data(), n,
+	    [&](const int* idx, int cnt, int slot, cudaStream_t s_up, vp8_gpu_batch** out) {
+		    const auto k = gather(kf, idx, cnt);
+		    const auto f = gather(frames, idx, cnt);
+		    (compact ? c->last_compact_chunks : c->last_dense_chunks)++;
+		    return compact ? batch_create_compact(c, k.data(), f.data(), cnt, slot, s_up, out)
+		                   : batch_create(c, k.data(), f.data(), cnt, true, out, s_up, true);
+	    },
+	    filtered, format, dst, cap, offsets, sizes, chunk);
 }
 
 int vp8_gpu_decode_i420(vp8_gpu_ctx* c, const Vp8KeyFrameHeader* const* kf, const Vp8DecodedFrame* const* frames, int n, int filtered,
@@ -2630,87 +2515,71 @@ int vp8_gpu_decode_compact(vp8_gpu_ctx* c, const Vp8CompactFrame* const* frames,
 		if (validate_compact(frames[i])) return -1;
 		g[i] = {frames[i]->width, frames[i]->height};
 	}
-	return in_processing_order(g, n, offsets, sizes, [&](const FrameGeom* gp, const std::vector<int>& idx, size_t* op, size_t* sp) {
-		std::vector<const Vp8CompactFrame*> frp(n);
-		for (int j = 0; j < n; j++) frp[j] = frames[idx[j]];
-		return decode_pipelined(
-		    c, gp, n,
-		    [&](int first, int cnt, int slot, cudaStream_t s_up, bool, vp8_gpu_batch** out) {
-			    return batch_create_precompact(c, frp.data() + first, cnt, slot, s_up, out);
-		    },
-		    ppm ? 1 : filtered, out_format(ppm), dst, cap, op, sp, chunk);
-	});
+	return decode_pipelined(
+	    c, g.data(), n,
+	    [&](const int* idx, int cnt, int slot, cudaStream_t s_up, vp8_gpu_batch** out) {
+		    return batch_create_precompact(c, gather(frames, idx, cnt).data(), cnt, slot, s_up, out);
+	    },
+	    ppm ? 1 : filtered, out_format(ppm), dst, cap, offsets, sizes, chunk);
 }
 
-int vp8_gpu_decode_webp(vp8_gpu_ctx* c, const uint8_t* const* files, const size_t* file_sizes, int n, int filtered, int ppm, uint8_t* dst,
-                        size_t cap, size_t* offsets, size_t* sizes, int chunk) {
-	if (!c || !files || !file_sizes || !dst || n <= 0) return fail(EINVAL, "bad arguments");
-	std::vector<FrameGeom> g(n);
-	for (int i = 0; i < n; i++) {
-		uint32_t w = 0, h = 0;
-		if (vp8_parse_webp_size(files[i], file_sizes[i], &w, &h)) return fail(errno ? errno : EINVAL, "not a simple lossy WebP key frame");
-		g[i] = {w, h};
-	}
-	return in_processing_order(g, n, offsets, sizes, [&](const FrameGeom* gp, const std::vector<int>& idx, size_t* op, size_t* sp) {
-		std::vector<const uint8_t*> fp(n);
-		std::vector<size_t> fs(n);
-		for (int j = 0; j < n; j++) fp[j] = files[idx[j]], fs[j] = file_sizes[idx[j]];
-		return decode_pipelined(
-		    c, gp, n,
-		    [&](int first, int cnt, int slot, cudaStream_t s_up, bool, vp8_gpu_batch** out) {
-			    return batch_create_webp(c, fp.data() + first, fs.data() + first, gp + first, cnt, slot, s_up, out);
-		    },
-		    ppm ? 1 : filtered, out_format(ppm), dst, cap, op, sp, chunk, /*ramp*/ false);
-	});
-}
-
-size_t vp8_gpu_decode_webp_bytes(const uint8_t* const* files, const size_t* file_sizes, int n, int ppm) {
-	size_t total = 0;
-	for (int i = 0; files && file_sizes && i < n; i++) {
-		uint32_t w = 0, h = 0;
-		if (vp8_parse_webp_size(files[i], file_sizes[i], &w, &h)) return 0;
-		if (ppm == VP8_GPU_OUT_PNG && !png_fits(w, h)) return 0;
-		total += out_slot_bytes(w, h, out_format(ppm));
-	}
-	return total;
-}
-
-// Geometry probe of the RGBA door: frame size and whether an ALPH chunk is there (container rules of webp_locate).
-static int rgba_geometry(const uint8_t* const* files, const size_t* file_sizes, int n, std::vector<FrameGeom>& g) {
+// Geometry of .webp files for output `format`: the RGBA call (kOutPam) takes what webp_locate accepts and notes which files have
+// an ALPH chunk, the others take simple files only (vp8_parse_webp_size).
+static int webp_geometry(const uint8_t* const* files, const size_t* file_sizes, int n, int format, std::vector<FrameGeom>& g) {
 	g.resize(n);
 	for (int i = 0; i < n; i++) {
-		WebpParts p;
-		if (webp_locate(files[i], file_sizes[i], &p)) return fail(errno ? errno : EINVAL, "not a lossy WebP key frame (simple, or VP8X with optional ALPH)");
-		g[i] = {p.width, p.height, p.alph != nullptr};
+		if (format == kOutPam) {
+			WebpParts p;
+			if (webp_locate(files[i], file_sizes[i], &p)) return fail(errno ? errno : EINVAL, "not a lossy WebP key frame (simple, or VP8X with optional ALPH)");
+			g[i] = {p.width, p.height, p.alph != nullptr};
+		} else {
+			uint32_t w = 0, h = 0;
+			if (vp8_parse_webp_size(files[i], file_sizes[i], &w, &h)) return fail(errno ? errno : EINVAL, "not a simple lossy WebP key frame");
+			g[i] = {w, h};
+		}
 	}
 	return 0;
 }
 
-int vp8_gpu_decode_webp_rgba(vp8_gpu_ctx* c, const uint8_t* const* files, const size_t* file_sizes, int n, uint8_t* dst, size_t cap,
-                             size_t* offsets, size_t* sizes, int chunk) {
+// vp8_gpu_decode_webp (format from its `ppm` argument) and vp8_gpu_decode_webp_rgba (kOutPam).
+static int decode_webp(vp8_gpu_ctx* c, const uint8_t* const* files, const size_t* file_sizes, int n, int filtered, int format, uint8_t* dst,
+                       size_t cap, size_t* offsets, size_t* sizes, int chunk) {
 	if (!c || !files || !file_sizes || !dst || n <= 0) return fail(EINVAL, "bad arguments");
 	std::vector<FrameGeom> g;
-	if (rgba_geometry(files, file_sizes, n, g)) return -1;
-	return in_processing_order(g, n, offsets, sizes, [&](const FrameGeom* gp, const std::vector<int>& idx, size_t* op, size_t* sp) {
-		std::vector<const uint8_t*> fp(n);
-		std::vector<size_t> fs(n);
-		for (int j = 0; j < n; j++) fp[j] = files[idx[j]], fs[j] = file_sizes[idx[j]];
-		return decode_pipelined(
-		    c, gp, n,
-		    [&](int first, int cnt, int slot, cudaStream_t s_up, bool, vp8_gpu_batch** out) {
-			    return batch_create_webp_rgba(c, fp.data() + first, fs.data() + first, gp + first, cnt, slot, s_up, out);
-		    },
-		    1, kOutPam, dst, cap, op, sp, chunk, /*ramp*/ false);
-	});
+	if (webp_geometry(files, file_sizes, n, format, g)) return -1;
+	return decode_pipelined(
+	    c, g.data(), n,
+	    [&](const int* idx, int cnt, int slot, cudaStream_t s_up, vp8_gpu_batch** out) {
+		    const auto f = gather(files, idx, cnt);
+		    const auto fs = gather(file_sizes, idx, cnt);
+		    const auto fg = gather(g.data(), idx, cnt);
+		    return batch_create_webp(c, f.data(), fs.data(), fg.data(), cnt, format == kOutPam, slot, s_up, out);
+	    },
+	    filtered, format, dst, cap, offsets, sizes, chunk, /*ramp*/ false);
+}
+
+static size_t webp_bytes(const uint8_t* const* files, const size_t* file_sizes, int n, int format) {
+	std::vector<FrameGeom> g;
+	if (!files || !file_sizes || n <= 0 || webp_geometry(files, file_sizes, n, format, g)) return 0;
+	return out_total_bytes(g.data(), n, format);
+}
+
+int vp8_gpu_decode_webp(vp8_gpu_ctx* c, const uint8_t* const* files, const size_t* file_sizes, int n, int filtered, int ppm, uint8_t* dst,
+                        size_t cap, size_t* offsets, size_t* sizes, int chunk) {
+	return decode_webp(c, files, file_sizes, n, ppm ? 1 : filtered, out_format(ppm), dst, cap, offsets, sizes, chunk);
+}
+
+size_t vp8_gpu_decode_webp_bytes(const uint8_t* const* files, const size_t* file_sizes, int n, int ppm) {
+	return webp_bytes(files, file_sizes, n, out_format(ppm));
+}
+
+int vp8_gpu_decode_webp_rgba(vp8_gpu_ctx* c, const uint8_t* const* files, const size_t* file_sizes, int n, uint8_t* dst, size_t cap,
+                             size_t* offsets, size_t* sizes, int chunk) {
+	return decode_webp(c, files, file_sizes, n, 1, kOutPam, dst, cap, offsets, sizes, chunk);
 }
 
 size_t vp8_gpu_decode_webp_rgba_bytes(const uint8_t* const* files, const size_t* file_sizes, int n) {
-	if (!files || !file_sizes || n <= 0) return 0;
-	std::vector<FrameGeom> g;
-	if (rgba_geometry(files, file_sizes, n, g)) return 0;
-	size_t total = 0;
-	for (const FrameGeom& f : g) total += out_slot_bytes(f.width, f.height, kOutPam);
-	return total;
+	return webp_bytes(files, file_sizes, n, kOutPam);
 }
 
 int vp8_gpu_last_transport(const vp8_gpu_ctx* c, int* dense_chunks, int* compact_chunks) {
@@ -2791,13 +2660,9 @@ int vp8_gpu_bind_host(vp8_gpu_ctx* c, int index, int share) {
 }
 
 size_t vp8_gpu_decode_bytes(const Vp8KeyFrameHeader* const* kf, int n, int ppm) {
-	size_t total = 0;
-	for (int i = 0; kf && i < n; i++) {
-		const size_t w = kf[i]->width, h = kf[i]->height;
-		if (ppm == VP8_GPU_OUT_PNG && !png_fits(w, h)) return 0;
-		total += out_slot_bytes(w, h, out_format(ppm));
-	}
-	return total;
+	std::vector<FrameGeom> g(kf && n > 0 ? n : 0);
+	for (size_t i = 0; i < g.size(); i++) g[i] = {kf[i]->width, kf[i]->height};
+	return out_total_bytes(g.data(), (int)g.size(), out_format(ppm));
 }
 
 size_t vp8_gpu_png_bound(uint32_t width, uint32_t height) {
@@ -2968,30 +2833,65 @@ int vp8_loopfilter_apply_keyframe(Yuv420Image* img, const Vp8DecodedFrame* decod
 	return 0;
 }
 
-static int rgb_for_writer(int fd, const Yuv420Image* img, std::vector<uint8_t>& rgb, bool as_png = false) {
+// The PPM or -png file (`format`) of a host I420 image, made on the device as a one-frame batch without coefficients: the
+// planes go into its tight I420 slot, then vp8_gpu_rgb (m08) and, for -png, vp8_gpu_png (m09). file[*at, *at + *len) is it.
+static int file_of_host_image(vp8_gpu_ctx* c, const Yuv420Image* img, int format, std::vector<uint8_t>& file, size_t* at, size_t* len) {
+	vp8_gpu_batch* b = new (std::nothrow) vp8_gpu_batch;
+	if (!b) return fail(ENOMEM, "batch");
+	b->n = 1;
+	b->stream = c->stream;
+	b->have_coeffs = false;
+	b->meta.resize(1);
+	FrameMeta& m = b->meta[0];
+	m.width = img->width;
+	m.height = img->height;
+	m.mb_cols = (m.width + 15) / 16;
+	m.mb_rows = (m.height + 15) / 16;
+	out_layout(b);
+	int rc = ensure_planes(c, b, VP8_GPU_TIGHT);
+	if (!rc) {
+		const PlaneView p = plane_view(b, m, true);
+		const uint32_t w = m.width, h = m.height, cw = (w + 1) / 2, ch = (h + 1) / 2;
+		Uploader up{c, b->stream};
+		// tighten strides on the way in
+		for (uint32_t r = 0; r < h && !rc; r++) rc = up.put(p.y + (size_t)r * w, img->y + (size_t)r * img->stride_y, w);
+		for (uint32_t r = 0; r < ch && !rc; r++) rc = up.put(p.u + (size_t)r * cw, img->u + (size_t)r * img->stride_uv, cw);
+		for (uint32_t r = 0; r < ch && !rc; r++) rc = up.put(p.v + (size_t)r * cw, img->v + (size_t)r * img->stride_uv, cw);
+		if (!rc) rc = up.flush();
+	}
+	if (!rc) {
+		b->state = PLANES_TIGHT;
+		rc = vp8_gpu_rgb(c, b);
+	}
+	if (!rc && format == VP8_GPU_OUT_PNG) rc = vp8_gpu_png(c, b);
+	if (!rc) {
+		file.resize(out_arena(b, format).bytes);
+		rc = format == VP8_GPU_OUT_PNG ? vp8_gpu_download_png(c, b, file.data(), file.size(), at, len)
+		                               : download_out(c, b, format, file.data(), file.size(), at, len);
+	}
+	const int saved = errno;
+	batch_destroy(c, b);
+	errno = saved;
+	return rc;
+}
+
+static int write_image(int fd, const Yuv420Image* img, int format) {
 	if (fd < 0 || !img || !img->y || !img->u || !img->v || img->width == 0 || img->height == 0) {
 		errno = EINVAL;
 		return -1;
 	}
-	std::lock_guard<std::mutex> lock(g_default_mu);
-	vp8_gpu_ctx* c = default_ctx();
-	if (!c) return -1;
-	return rgb_of_host_image(c, img, rgb, as_png);
+	std::vector<uint8_t> file;
+	size_t at = 0, len = 0;
+	{
+		std::lock_guard<std::mutex> lock(g_default_mu);
+		vp8_gpu_ctx* c = default_ctx(); // never has deflate on: its -png files are the reference's stored-deflate bytes
+		if (!c || file_of_host_image(c, img, format, file, &at, &len)) return -1;
+	}
+	return write_all(fd, file.data() + at, len);
 }
 
-int yuv420_write_ppm_fd(int fd, const Yuv420Image* img) {
-	std::vector<uint8_t> rgb;
-	if (rgb_for_writer(fd, img, rgb)) return -1;
-	char hdr[32];
-	const int hl = ppm_header(hdr, img->width, img->height);
-	if (write_all(fd, hdr, (size_t)hl) || write_all(fd, rgb.data(), rgb.size())) return -1;
-	return 0;
-}
+int yuv420_write_ppm_fd(int fd, const Yuv420Image* img) { return write_image(fd, img, VP8_GPU_OUT_PPM); }
 
-int yuv420_write_png_fd(int fd, const Yuv420Image* img) {
-	std::vector<uint8_t> png; // framed on the device: vp8_png_frame / vp8_png_finish behind the RGB kernel
-	if (rgb_for_writer(fd, img, png, true)) return -1;
-	return write_all(fd, png.data(), png.size());
-}
+int yuv420_write_png_fd(int fd, const Yuv420Image* img) { return write_image(fd, img, VP8_GPU_OUT_PNG); }
 
 } // extern "C"

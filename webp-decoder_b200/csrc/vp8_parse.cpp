@@ -735,14 +735,6 @@ void vp8_compact_rebase(Vp8CompactFrame* f, void* new_start) {
 
 } // extern "C"
 
-int vp8_parse_webp_shared(const uint8_t* file, size_t size, Vp8KeyFrameHeader* kf, Vp8CompactFrame* cf, uint8_t* base, size_t capacity,
-                          std::atomic<size_t>* cursor) {
-	const uint8_t* payload;
-	size_t psize;
-	if (find_vp8_chunk(file, size, &payload, &psize)) return -1;
-	return parse_payload_compact(payload, psize, kf, cf, base, capacity, cursor, 0);
-}
-
 int vp8_parse_payload_shared(const uint8_t* payload, size_t psize, Vp8KeyFrameHeader* kf, Vp8CompactFrame* cf, uint8_t* base, size_t capacity,
                              std::atomic<size_t>* cursor) {
 	return parse_payload_compact(payload, psize, kf, cf, base, capacity, cursor, 0);

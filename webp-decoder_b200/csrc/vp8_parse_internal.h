@@ -42,11 +42,6 @@ inline size_t shared_bound(size_t mb) { return layout(mb).o_packed + (kMbWorst *
 
 } // namespace vp8c
 
-// Parse one .webp file into a shared arena: the head and the block granules are taken from *cursor (threads parsing other
-// frames of the same chunk do the same), mb_first counts from `base`. cf->packed_off == 0, cf->bytes == 0.
-int vp8_parse_webp_shared(const uint8_t* file, size_t size, Vp8KeyFrameHeader* kf, Vp8CompactFrame* cf, uint8_t* base, size_t capacity,
-                          std::atomic<size_t>* cursor);
-
 // ---- extended files (webp_alpha.cpp). The parts of a .webp file the RGBA door needs: the 'VP8 ' payload, the frame size and,
 // for an extended (VP8X) file, its ALPH chunk. Simple files follow the reference's rules (vp8_simple_chunk); extended ones the
 // container rules of vp8_parse_webp_info (include/vp8_parse.h). -1 with errno set.
@@ -64,8 +59,9 @@ int webp_locate(const uint8_t* file, size_t size, WebpParts* out);
 // channel of the VP8L image stream.
 int webp_alpha_filtered(const WebpParts* parts, uint8_t* plane);
 
-// vp8_parse.cpp: the reference's simple-file rule (find_vp8_chunk), the frame size of a 'VP8 ' payload, and
-// vp8_parse_webp_shared for a payload that was located already.
+// vp8_parse.cpp: the reference's simple-file rule (find_vp8_chunk), the frame size of a 'VP8 ' payload, and the parse of a
+// located 'VP8 ' payload into a shared arena: the head and the block granules are taken from *cursor (threads parsing other
+// frames of the same chunk do the same), mb_first counts from `base`. cf->packed_off == 0, cf->bytes == 0.
 int vp8_simple_chunk(const uint8_t* file, size_t size, const uint8_t** payload, size_t* psize);
 int vp8_frame_size(const uint8_t* payload, size_t size, uint32_t* width, uint32_t* height);
 int vp8_parse_payload_shared(const uint8_t* payload, size_t psize, Vp8KeyFrameHeader* kf, Vp8CompactFrame* cf, uint8_t* base, size_t capacity,
